@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- the hot path's headline metrics on B200 (contract: see the task statement / DESIGN.md section 6).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload train|infer]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload train|infer] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Default workload = BASELINE.json configs[1]: dilated_grsl (Dilated6Pooling), multinomial patch sizes
@@ -14,6 +14,14 @@ Potsdam-shaped 6000x6000x5 scene with dilated_grsl_rate8 (configs[3]) in Mpixel/
 
 --impl reference times the reference-equivalent CPU path (TensorFlow is not installable here: the oracle's
 PyTorch-CPU restatement of the graph + the NumPy restatement of the host loops) on a bounded sample.
+
+--dump-outputs DIR writes, after the timed steps, what the timed path computed in its last timed step as DIR/<name>.npy
+(float32 / float64, rank 0 only), so that two builds can be compared output for output on the same seeded inputs:
+  train_loss, train_confusion, train_n_correct, train_pred   what the training step returns (loss, per-crop confusion
+                                                               matrix, correct pixels, predicted labels [B, crop, crop])
+  train_var__<scope>__<name>                                   every variable and momentum slot after that step
+  infer_label_counts                                           pixels per class of the last timed scene pass's label map
+  infer_labels_sample, infer_labels_sample_index               2^20 of its pixels at fixed seeded flat indices
 """
 import argparse
 import json
@@ -201,7 +209,8 @@ def conv_flops_train(net, C, K, M):
 # ----------------------------------------------------------------------------------------------------------------
 # ours
 # ----------------------------------------------------------------------------------------------------------------
-def run_train_ours(args, rank, world, local, cfg=None, sync_bn=False, extras=True):
+def run_train_ours(args, rank, world, local, cfg=None, sync_bn=False, extras=True, outputs=None):
+    """`outputs`: a dict that receives the results of the last timed step and the variables it left (see --dump-outputs)."""
     import torch
     import torch.distributed as dist
     import drs_b200
@@ -235,6 +244,15 @@ def run_train_ours(args, rank, world, local, cfg=None, sync_bn=False, extras=Tru
         return orig_submit(plan, loss_mask)
 
     be.submit_train = submit
+    last_result = [None]
+    if outputs is not None:
+        orig_result = be.train_result
+
+        def train_result(ticket):
+            last_result[0] = orig_result(ticket)
+            return last_result[0]
+
+        be.train_result = train_result
 
     def barrier():
         if world > 1:
@@ -255,6 +273,17 @@ def run_train_ours(args, rank, world, local, cfg=None, sync_bn=False, extras=Tru
             pipe.flush()
             barrier()
             clocks[0] = sampler.stop() if rank == 0 else None
+            if outputs is not None:
+                # the flush handed over this step's result last; step W+K+1 has not been enqueued, so the prediction buffer
+                # and the variables are still those of step W+K
+                loss, cm, n_correct = last_result[0]
+                c = crops[-1]
+                outputs["train_loss"] = np.array([loss], dtype=np.float64)
+                outputs["train_confusion"] = cm.astype(np.float64)
+                outputs["train_n_correct"] = np.array([n_correct], dtype=np.float64)
+                outputs["train_pred"] = be._pred[:B * c * c].cpu().numpy().astype(np.float32).reshape(B, c, c)
+                for name, v in s.variables().items():
+                    outputs["train_var__" + name.replace("/", "__")] = np.asarray(v, dtype=np.float32)
 
     run_isprs_loop(be, wl, cfg, B * world, niter, hook)
     ms = ev[0].elapsed_time(ev[1])
@@ -553,9 +582,10 @@ def dp_check(s, be, cfg, rank, world, dev, sync_bn):
     return res
 
 
-def run_infer_ours(args, rank, world, local, steps=3, cfg=None):
+def run_infer_ours(args, rank, world, local, steps=3, cfg=None, outputs=None):
     """Full-scene sliding-window inference (isprs:1241-1284), row stripes over the ranks, label map assembled on rank 0.
-    `steps` whole passes are timed one by one (barrier + synchronize on both sides of each); value = median pass."""
+    `steps` whole passes are timed one by one (barrier + synchronize on both sides of each); value = median pass.
+    `outputs`: a dict that receives a fixed sample of the last timed pass's label map (see --dump-outputs)."""
     import torch
     import torch.distributed as dist
     import drs_b200
@@ -604,12 +634,19 @@ def run_infer_ours(args, rank, world, local, steps=3, cfg=None):
         barrier()
         l0 = s.launch_count
         e0.record()
-        one_pass()
+        labels = one_pass()
         e1.record()
         barrier()
         times.append(e0.elapsed_time(e1))
         launches = s.launch_count - l0
     clocks = sampler.stop() if rank == 0 else None
+    if outputs is not None:
+        # the whole map as float32 would exceed the dump's 64 MB: class counts of every pixel plus a fixed seeded sample
+        flat = np.asarray(labels).reshape(-1)
+        idx = np.sort(np.random.RandomState(0).randint(0, flat.size, size=1 << 20))
+        outputs["infer_label_counts"] = np.bincount(flat, minlength=cfg["K"]).astype(np.float64)
+        outputs["infer_labels_sample"] = flat[idx].astype(np.float32)
+        outputs["infer_labels_sample_index"] = idx.astype(np.float64)
     # kernel timing pass (roofline): the same pass once more with a CUDA-event pair around every tensor-core launch
     s.set_profiling(True)
     s.scene_infer(0, cfg["crop"], cfg["batch"], H, W, row_begin=r0, row_end=r1, keep_on_device=True)
@@ -820,6 +857,20 @@ def run_reference(args, rank, world):
     return line
 
 
+DUMP_LIMIT = 64 << 20
+
+
+def write_outputs(path, outputs):
+    """--dump-outputs: one float32 / float64 .npy per array, 64 MB in all at most."""
+    total = sum(a.nbytes for a in outputs.values())
+    if total > DUMP_LIMIT:
+        raise SystemExit("bench.py: %d bytes of outputs exceed the %d-byte dump limit" % (total, DUMP_LIMIT))
+    os.makedirs(path, exist_ok=True)
+    for name, a in outputs.items():
+        assert a.dtype in (np.float32, np.float64), (name, a.dtype)
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -832,10 +883,16 @@ def main():
     ap.add_argument("--no-cli", action="store_true", help="skip the command-line level rate")
     ap.add_argument("--no-extra", action="store_true", help="skip the other BASELINE configs (configs[0], [2], [4], [3] at crop 65)")
     ap.add_argument("--small", action="store_true", help="1500x1500 inference scene (profiling runs)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs dumps the GPU path (--impl ours)")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     rank, world, local = dist_env()
     base = dict(n_gpus=world, steps=args.steps, warmup=args.warmup, higher_is_better=True, vs_baseline=None, data="synthetic")
+    outputs = {} if args.dump_outputs and rank == 0 else None
 
     if args.impl == "reference":
         line = run_reference(args, rank, world)
@@ -853,14 +910,14 @@ def main():
         dist.init_process_group("nccl", device_id=torch.device("cuda", local))
     try:
         if args.workload == "train":
-            line = run_train_ours(args, rank, world, local)
+            line = run_train_ours(args, rank, world, local, outputs=outputs)
             if world > 1 and not args.no_secondary:
                 # the parity mode of data parallelism (SURVEY 8e): BN statistics over the global batch, forward and backward
                 sb = run_train_ours(args, rank, world, local, sync_bn=True, extras=False)
                 line["sync_bn"] = {k: sb[k] for k in ("value", "unit", "ms_per_step", "gpu_launches")}
-            second = None if args.no_secondary else run_infer_ours(args, rank, world, local)
+            second = None if args.no_secondary else run_infer_ours(args, rank, world, local, outputs=outputs)
         else:
-            line = run_infer_ours(args, rank, world, local, steps=max(3, min(args.steps, 5)))
+            line = run_infer_ours(args, rank, world, local, steps=args.steps, outputs=outputs)
             second = None
         if rank == 0:
             base.update(line)
@@ -879,6 +936,8 @@ def main():
                 base["cpu_baseline"] = cpu_train_baseline(8, 2) if args.workload == "train" else cpu_infer_baseline()
                 if second is not None:
                     base["inference"]["cpu_baseline"] = cpu_infer_baseline()
+            if outputs is not None:
+                write_outputs(args.dump_outputs, outputs)
             print(json.dumps(base), flush=True)
     finally:
         if world > 1:
