@@ -38,8 +38,6 @@ struct ConvTcParams {
                       // filter slice per K block (two accumulators), see ConvSched
   int stages;         // smem pipeline depth
   int kps;            // K blocks (BLOCK_K channels of one tap) per pipeline stage: one barrier round trip per kps blocks
-  int dual;           // experiment (off, see CONV_TC_DUAL_MAX_CO): two MMA-issuing warps, even / odd stages of a tile
-                      // accumulate into two TMEM accumulators that the epilogue adds
   int acc_stride;     // TMEM columns of one accumulator
   int tmem_cols;      // allocated TMEM columns (power of two >= 32)
   int act;
@@ -169,7 +167,7 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
       ptx::mbar_init(&empty_bar[s], 1);
     }
     for (int s = 0; s < 2; ++s) {
-      ptx::mbar_init(&tmem_full[s], p.dual ? 2 : 1);   // one commit per issuing warp
+      ptx::mbar_init(&tmem_full[s], 1);    // one commit by the MMA issuer
       ptx::mbar_init(&tmem_empty[s], 4);   // one arrive per epilogue warp
     }
     ptx::fence_barrier_init();
@@ -272,73 +270,63 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
       p.diag[7] = static_cast<uint32_t>(t_exp);
       p.diag[8] = static_cast<uint32_t>(t_tma);
     }
-  } else if (warp == 1 || (warp == 2 && p.dual)) {
+  } else if (warp == 1) {
     // ------------------------------------------------------------------ MMA issuer (convergent warp, elected lane issues)
-    // dual mode: warp 1 takes the even stages of every tile, warp 2 the odd ones, each into its own accumulator (the
-    // assignment depends on the stage index inside the tile only, so the summation order of a pixel never depends on
-    // where its tile runs: results stay batch-invariant and run-to-run identical)
-    {
-      const int pipe = warp == 1 ? 0 : 1;
-      const bool leader = ptx::elect_one_sync();
-      uint32_t soff = 0, boff = 0, phase = 0;
-      int as = 0;
-      uint32_t aphase = 0;
-      long long t_begin = 0, t_wait = 0, t_wait_acc = 0, t_mma = 0, t_commit = 0;
-      if (INSTR) t_begin = clock64();
-      // descriptor words: low = address >> 4 | LBO(16 B) << 16, high = SBO >> 4 | version | layout
-      const uint32_t desc_lo0 = ((smem_base >> 4) & 0x3FFFu) | (1u << 16);
-      const uint32_t desc_hi = ((OP_SBO >> 4) & 0x3FFFu) | (1u << 14) | (OP_LAYOUT << 29);
-      const uint32_t kb_step = static_cast<uint32_t>(kb_bytes) >> 4;
-      const int acc_per_stage = p.dual ? 2 : p.mt;
-      for (int it = 0; it < sched.iters; ++it) {
-        bool two;
-        (void)sched.unit(it, two);
-        if (INSTR) {
-          const long long t0 = clock64();
-          ptx::mbar_wait(&tmem_empty[as], aphase ^ 1, p.diag, 0x200 + as);
-          t_wait_acc += clock64() - t0;
-        } else {
-          ptx::mbar_wait(&tmem_empty[as], aphase ^ 1, p.diag, 0x200 + as);
-        }
-        const uint32_t d_tmem = tmem_base + static_cast<uint32_t>((as * acc_per_stage + (p.dual ? pipe : 0)) * p.acc_stride);
-        uint32_t fresh = 0;                                  // 0 until this warp's first MMA of the tile (overwrites D)
-        int g = 0;
-        for (int kb0 = 0; kb0 < num_kb; kb0 += p.kps, ++g) {
-          if (!p.dual || (g & 1) == pipe) {
-            const int nk = min(p.kps, num_kb - kb0);
-            long long t0 = 0, t1 = 0, t2 = 0;
-            if (INSTR) t0 = clock64();
-            ptx::mbar_wait_addr(full0 + boff, phase, p.diag, 0x300);
-            ptx::tcgen05_fence_after();
-            if (INSTR) { t1 = clock64(); t_wait += t1 - t0; }
-            if (leader && !no_mma) {
-              uint32_t a_lo = desc_lo0 + (soff >> 4);
-              for (int j = 0; j < nk; ++j, a_lo += kb_step) {
-                const uint32_t b_lo = a_lo + (static_cast<uint32_t>(a_bytes) >> 4);
-                ptx::umma_f16_kblock<BLOCK_K / 16>(d_tmem, a_lo, b_lo, desc_hi, p.idesc, fresh);
-                if (two)      // the pair's second unit: same filter slice, its own accumulator
-                  ptx::umma_f16_kblock<BLOCK_K / 16>(d_tmem + p.acc_stride, a_lo + (A_BYTES >> 4), b_lo, desc_hi, p.idesc, fresh);
-                fresh = 1;
-              }
-            }
-            if (INSTR) { t2 = clock64(); t_mma += t2 - t1; }
-            if (leader) ptx::umma_commit_addr(empty0 + boff);   // frees the smem slot when these MMAs retire
-            if (INSTR) t_commit += clock64() - t2;
+    const bool leader = ptx::elect_one_sync();
+    uint32_t soff = 0, boff = 0, phase = 0;
+    int as = 0;
+    uint32_t aphase = 0;
+    long long t_begin = 0, t_wait = 0, t_wait_acc = 0, t_mma = 0, t_commit = 0;
+    if (INSTR) t_begin = clock64();
+    // descriptor words: low = address >> 4 | LBO(16 B) << 16, high = SBO >> 4 | version | layout
+    const uint32_t desc_lo0 = ((smem_base >> 4) & 0x3FFFu) | (1u << 16);
+    const uint32_t desc_hi = ((OP_SBO >> 4) & 0x3FFFu) | (1u << 14) | (OP_LAYOUT << 29);
+    const uint32_t kb_step = static_cast<uint32_t>(kb_bytes) >> 4;
+    for (int it = 0; it < sched.iters; ++it) {
+      bool two;
+      (void)sched.unit(it, two);
+      if (INSTR) {
+        const long long t0 = clock64();
+        ptx::mbar_wait(&tmem_empty[as], aphase ^ 1, p.diag, 0x200 + as);
+        t_wait_acc += clock64() - t0;
+      } else {
+        ptx::mbar_wait(&tmem_empty[as], aphase ^ 1, p.diag, 0x200 + as);
+      }
+      const uint32_t d_tmem = tmem_base + static_cast<uint32_t>(as * p.mt * p.acc_stride);
+      uint32_t fresh = 0;                                  // 0 until the first MMA of the tile (overwrites D)
+      for (int kb0 = 0; kb0 < num_kb; kb0 += p.kps) {
+        const int nk = min(p.kps, num_kb - kb0);
+        long long t0 = 0, t1 = 0, t2 = 0;
+        if (INSTR) t0 = clock64();
+        ptx::mbar_wait_addr(full0 + boff, phase, p.diag, 0x300);
+        ptx::tcgen05_fence_after();
+        if (INSTR) { t1 = clock64(); t_wait += t1 - t0; }
+        if (leader && !no_mma) {
+          uint32_t a_lo = desc_lo0 + (soff >> 4);
+          for (int j = 0; j < nk; ++j, a_lo += kb_step) {
+            const uint32_t b_lo = a_lo + (static_cast<uint32_t>(a_bytes) >> 4);
+            ptx::umma_f16_kblock<BLOCK_K / 16>(d_tmem, a_lo, b_lo, desc_hi, p.idesc, fresh);
+            if (two)      // the pair's second unit: same filter slice, its own accumulator
+              ptx::umma_f16_kblock<BLOCK_K / 16>(d_tmem + p.acc_stride, a_lo + (A_BYTES >> 4), b_lo, desc_hi, p.idesc, fresh);
+            fresh = 1;
           }
-          soff += stage_bytes;
-          boff += 8;
-          if (soff == ring_bytes) { soff = 0; boff = 0; phase ^= 1; }
         }
-        if (leader) ptx::umma_commit(&tmem_full[as]);        // accumulator complete -> epilogue
-        if (++as == 2) { as = 0; aphase ^= 1; }
+        if (INSTR) { t2 = clock64(); t_mma += t2 - t1; }
+        if (leader) ptx::umma_commit_addr(empty0 + boff);   // frees the smem slot when these MMAs retire
+        if (INSTR) t_commit += clock64() - t2;
+        soff += stage_bytes;
+        boff += 8;
+        if (soff == ring_bytes) { soff = 0; boff = 0; phase ^= 1; }
       }
-      if (INSTR && pipe == 0 && leader && blockIdx.x == 0 && p.diag) {
-        p.diag[9] = static_cast<uint32_t>(clock64() - t_begin);
-        p.diag[10] = static_cast<uint32_t>(t_wait);
-        p.diag[11] = static_cast<uint32_t>(t_mma);
-        p.diag[12] = static_cast<uint32_t>(t_commit);
-        p.diag[13] = static_cast<uint32_t>(t_wait_acc);
-      }
+      if (leader) ptx::umma_commit(&tmem_full[as]);        // accumulator complete -> epilogue
+      if (++as == 2) { as = 0; aphase ^= 1; }
+    }
+    if (INSTR && leader && blockIdx.x == 0 && p.diag) {
+      p.diag[9] = static_cast<uint32_t>(clock64() - t_begin);
+      p.diag[10] = static_cast<uint32_t>(t_wait);
+      p.diag[11] = static_cast<uint32_t>(t_mma);
+      p.diag[12] = static_cast<uint32_t>(t_commit);
+      p.diag[13] = static_cast<uint32_t>(t_wait_acc);
     }
   } else if (warp >= 4) {
     // ------------------------------------------------------------------ epilogue
@@ -356,7 +344,6 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
     float st0[STAT_MAX_CHUNKS], st1[STAT_MAX_CHUNKS];      // this thread's (channel, row group) sums, per output chunk
 #pragma unroll
     for (int q = 0; q < STAT_MAX_CHUNKS; ++q) { st0[q] = 0.0f; st1[q] = 0.0f; }
-    const int acc_per_stage = p.dual ? 2 : p.mt;
     for (int it = 0; it < sched.iters; ++it) {
       bool two;
       const int unit0 = sched.unit(it, two);
@@ -365,23 +352,12 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
       for (int sub = 0; sub < (two ? 2 : 1); ++sub) {
       const int tile = unit0 + sub;                // 128-pixel unit of this accumulator
       const uint32_t t_row = tmem_base + (static_cast<uint32_t>(quad * 32) << 16) +
-                             static_cast<uint32_t>((as * acc_per_stage + sub) * p.acc_stride);
+                             static_cast<uint32_t>((as * p.mt + sub) * p.acc_stride);
       for (int ch = 0; ch < ((p.exp_mode == 4 || p.exp_mode == 10) ? 0 : n_chunks); ++ch) {
         uint32_t v[EPI_C];
         ptx::tmem_ld_32x32b_x32(t_row + ch * EPI_C, v);
         if (EPI_C == 64) ptx::tmem_ld_32x32b_x32(t_row + ch * EPI_C + 32, v + (EPI_C == 64 ? 32 : 0));
         ptx::tmem_wait_ld();
-        if (p.dual) {
-          // second accumulator (odd stages): even + odd, always in this order
-#pragma unroll
-          for (int hf = 0; hf < EPI_C / 32; ++hf) {
-            uint32_t w[32];
-            ptx::tmem_ld_32x32b_x32(t_row + p.acc_stride + ch * EPI_C + hf * 32, w);
-            ptx::tmem_wait_ld();
-#pragma unroll
-            for (int i = 0; i < 32; ++i) v[hf * 32 + i] = __float_as_uint(__uint_as_float(v[hf * 32 + i]) + __uint_as_float(w[i]));
-          }
-        }
         // the TMA store that last read staging buffer `sbuf` (two chunks ago) must have drained
         if (warp == 4 && ptx::elect_one_sync()) ptx::tma_store_wait_read<1>();
         asm volatile("bar.sync 1, 128;" ::: "memory");
@@ -579,32 +555,14 @@ static void encode_im2col(Handle* h, CUtensorMap* tm, int etype, const void* bas
 }
 
 static int g_conv_exp_mode = -1;   // drs_bench_conv override of DRS_EXP_MODE
-#ifndef CONV_TC_DUAL_MAX_CO
-// Two MMA-issuing warps (experiment, OFF): after the issue-path fixes the Co <= 128 layers are bound by L2 -> SM operand
-// traffic (16-19 TB/s), so a second issuing warp buys 8 % on N=64 and nothing on N=128 (profiles/r1b_conv_dual_issuer.txt),
-// and a batch-64 DenseDilated6 training step dead-locked with it.  Reachable only through experiment bit 18.
-#define CONV_TC_DUAL_MAX_CO 0
-#endif
 #ifndef CONV_TC_KPS2_MAX_CO
 #define CONV_TC_KPS2_MAX_CO 128      // two K blocks per stage for Co <= this
 #endif
 
-// two CTAs per SM for the small-N layers (DRS_CONV_2CTA=0 turns it off, =128 extends it to Co <= 128).  Measured per
-// 0.76 M-pixel chunk (profiles/r2_conv_two_cta.txt): N=32 161 -> 119 us, N=64 208 -> 190 / 138 -> 130 / 253 -> 237 us; at
-// N=128 the halved shared memory leaves only two 32 KB K blocks in flight per CTA and it loses (184 -> 199, 341 -> 371 us).
-static inline bool conv_tc_two_cta(int co) {
-  static const int lim = getenv("DRS_CONV_2CTA") ? atoi(getenv("DRS_CONV_2CTA")) : 64;
-  return co <= (lim == 1 ? 64 : lim);
-}
-
-// Pairs of 128-pixel units on one filter slice (mt = 2) for Co <= this (DRS_CONV_M2=0 turns it off).  The Co <= 128 layers
-// are bound by the bytes an SM takes in per MMA (an im2col K block is 16 KB of A plus Co*128 B of B for 128*64*Co MACs);
-// two units per filter slice cut them from 24 to 20 KB per unit (Co = 64) and from 32 to 24 KB (Co = 128).  Needs
-// 4 * acc_stride <= 512 TMEM columns, hence not above 128.
-static inline int conv_tc_m2_max_co() {
-  static const int lim = getenv("DRS_CONV_M2") ? atoi(getenv("DRS_CONV_M2")) : 128;
-  return lim > 128 ? 128 : lim;
-}
+// two CTAs per SM for the small-N layers.  Measured per 0.76 M-pixel chunk (profiles/r2_conv_two_cta.txt): N=32 161 -> 119 us,
+// N=64 208 -> 190 / 138 -> 130 / 253 -> 237 us; at N=128 the halved shared memory leaves only two 32 KB K blocks in flight
+// per CTA and it loses (184 -> 199, 341 -> 371 us).
+static inline bool conv_tc_two_cta(int co) { return co <= 64; }
 
 template <int BLOCK_K, int EPI_C, typename OutT>
 static void launch_conv_tc_t(Handle* h, const ConvTcArgs& a) {
@@ -612,7 +570,7 @@ static void launch_conv_tc_t(Handle* h, const ConvTcArgs& a) {
   const int64_t M = (int64_t)a.B * a.crop * a.crop;
   const int taps = a.k * a.k;
   const int sw_op = BLOCK_K * 2;
-  // experiment word: bits 0-7 timing mode, bits 12-15 K blocks per stage (0 = default), bit 16 instrumented twin, bit 18 dual MMA warps,
+  // experiment word: bits 0-7 timing mode, bits 12-15 K blocks per stage (0 = default), bit 16 instrumented twin,
   // bits 20-21 tile pairing (1 = single units, 2 = pairs)
   const int exp_word = g_conv_exp_mode >= 0 ? g_conv_exp_mode : (getenv("DRS_EXP_MODE") ? atoi(getenv("DRS_EXP_MODE")) : 0);
   const int exp_mode = exp_word & 0xff;
@@ -646,11 +604,12 @@ static void launch_conv_tc_t(Handle* h, const ConvTcArgs& a) {
   p.exp_mode = exp_mode;
   if (a.stats) p.stats = *a.stats; else memset(&p.stats, 0, sizeof(p.stats));
 
-  const int dual_max_co = ((exp_word >> 18) & 1) ? 128 : CONV_TC_DUAL_MAX_CO;   // experiment bit 18: dual MMA warps for Co <= 128
-  const bool dual_wanted = a.co <= dual_max_co;
-  // experiment bits 20-21: 1 = force single units, 2 = force pairs (Co <= 128)
+  // Pairs of 128-pixel units on one filter slice (mt = 2) for Co <= 128.  These layers are bound by the bytes an SM takes in
+  // per MMA (an im2col K block is 16 KB of A plus Co*128 B of B for 128*64*Co MACs); two units per filter slice cut them from
+  // 24 to 20 KB per unit (Co = 64) and from 32 to 24 KB (Co = 128).  Needs 4 * acc_stride <= 512 TMEM columns, hence not
+  // above 128.  Experiment bits 20-21: 1 = force single units, 2 = force pairs.
   const int m2_force = (exp_word >> 20) & 3;
-  const int mt = (!dual_wanted && a.co <= 128 && M > CONV_TC_BM && (m2_force == 2 || (m2_force == 0 && a.co <= conv_tc_m2_max_co()))) ? 2 : 1;
+  const int mt = (a.co <= 128 && M > CONV_TC_BM && (m2_force == 0 || m2_force == 2)) ? 2 : 1;
   if (mt == 2 && !((exp_word >> 12) & 0xf)) kps = 1;                 // a pair is already two im2col tiles per barrier round
   if (kps > taps_kb) kps = taps_kb;
   const int kb_bytes = mt * CONV_TC_BM * BLOCK_K * 2 + a.co * BLOCK_K * 2;
@@ -670,9 +629,8 @@ static void launch_conv_tc_t(Handle* h, const ConvTcArgs& a) {
   DRS_CHECK(stages >= 2, "conv_tc: tile does not fit shared memory (co=%d)", a.co);
   p.stages = stages;
   p.kps = kps;
-  p.dual = (dual_wanted && (taps_kb + kps - 1) / kps >= 2) ? 1 : 0;
   p.mt = mt;
-  p.tmem_cols = (p.dual ? 4 : 2 * mt) * p.acc_stride;
+  p.tmem_cols = 2 * mt * p.acc_stride;
   p.smem_needed = fixed + stages * stage_bytes;
   const int smem_bytes = p.smem_needed + 1024 <= budget ? p.smem_needed + 1024 : budget;
   p.smem_provided = smem_bytes;

@@ -196,8 +196,8 @@ struct HandleExtra {
   cudaEvent_t ev_x8 = nullptr;          // conv1's padded input is ready: the side stream builds the im2col matrix under the forward
   bool use_graphs = false;          // opt-in (DRS_GRAPHS=1): measured 6-9 % per step in steady state, see DESIGN.md
   double conv_ms_acc = 0;            // device time of profiled launches already read back
-  InferLane lanes[2];             // scene-inference lanes (drs_scene_api.cuh)
-  cudaEvent_t lanes_ready = nullptr;
+  InferLane lane;                 // scene-inference lane (drs_scene_api.cuh)
+  cudaEvent_t lane_ready = nullptr;
   // streamed scene upload (drs_scene_infer_host): copy stream + "rows uploaded" event
   cudaStream_t copy_stream = nullptr;
   cudaEvent_t up_ev[1] = {nullptr};
@@ -252,7 +252,7 @@ static void* slot_buf(Handle* h, int slot, size_t bytes) {
   }
   return x->slot_ptr[slot];
 }
-static void lanes_release(Handle* h);
+static void lane_release(Handle* h);
 static void pass_geometry_release(Handle* h);
 
 static void free_packed(Handle* h) {
@@ -400,7 +400,7 @@ extern "C" int drs_destroy(drs_handle_t h) {
       if (x->ev_dz[i]) cudaEventDestroy(x->ev_dz[i]);
       if (x->ev_wgrad[i]) cudaEventDestroy(x->ev_wgrad[i]);
     }
-    lanes_release(h);
+    lane_release(h);
     for (int i = 0; i < 8; ++i)
       if (x->slot_ptr[i]) cudaFree(x->slot_ptr[i]);
     for (auto& kv : x->graphs) {

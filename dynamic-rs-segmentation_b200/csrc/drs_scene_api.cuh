@@ -375,47 +375,43 @@ extern "C" int drs_accumulate_argmax(drs_handle_t h, const float* logits_dev, co
   API_END
 }
 
-// Two lanes (stream + workspace each) alternate over the chunks of a scene: while lane A's tensor-core convolutions
-// run, lane B's HBM-bound kernels (gather, pooling, classifier) fill the rest of the machine.  The ordered
-// accumulation stays on the handle's stream, chunk after chunk, so per-pixel sums keep the script's visiting order.
-// Lanes are kept in the handle between calls (their workspace is several GB for a Potsdam tile).
-static void lanes_release(Handle* h) {
+// The chunks of a scene run on a lane of their own (stream + workspace); the ordered accumulation stays on the handle's
+// stream, chunk after chunk, so per-pixel sums keep the script's visiting order.  The lane is kept in the handle between
+// calls (its workspace is several GB for a Potsdam tile).
+static void lane_release(Handle* h) {
   HandleExtra* x = X(h);
-  for (auto& L : x->lanes) {
-    if (L.stream) { cudaStreamSynchronize(L.stream); cudaStreamDestroy(L.stream); }
+  InferLane& L = x->lane;
+  if (L.stream) { cudaStreamSynchronize(L.stream); cudaStreamDestroy(L.stream); }
+  if (L.arena.base) cudaFree(L.arena.base);
+  if (L.x) cudaFree(L.x);
+  if (L.lg) cudaFree(L.lg);
+  if (L.fwd_done) cudaEventDestroy(L.fwd_done);
+  if (L.acc_done) cudaEventDestroy(L.acc_done);
+  L = InferLane();
+  if (x->lane_ready) cudaEventDestroy(x->lane_ready);
+  x->lane_ready = nullptr;
+}
+static void lane_ensure(Handle* h, size_t arena_bytes, size_t x_bytes, size_t lg_bytes) {
+  HandleExtra* x = X(h);
+  if (!x->lane_ready) CUDA_CHECK(cudaEventCreateWithFlags(&x->lane_ready, cudaEventDisableTiming));
+  InferLane& L = x->lane;
+  if (!L.stream) {
+    CUDA_CHECK(cudaStreamCreateWithFlags(&L.stream, cudaStreamNonBlocking));
+    CUDA_CHECK(cudaEventCreateWithFlags(&L.fwd_done, cudaEventDisableTiming));
+    CUDA_CHECK(cudaEventCreateWithFlags(&L.acc_done, cudaEventDisableTiming));
+  }
+  if (L.arena.cap < arena_bytes || L.x_cap < x_bytes || L.lg_cap < lg_bytes) {
+    CUDA_CHECK(cudaStreamSynchronize(L.stream));
     if (L.arena.base) cudaFree(L.arena.base);
     if (L.x) cudaFree(L.x);
     if (L.lg) cudaFree(L.lg);
-    if (L.fwd_done) cudaEventDestroy(L.fwd_done);
-    if (L.acc_done) cudaEventDestroy(L.acc_done);
-    L = InferLane();
-  }
-  if (x->lanes_ready) cudaEventDestroy(x->lanes_ready);
-  x->lanes_ready = nullptr;
-}
-static void lanes_ensure(Handle* h, int n_lanes, size_t arena_bytes, size_t x_bytes, size_t lg_bytes) {
-  HandleExtra* x = X(h);
-  if (!x->lanes_ready) CUDA_CHECK(cudaEventCreateWithFlags(&x->lanes_ready, cudaEventDisableTiming));
-  for (int l = 0; l < n_lanes; ++l) {
-    InferLane& L = x->lanes[l];
-    if (!L.stream) {
-      CUDA_CHECK(cudaStreamCreateWithFlags(&L.stream, cudaStreamNonBlocking));
-      CUDA_CHECK(cudaEventCreateWithFlags(&L.fwd_done, cudaEventDisableTiming));
-      CUDA_CHECK(cudaEventCreateWithFlags(&L.acc_done, cudaEventDisableTiming));
-    }
-    if (L.arena.cap < arena_bytes || L.x_cap < x_bytes || L.lg_cap < lg_bytes) {
-      CUDA_CHECK(cudaStreamSynchronize(L.stream));
-      if (L.arena.base) cudaFree(L.arena.base);
-      if (L.x) cudaFree(L.x);
-      if (L.lg) cudaFree(L.lg);
-      L.arena = Arena(); L.x = L.lg = nullptr; L.x_cap = L.lg_cap = 0;
-      CUDA_CHECK(cudaMalloc(&L.arena.base, arena_bytes));
-      L.arena.cap = arena_bytes;
-      CUDA_CHECK(cudaMalloc(&L.x, x_bytes));
-      L.x_cap = x_bytes;
-      CUDA_CHECK(cudaMalloc(&L.lg, lg_bytes));
-      L.lg_cap = lg_bytes;
-    }
+    L.arena = Arena(); L.x = L.lg = nullptr; L.x_cap = L.lg_cap = 0;
+    CUDA_CHECK(cudaMalloc(&L.arena.base, arena_bytes));
+    L.arena.cap = arena_bytes;
+    CUDA_CHECK(cudaMalloc(&L.x, x_bytes));
+    L.x_cap = x_bytes;
+    CUDA_CHECK(cudaMalloc(&L.lg, lg_bytes));
+    L.lg_cap = lg_bytes;
   }
 }
 
@@ -447,9 +443,8 @@ static void feed_rows(Handle* h, HostSceneFeed& f, const Scene& sc, int rows_nee
     CUDA_CHECK(cudaEventRecord(x->up_ev[0], x->copy_stream));
     f.recorded = true;
   }
-  // Every consumer waits for the latest "rows uploaded" event, also when this call enqueued nothing: with two lanes the
-  // rows a lane needs may have been enqueued by the OTHER lane's look-ahead, and that lane's stream never saw the event.
-  // (Copies on one stream complete in order, so the latest event covers every earlier piece.)
+  // The consumer waits for the latest "rows uploaded" event (copies on one stream complete in order, so it covers every
+  // earlier piece).
   if (f.recorded) CUDA_CHECK(cudaStreamWaitEvent(consumer, x->up_ev[0], 0));
 }
 
@@ -552,9 +547,6 @@ static void scene_infer_impl(drs_handle_t h, int32_t scene_id, int32_t crop, int
   const int waves = getenv("DRS_CHUNK_WAVES") ? std::max(1, atoi(getenv("DRS_CHUNK_WAVES"))) : 40;
   const int64_t target_tiles = (int64_t)h->sm_count * waves;
   int chunk = (int)std::max<int64_t>(1, std::min<int64_t>(P, (target_tiles * CONV_TC_BM) / pp));
-  // A second lane (DRS_TWO_LANES=1) overlaps one chunk's HBM-bound kernels with the other's convolutions; measured on
-  // B200 it loses (L2 thrash + power cap: 1174 ms vs 979 ms for a 6000x6000 tile), so one lane is the default.
-  const int n_lanes = (P > chunk && getenv("DRS_TWO_LANES")) ? 2 : 1;
   ScenePass sp;
   int32_t* inst_dev = nullptr;
   HandleExtra* hx = X(h);
@@ -564,8 +556,7 @@ static void scene_infer_impl(drs_handle_t h, int32_t scene_id, int32_t crop, int
     h->stream = main_stream;
     h->arena = main_arena;
     cudaStreamSynchronize(main_stream);
-    for (auto& L : hx->lanes)
-      if (L.stream) cudaStreamSynchronize(L.stream);
+    if (hx->lane.stream) cudaStreamSynchronize(hx->lane.stream);
     sp.release();
   };
   try {
@@ -573,17 +564,16 @@ static void scene_infer_impl(drs_handle_t h, int32_t scene_id, int32_t crop, int
     const std::vector<int32_t>& inst = pg.inst;
     inst_dev = (int32_t*)slot_buf(h, 6, std::max<size_t>(inst.size(), 1) * 4);
     CUDA_CHECK(cudaMemcpyAsync(inst_dev, inst.data(), inst.size() * 4, cudaMemcpyHostToDevice, h->stream));
-    refresh_packed(h, false);                       // packed weights / folded BN once, before the lanes start
-    lanes_ensure(h, n_lanes, forward_eval_workspace(h, chunk, crop), (size_t)chunk * pp * C * 4, (size_t)chunk * pp * K * 4);
-    CUDA_CHECK(cudaEventRecord(hx->lanes_ready, main_stream));
-    for (int l = 0; l < n_lanes; ++l) CUDA_CHECK(cudaStreamWaitEvent(hx->lanes[l].stream, hx->lanes_ready, 0));
-    int ci = 0;
-    for (int s0 = 0; s0 < P; s0 += chunk, ++ci) {
-      InferLane& L = hx->lanes[ci % n_lanes];
+    refresh_packed(h, false);                       // packed weights / folded BN once, before the lane starts
+    lane_ensure(h, forward_eval_workspace(h, chunk, crop), (size_t)chunk * pp * C * 4, (size_t)chunk * pp * K * 4);
+    InferLane& L = hx->lane;
+    CUDA_CHECK(cudaEventRecord(hx->lane_ready, main_stream));
+    CUDA_CHECK(cudaStreamWaitEvent(L.stream, hx->lane_ready, 0));
+    for (int s0 = 0; s0 < P; s0 += chunk) {
       const int nb = std::min(chunk, P - s0);
       h->stream = L.stream;
       h->arena = L.arena;
-      if (ci >= n_lanes) CUDA_CHECK(cudaStreamWaitEvent(L.stream, L.acc_done, 0));   // logits buffer consumed
+      if (s0 > 0) CUDA_CHECK(cudaStreamWaitEvent(L.stream, L.acc_done, 0));   // logits buffer of the previous chunk consumed
       if (feed) {
         // rows this chunk's patches read, plus one more chunk's worth so that the copy runs ahead of the compute
         int need = 0;

@@ -15,10 +15,7 @@ __global__ void unpack_extras_kernel(const float* __restrict__ src, float* __res
 __global__ void add2_kernel(const float* __restrict__ a, float* __restrict__ out) { pdl_sync(); out[2] = a[0] + a[1]; }
 
 // blocks per SM of the classifier's filter-gradient kernel (its K-round shared-memory epilogue wants long-lived blocks)
-static int cls_w_blocks_per_sm() {
-  static const int v = getenv("DRS_CLSW_BPSM") ? atoi(getenv("DRS_CLSW_BPSM")) : 2;
-  return v;
-}
+constexpr int CLS_W_BLOCKS_PER_SM = 2;
 
 static size_t train_workspace_bytes(Handle* h, int B, int crop, size_t es) {
   NetDesc& n = h->net;
@@ -49,7 +46,7 @@ static size_t train_workspace_bytes(Handle* h, int B, int crop, size_t es) {
   add((size_t)nb_bn * 2 * 256 * 4);
   const int nb_ce = (int)ceil_div(M, CE_THREADS);
   add((size_t)nb_ce * 4);
-  const int nb_cls = (int)std::min<int64_t>(ceil_div(M, 128), (int64_t)h->sm_count * cls_w_blocks_per_sm());
+  const int nb_cls = (int)std::min<int64_t>(ceil_div(M, 128), (int64_t)h->sm_count * CLS_W_BLOCKS_PER_SM);
   const int cls_rows = (int)ceil_div(M, nb_cls);
   add((size_t)nb_cls * (n.cls_in + 1) * K * 4);
   const int max_splits = 48;
@@ -79,7 +76,7 @@ static void train_step_t(Handle* h, const float* x_dev, const float* y_dev, cons
   const int nb_bn = (int)std::min<int64_t>(ceil_div(M, 128), (int64_t)h->sm_count * DRS_BN_MINBLK);   // one wave of resident blocks
   const int bn_rows = (int)ceil_div(M, nb_bn);
   const int nb_ce = (int)ceil_div(M, CE_THREADS);
-  const int nb_cls = (int)std::min<int64_t>(ceil_div(M, 128), (int64_t)h->sm_count * cls_w_blocks_per_sm());
+  const int nb_cls = (int)std::min<int64_t>(ceil_div(M, 128), (int64_t)h->sm_count * CLS_W_BLOCKS_PER_SM);
   const int cls_rows = (int)ceil_div(M, nb_cls);
   const int max_splits = 48;
   size_t max_w = 0;
@@ -157,8 +154,7 @@ static void train_step_t(Handle* h, const float* x_dev, const float* y_dev, cons
     if (n.dense) return ActBuf{F, n.feat_stride, c.out_coff};
     return ActBuf{Xn[l], c.out_cs > 0 ? c.out_cs : c.co, c.out_cs > 0 ? c.out_coff : 0};
   };
-  const bool conv1_on_tc = ElemTag<TA>::v == ET_BF16 && !getenv("DRS_NO_CONV1_TC_TRAIN") &&
-                           conv1_tc_supported(n.convs[0].k, n.convs[0].rate, n.convs[0].ci, n.convs[0].co);
+  const bool conv1_on_tc = ElemTag<TA>::v == ET_BF16 && conv1_tc_supported(n.convs[0].k, n.convs[0].rate, n.convs[0].ci, n.convs[0].co);
   // conv1's filter gradient on the tensor cores needs the (bf16) im2col matrix of the input: built next to the forward
   const bool wgrad1_on_tc = conv1_on_tc && 25 * n.convs[0].ci <= 128 && wgrad_tc_supported(128, n.convs[0].co) && !getenv("DRS_NO_WGRAD_CONV1_TC");
   TA* xcol = nullptr;
@@ -172,8 +168,7 @@ static void train_step_t(Handle* h, const float* x_dev, const float* y_dev, cons
     float* istd = x->inv_std + c.mm_off;
     BnFinish fin{x->bn_acc, 1048576.0, x->bn_counter, x->sums, nullptr, nullptr, nullptr, nullptr, bn_count, h->cfg.bn_eps, h->cfg.bn_decay, h->cfg.bn_unbiased_ema};
     if (!h->sync_bn) { fin.mean = mean; fin.inv_std = istd; fin.mov_mean = h->bnstat + c.mm_off; fin.mov_var = h->bnstat + c.mv_off; }
-    const bool fused_stats = (l > 0 || (conv1_on_tc && !getenv("DRS_NO_FUSED_STATS_CONV1"))) && ElemTag<TA>::v != ET_F32 &&
-                             !getenv("DRS_NO_FUSED_STATS");
+    const bool fused_stats = (l > 0 || conv1_on_tc) && ElemTag<TA>::v != ET_F32;
     if (l == 0 && conv1_on_tc) {
       // conv1 on the tensor cores as in inference (conv1_tc.cuh): input and filter rounded to bf16 like every other layer's
       // operands; the filter is re-packed every step (13 K elements).  The filter gradient keeps the fp32 input.
@@ -307,11 +302,10 @@ static void train_step_t(Handle* h, const float* x_dev, const float* y_dev, cons
   std::vector<char> grad_written(L, 0);        // squeeze: has the gradient buffer led by layer g been written in this step?
   {
     const int cvc = n.cls_in / 8;
-    if (cvc <= 256 && ElemTag<TA>::v != ET_F32 && !getenv("DRS_NO_CLS_REG")) {
+    if (cvc <= 256 && ElemTag<TA>::v != ET_F32) {
       const int rows = 256 / cvc;
-      // few, long-lived blocks: a thread first loads its 8 x K weights (48 scalar loads), which must be amortised
-      static const int cls_bpsm = getenv("DRS_CLS_BPSM") ? atoi(getenv("DRS_CLS_BPSM")) : 2;
-      int blocks = (int)std::min<int64_t>(ceil_div(M, 2 * rows), (int64_t)h->sm_count * cls_bpsm);
+      // few, long-lived blocks (two per SM): a thread first loads its 8 x K weights (48 scalar loads), which must be amortised
+      int blocks = (int)std::min<int64_t>(ceil_div(M, 2 * rows), (int64_t)h->sm_count * 2);
       launch_pdl(h, classifier_bwd_data_reg_kernel<TA>, dim3(blocks), dim3(256), 0, dlogits, h->params + n.cls_w_off, K, Gcur, gcs0, 0, n.cls_in, M);
     } else {
       int blocks = (int)std::min<int64_t>(ceil_div(M * (n.cls_in / 8), 256), (int64_t)h->sm_count * 16);
@@ -329,16 +323,12 @@ static void train_step_t(Handle* h, const float* x_dev, const float* y_dev, cons
     float* mean = x->mean + c.mm_off;
     float* istd = x->inv_std + c.mm_off;
     BnFinish finb{x->bn_acc, 1099511627776.0, x->bn_counter, x->sums, nullptr, nullptr, nullptr, nullptr, bn_count, 0.0f, 0.0f, 0};
-    // Experiment (off): the pool backward can also reduce the BN-backward sums of the dIn it produces (one pass over Z
-    // and dIn less per layer).  Measured slower: the pool backward is issue-bound already and the extra registers cost it
-    // a resident CTA (batch 64: crop 37 1.684 vs 1.643 ms/step, crop 49 2.586 vs 2.515).
-    const bool fused_bwd_stats = n.pool && ElemTag<TA>::v == ET_BF16 && getenv("DRS_FUSED_BWD_STATS");
     // Pooling nets, bf16: two passes instead of four.  The BN-backward sums are taken on the pooled side (window gradients
     // and pooled activations: bn_partial_kernel MODE 2), then ONE kernel scatters the window gradients to their winners and
     // applies the BN backward to the finished fp32 row: the pool's input gradient is never written (it used to be stored as
     // bf16, read by the statistics pass and read again by bn_bwd_apply_kernel).
     const bool fused_pool_apply = n.pool && !n.dense && !n.squeeze && c.post == 0 && ElemTag<TA>::v == ET_BF16 && c.co <= 512 &&
-                                  pool_lean_enabled() && !x->debug_keep && !fused_bwd_stats && !getenv("DRS_NO_FUSED_POOL_APPLY");
+                                  pool_lean_enabled() && !x->debug_keep && !getenv("DRS_NO_FUSED_POOL_APPLY");
     if (fused_pool_apply) {
       launch_pdl(h, bn_partial_kernel<TA, TA, 2>, dim3(nb_bn), dim3(BN_THREADS), 0, (const TA*)Xn[l], c.co, 0, (const TA*)dOut.p, dOut.cs, dOut.co,
                  (const float*)mean, (const float*)istd, n.act, part_bn, c.co, M, bn_rows, finb);
@@ -347,14 +337,13 @@ static void train_step_t(Handle* h, const float* x_dev, const float* y_dev, cons
       TA* DZf = DZb[l & 1];
       if (l + 2 <= L - 1) {
         CUDA_CHECK(cudaStreamWaitEvent(h->stream, x->ev_wgrad[l & 1], 0));
-        if (!getenv("DRS_PDL_ACROSS_EVENTS")) h->pdl_prev = false;
+        h->pdl_prev = false;
       }
       launch_maxpool3_bwd_apply(h, (const __nv_bfloat16*)dOut.p, dOut.cs, dOut.co, idx[l], (__nv_bfloat16*)DZf, c.co, 0, c.co, B, crop,
                                 (const __nv_bfloat16*)Z[l], mean, istd, x->sums, 1.0 / bn_count, n.act);
     } else {
     if (n.pool) {
-      if (fused_bwd_stats) launch_maxpool3_bwd<TA>(h, (const TA*)dOut.p, dOut.cs, dOut.co, idx[l], T, c.co, 0, c.co, B, crop, &finb, Z[l], mean, istd, n.act);
-      else launch_maxpool3_bwd<TA>(h, (const TA*)dOut.p, dOut.cs, dOut.co, idx[l], T, c.co, 0, c.co, B, crop);
+      launch_maxpool3_bwd<TA>(h, (const TA*)dOut.p, dOut.cs, dOut.co, idx[l], T, c.co, 0, c.co, B, crop);
       dA = ActBuf{T, c.co, 0};
     }
     if (c.post == 1) {
@@ -379,11 +368,9 @@ static void train_step_t(Handle* h, const float* x_dev, const float* y_dev, cons
       LAUNCH_CHECK(h);
       dA = ActBuf{T, c.co, 0};
     }
-    if (!fused_bwd_stats) {
-      launch_pdl(h, bn_partial_kernel<TA, TA, 1>, dim3(nb_bn), dim3(BN_THREADS), 0, (const TA*)Z[l], c.co, 0, (const TA*)dA.p, dA.cs, dA.co,
-                 (const float*)mean, (const float*)istd, n.act, part_bn, c.co, M, bn_rows, finb);
-      LAUNCH_CHECK(h);
-    }
+    launch_pdl(h, bn_partial_kernel<TA, TA, 1>, dim3(nb_bn), dim3(BN_THREADS), 0, (const TA*)Z[l], c.co, 0, (const TA*)dA.p, dA.cs, dA.co,
+               (const float*)mean, (const float*)istd, n.act, part_bn, c.co, M, bn_rows, finb);
+    LAUNCH_CHECK(h);
     if (h->sync_bn) do_allreduce(h, x->sums, 2 * c.co);
     // The filter gradient of layer l is off the critical path (only the optimizer needs it): it runs on a side stream and
     // overlaps the HBM-bound kernels of layer l-1's backward.  dZ is double-buffered; before a buffer is rewritten the
@@ -391,7 +378,7 @@ static void train_step_t(Handle* h, const float* x_dev, const float* y_dev, cons
     TA* DZ = DZb[l & 1];
     if (l + 2 <= L - 1) {
       CUDA_CHECK(cudaStreamWaitEvent(h->stream, x->ev_wgrad[l & 1], 0));
-      if (!getenv("DRS_PDL_ACROSS_EVENTS")) h->pdl_prev = false;       // the next kernel also depends on another stream
+      h->pdl_prev = false;                 // the next kernel also depends on another stream
     }
     launch_pdl(h, bn_bwd_apply_kernel<TA, TA>, dim3(bne_grid(M, h->sm_count)), dim3(BNE_THREADS), 0, (const TA*)Z[l], c.co, 0, (const TA*)dA.p, dA.cs,
                dA.co, (const float*)mean, (const float*)istd, (const float*)x->sums, 1.0 / bn_count, n.act, DZ, c.co, 0, c.co, M);
@@ -421,7 +408,7 @@ static void train_step_t(Handle* h, const float* x_dev, const float* y_dev, cons
       } else if (l == 0) {
         // conv1: K = 25*C <= 125 rows only -> parallelism must come from many short pixel splits
         // (fp32 mode keeps the generic kernel: its summation order is what the fp32 parity tests pin)
-        const bool fast1 = ElemTag<TA>::v != ET_F32 && !getenv("DRS_NO_WGRAD_CONV1") &&
+        const bool fast1 = ElemTag<TA>::v != ET_F32 &&
                            launch_wgrad_conv1<TA>(h, x_dev, n.channels, DZ, c.co, 0, c.co, h->grads + c.w_off, part_w, max_w * max_splits, B, crop, c.k, c.rate);
         if (!fast1) {
           const int conv1_splits = (int)std::min<int64_t>((int64_t)(max_w * max_splits) / ((int64_t)c.k * c.k * c.ci * c.co), 4 * h->sm_count);
@@ -540,7 +527,7 @@ static void train_step(Handle* h, const float* x_dev, const float* y_dev, const 
   TrainGraph* replay = nullptr;
   // (the legacy default stream cannot be captured)
   // (data parallel: capturable only when the exchange is the in-library NCCL call, not a host callback)
-  const bool graphable = x->use_graphs && (h->world <= 1 || x->nccl) && !getenv("DRS_DEBUG_KEEP") && !getenv("DRS_NO_GRAPHS") &&
+  const bool graphable = x->use_graphs && (h->world <= 1 || x->nccl) && !getenv("DRS_DEBUG_KEEP") &&
                          h->cfg.precision != DRS_PREC_F16 && h->stream != nullptr;
   if (!graphable) {
     if (capture_only) return;

@@ -32,7 +32,7 @@ struct alignas(16) Vec8 {
 // the horizontal 3-max of the two previous rows in registers, so every input element is loaded 3 times (from L1)
 // instead of 9.  Adjacent threads cover adjacent channel groups, then adjacent columns: each row access of a warp is
 // one contiguous run.
-template <typename T, bool WITH_IDX>
+template <typename T>
 __device__ __forceinline__ void pool_row_max(const T* __restrict__ in, int in_cs, int64_t pix_row0, int x, int crop, int y,
                                              float (&v)[8], int (&d)[8]) {
 #pragma unroll
@@ -46,12 +46,12 @@ __device__ __forceinline__ void pool_row_max(const T* __restrict__ in, int in_cs
 #pragma unroll
     for (int e = 0; e < 8; ++e) {
       const float f = to_f32(q.v[e]);
-      if (f > v[e]) { v[e] = f; if (WITH_IDX) d[e] = dx + 1; }
+      if (f > v[e]) { v[e] = f; d[e] = dx + 1; }
     }
   }
 }
 
-template <typename T, bool WITH_IDX, bool FUSE_BN>
+template <typename T>
 __global__ void __launch_bounds__(256)
 maxpool3_fwd_kernel(const T* __restrict__ in, int in_cs, int in_co, T* __restrict__ out, int out_cs, int out_co,
                     uint8_t* __restrict__ idx, int C, int B, int crop, int seg, int nseg, const float* __restrict__ bn_mean,
@@ -73,14 +73,12 @@ maxpool3_fwd_kernel(const T* __restrict__ in, int in_cs, int in_co, T* __restric
   // Training forward of the pooling nets: max-pool commutes with the (strictly increasing) normalise + LeakyReLU, so the
   // pool runs on the raw conv output and act((max - mean) * inv_std) is applied to the winner only.
   float mu[8], is[8];
-  if (FUSE_BN) {
 #pragma unroll
-    for (int e = 0; e < 8; ++e) { mu[e] = bn_mean[cg * 8 + e]; is[e] = bn_inv_std[cg * 8 + e]; }
-  }
-  pool_row_max<T, WITH_IDX>(inp, in_cs, img0, x, crop, y0 - 1, r0, d0);
-  pool_row_max<T, WITH_IDX>(inp, in_cs, img0, x, crop, y0, r1, d1);
+  for (int e = 0; e < 8; ++e) { mu[e] = bn_mean[cg * 8 + e]; is[e] = bn_inv_std[cg * 8 + e]; }
+  pool_row_max<T>(inp, in_cs, img0, x, crop, y0 - 1, r0, d0);
+  pool_row_max<T>(inp, in_cs, img0, x, crop, y0, r1, d1);
   for (int y = y0; y < y1; ++y) {
-    pool_row_max<T, WITH_IDX>(inp, in_cs, img0, x, crop, y + 1, r2, d2);
+    pool_row_max<T>(inp, in_cs, img0, x, crop, y + 1, r2, d2);
     Vec8<T> o;
     int code[8];
 #pragma unroll
@@ -90,18 +88,16 @@ maxpool3_fwd_kernel(const T* __restrict__ in, int in_cs, int in_co, T* __restric
       int c = d0[e];
       if (r1[e] > best) { best = r1[e]; c = 3 + d1[e]; }
       if (r2[e] > best) { best = r2[e]; c = 6 + d2[e]; }
-      if (FUSE_BN) best = apply_act((best - mu[e]) * is[e], act);
+      best = apply_act((best - mu[e]) * is[e], act);
       o.v[e] = from_f32<T>(best);
       code[e] = c;
     }
     const int64_t m = img0 + (int64_t)y * crop + x;
     *reinterpret_cast<Vec8<T>*>(out + m * out_cs + out_co + cg * 8) = o;
-    if (WITH_IDX) {
-      uint2 pk;
-      pk.x = code[0] | (code[1] << 8) | (code[2] << 16) | (code[3] << 24);
-      pk.y = code[4] | (code[5] << 8) | (code[6] << 16) | (code[7] << 24);
-      *reinterpret_cast<uint2*>(idx + m * C + cg * 8) = pk;
-    }
+    uint2 pk;
+    pk.x = code[0] | (code[1] << 8) | (code[2] << 16) | (code[3] << 24);
+    pk.y = code[4] | (code[5] << 8) | (code[6] << 16) | (code[7] << 24);
+    *reinterpret_cast<uint2*>(idx + m * C + cg * 8) = pk;
 #pragma unroll
     for (int e = 0; e < 8; ++e) { r0[e] = r1[e]; r1[e] = r2[e]; d0[e] = d1[e]; d1[e] = d2[e]; }
   }
@@ -126,54 +122,13 @@ __device__ __forceinline__ void vmax8(Vec8<__nv_bfloat16>& a, const Vec8<__nv_bf
   for (int e = 0; e < 4; ++e) pa[e] = __hmax2(pa[e], pb[e]);
 }
 
-template <typename T>
-__device__ __forceinline__ bool pool_row_vmax(const T* __restrict__ in, int in_cs, int64_t pix_row0, int x, int crop, int y,
-                                              Vec8<T>& v) {
-  if (y < 0 || y >= crop) return false;
-  const T* row = in + (pix_row0 + (int64_t)y * crop) * in_cs;
-  v = *reinterpret_cast<const Vec8<T>*>(row + (int64_t)x * in_cs);
-  if (x > 0) vmax8(v, *reinterpret_cast<const Vec8<T>*>(row + (int64_t)(x - 1) * in_cs));
-  if (x + 1 < crop) vmax8(v, *reinterpret_cast<const Vec8<T>*>(row + (int64_t)(x + 1) * in_cs));
-  return true;
-}
-
-template <typename T>
-__global__ void __launch_bounds__(256)
-maxpool3_fwd_packed_kernel(const T* __restrict__ in, int in_cs, int in_co, T* __restrict__ out, int out_cs, int out_co, int C,
-                           int B, int crop, int seg, int nseg) {
-  const int cv = C >> 3;
-  const int64_t gid = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (gid >= (int64_t)B * nseg * crop * cv) return;
-  const int cg = (int)(gid % cv);
-  int64_t t = gid / cv;
-  const int x = (int)(t % crop);
-  t /= crop;
-  const int sg = (int)(t % nseg);
-  const int b = (int)(t / nseg);
-  const int y0 = sg * seg, y1 = min(crop, y0 + seg);
-  const int64_t img0 = (int64_t)b * crop * crop;
-  const T* inp = in + in_co + cg * 8;
-  Vec8<T> r0, r1, r2;
-  bool v0 = pool_row_vmax<T>(inp, in_cs, img0, x, crop, y0 - 1, r0);
-  bool v1 = pool_row_vmax<T>(inp, in_cs, img0, x, crop, y0, r1);      // always valid
-  for (int y = y0; y < y1; ++y) {
-    const bool v2 = pool_row_vmax<T>(inp, in_cs, img0, x, crop, y + 1, r2);
-    Vec8<T> o = r1;
-    if (v0) vmax8(o, r0);
-    if (v2) vmax8(o, r2);
-    *reinterpret_cast<Vec8<T>*>(out + (img0 + (int64_t)y * crop + x) * out_cs + out_co + cg * 8) = o;
-    r0 = r1; v0 = v1;
-    r1 = r2; v1 = v2;
-  }
-}
-
-// Two columns per thread, next row's loads in flight (default; DRS_POOL_INFER=1 selects the one-column kernel above).  The one-column kernel above is
-// latency-bound on its reads: a thread has one row of loads outstanding and two of its three 16-byte loads hit L1 (the
-// neighbours' centres), so only 16 unique bytes per thread are on their way from DRAM at any time.  Here a thread owns
-// columns (x0, x0+1): four loads per row for two outputs (x0-1, x0, x0+1, x0+2), three packed maxima for the two horizontal
-// results (the centre pair's maximum is shared), and the loads of row y+2 are issued before row y+1 is reduced.
-// Measured: the seven pools of a 0.76 M-pixel Dilated8Pooling chunk 722 -> ~600 us (5.2 TB/s of read + write traffic, 80 % of
-// the measured HBM peak), the scene pass -3 % (profiles/r2c_conv_pairs_uniform_ab.txt, section 7).  Same bits: max is exact.
+// Two columns per thread, next row's loads in flight.  The reads are latency-bound: with one column per thread a thread
+// has one row of loads outstanding and two of its three 16-byte loads hit L1 (the neighbours' centres), so only 16 unique
+// bytes per thread are on their way from DRAM at any time.  Here a thread owns columns (x0, x0+1): four loads per row for
+// two outputs (x0-1, x0, x0+1, x0+2), three packed maxima for the two horizontal results (the centre pair's maximum is
+// shared), and the loads of row y+2 are issued before row y+1 is reduced.  Measured against the one-column kernel: the
+// seven pools of a 0.76 M-pixel Dilated8Pooling chunk 722 -> ~600 us (5.2 TB/s of read + write traffic, 80 % of the
+// measured HBM peak), the scene pass -3 % (profiles/r2c_conv_pairs_uniform_ab.txt, section 7).  Same bits: max is exact.
 template <typename T>
 __global__ void __launch_bounds__(256)
 maxpool3_fwd_packed2_kernel(const T* __restrict__ in, int in_cs, int in_co, T* __restrict__ out, int out_cs, int out_co, int C,
@@ -238,91 +193,9 @@ maxpool3_fwd_packed2_kernel(const T* __restrict__ in, int in_cs, int in_co, T* _
 
 // Training variant for bf16 (winner codes + fused normalise/activation) on packed 2-wide compare / max / select: a third
 // of the instructions of the scalar float version, same first-maximum semantics (strictly-greater replaces, row-major).
-__device__ __forceinline__ void pool_pk_row(const __nv_bfloat16* __restrict__ in, int in_cs, int64_t pix_row0, int x, int crop,
-                                            int y, __nv_bfloat162 (&rv)[4], unsigned (&ri)[4]) {
-  const unsigned ninf2 = 0xFF80FF80u;
-#pragma unroll
-  for (int w = 0; w < 4; ++w) { rv[w] = *reinterpret_cast<const __nv_bfloat162*>(&ninf2); ri[w] = 0u; }
-  if (y < 0 || y >= crop) return;
-#pragma unroll
-  for (int dx = -1; dx <= 1; ++dx) {
-    const int xx = x + dx;
-    if (xx < 0 || xx >= crop) continue;
-    const uint4 raw = *reinterpret_cast<const uint4*>(in + (pix_row0 + (int64_t)y * crop + xx) * in_cs);
-    const __nv_bfloat162* q = reinterpret_cast<const __nv_bfloat162*>(&raw);
-    const unsigned code2 = (unsigned)(dx + 1) * 0x00010001u;
-#pragma unroll
-    for (int w = 0; w < 4; ++w) {
-      const unsigned m = __hgt2_mask(q[w], rv[w]);
-      rv[w] = __hmax2(rv[w], q[w]);
-      ri[w] = (ri[w] & ~m) | (code2 & m);
-    }
-  }
-}
-
-__global__ void __launch_bounds__(256)
-maxpool3_fwd_train_bf16_kernel(const __nv_bfloat16* __restrict__ in, int in_cs, int in_co, __nv_bfloat16* __restrict__ out,
-                               int out_cs, int out_co, uint8_t* __restrict__ idx, int C, int B, int crop, int seg, int nseg,
-                               const float* __restrict__ bn_mean, const float* __restrict__ bn_inv_std, int act) {
-  const int cv = C >> 3;
-  const int64_t gid = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (gid >= (int64_t)B * nseg * crop * cv) return;
-  const int cg = (int)(gid % cv);
-  int64_t t = gid / cv;
-  const int x = (int)(t % crop);
-  t /= crop;
-  const int sg = (int)(t % nseg);
-  const int b = (int)(t / nseg);
-  const int y0 = sg * seg, y1 = min(crop, y0 + seg);
-  const int64_t img0 = (int64_t)b * crop * crop;
-  const __nv_bfloat16* inp = in + in_co + cg * 8;
-  float mu[8], is[8];
-  if (bn_mean) {
-#pragma unroll
-    for (int e = 0; e < 8; ++e) { mu[e] = bn_mean[cg * 8 + e]; is[e] = bn_inv_std[cg * 8 + e]; }
-  }
-  __nv_bfloat162 v0[4], v1[4], v2[4];
-  unsigned i0[4], i1[4], i2[4];
-  pool_pk_row(inp, in_cs, img0, x, crop, y0 - 1, v0, i0);
-  pool_pk_row(inp, in_cs, img0, x, crop, y0, v1, i1);
-  for (int y = y0; y < y1; ++y) {
-    pool_pk_row(inp, in_cs, img0, x, crop, y + 1, v2, i2);
-    uint4 o;
-    unsigned code[4];
-    unsigned* ow = reinterpret_cast<unsigned*>(&o);
-#pragma unroll
-    for (int w = 0; w < 4; ++w) {
-      __nv_bfloat162 best = v0[w];
-      unsigned bi = i0[w];
-      unsigned m = __hgt2_mask(v1[w], best);
-      best = __hmax2(best, v1[w]);
-      bi = (bi & ~m) | ((i1[w] + 0x00030003u) & m);
-      m = __hgt2_mask(v2[w], best);
-      best = __hmax2(best, v2[w]);
-      bi = (bi & ~m) | ((i2[w] + 0x00060006u) & m);
-      code[w] = bi;
-      if (bn_mean) {
-        const float lo = apply_act((__low2float(best) - mu[2 * w]) * is[2 * w], act);
-        const float hi = apply_act((__high2float(best) - mu[2 * w + 1]) * is[2 * w + 1], act);
-        best = __floats2bfloat162_rn(lo, hi);
-      }
-      ow[w] = *reinterpret_cast<unsigned*>(&best);
-    }
-    const int64_t m = img0 + (int64_t)y * crop + x;
-    *reinterpret_cast<uint4*>(out + m * out_cs + out_co + cg * 8) = o;
-    uint2 pk;
-    pk.x = __byte_perm(code[0], code[1], 0x6420);      // low byte of every 16-bit lane
-    pk.y = __byte_perm(code[2], code[3], 0x6420);
-    *reinterpret_cast<uint2*>(idx + m * C + cg * 8) = pk;
-#pragma unroll
-    for (int w = 0; w < 4; ++w) { v0[w] = v1[w]; v1[w] = v2[w]; i0[w] = i1[w]; i1[w] = i2[w]; }
-  }
-}
-
-// Software-pipelined variant of the kernel above: the three 16-byte loads of window row y+2 are issued before the
-// arithmetic of row y+1 starts, so a thread always has a row of loads in flight (the plain version consumes each row's
-// loads immediately and is latency-bound: 48 % issue utilisation at 17 % DRAM under ncu).  Out-of-image positions load as
-// -inf, which never wins a strictly-greater compare: same first-maximum semantics and codes as pool_pk_row.
+// Software-pipelined: the three 16-byte loads of window row y+2 are issued before the arithmetic of row y+1 starts, so a
+// thread always has a row of loads in flight (consuming each row's loads immediately is latency-bound: 48 % issue
+// utilisation at 17 % DRAM under ncu).  Out-of-image positions load as -inf, which never wins a strictly-greater compare.
 struct PoolRawRow { uint4 q[3]; };
 __device__ __forceinline__ void pool_load_raw(const __nv_bfloat16* __restrict__ in, int in_cs, int64_t pix_row0, int x, int crop,
                                               int y, PoolRawRow& r) {
@@ -457,115 +330,45 @@ __device__ __forceinline__ void pool_bwd_acc(const PoolBwdRow& r, int dy, float 
   }
 }
 
-// STATS: the same pass also reduces the two sums of the batch-norm backward of the layer below the pool,
-//   s0 = sum_m g, s1 = sum_m g * xh,  g = dIn * act'(xh), xh = (z - mean) * inv_std
-// over the (bf16-rounded) dIn it has just produced -- bn_partial_kernel<MODE 1> needs no pass of its own (it re-read Z and
-// dIn: M*C*4 bytes per layer).  Per-thread sums -> fixed-order block sums in shared memory -> 64-bit fixed point -> integer
-// atomics (order-independent), last block publishes them (same protocol as bn_partial_kernel).
-template <bool STATS>
 __global__ void __launch_bounds__(256, DRS_POOL_MINBLK)
 maxpool3_bwd_bf16_kernel(const __nv_bfloat16* __restrict__ dout, int do_cs, int do_co, const uint8_t* __restrict__ idx,
-                         __nv_bfloat16* __restrict__ din, int di_cs, int di_co, int C, int B, int crop, int seg, int nseg,
-                         const __nv_bfloat16* __restrict__ z, const float* __restrict__ mean, const float* __restrict__ inv_std,
-                         int act, BnFinish fin) {
+                         __nv_bfloat16* __restrict__ din, int di_cs, int di_co, int C, int B, int crop, int seg, int nseg) {
   const int cv = C >> 3;
   const int64_t gid = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  const bool live = gid < (int64_t)B * nseg * crop * cv;
-  if (!STATS && !live) return;
+  if (gid >= (int64_t)B * nseg * crop * cv) return;
   const int cg = (int)(gid % cv);
-  float s0[8], s1[8];
-  if (STATS) {
+  int64_t t = gid / cv;
+  const int x = (int)(t % crop);
+  t /= crop;
+  const int sg = (int)(t % nseg);
+  const int b = (int)(t / nseg);
+  const int y0 = sg * seg, y1 = min(crop, y0 + seg);
+  const int64_t img0 = (int64_t)b * crop * crop;
+  const __nv_bfloat16* dp = dout + do_co + cg * 8;
+  const uint8_t* ip = idx + cg * 8;
+  PoolBwdRow ra, rb, rc;                 // window rows y-1, y, y+1
+  pool_bwd_load(dp, do_cs, ip, C, img0, x, crop, y0 - 1, ra);
+  pool_bwd_load(dp, do_cs, ip, C, img0, x, crop, y0, rb);
+  for (int y = y0; y < y1; ++y) {
+    pool_bwd_load(dp, do_cs, ip, C, img0, x, crop, y + 1, rc);
+    float acc[8];
 #pragma unroll
-    for (int e = 0; e < 8; ++e) { s0[e] = 0.0f; s1[e] = 0.0f; }
-  }
-  if (live) {
-    int64_t t = gid / cv;
-    const int x = (int)(t % crop);
-    t /= crop;
-    const int sg = (int)(t % nseg);
-    const int b = (int)(t / nseg);
-    const int y0 = sg * seg, y1 = min(crop, y0 + seg);
-    const int64_t img0 = (int64_t)b * crop * crop;
-    const __nv_bfloat16* dp = dout + do_co + cg * 8;
-    const uint8_t* ip = idx + cg * 8;
-    float mu[8], is[8];
-    if (STATS) {
+    for (int e = 0; e < 8; ++e) acc[e] = 0.0f;
+    // same summation order as the gather formulation: dy = -1 (window row y+1), 0, +1 (window row y-1); dx = -1, 0, +1
+    pool_bwd_acc(rc, -1, acc);
+    pool_bwd_acc(rb, 0, acc);
+    pool_bwd_acc(ra, 1, acc);
+    uint4 o;
+    unsigned* ow = reinterpret_cast<unsigned*>(&o);
 #pragma unroll
-      for (int e = 0; e < 8; ++e) { mu[e] = mean[cg * 8 + e]; is[e] = inv_std[cg * 8 + e]; }
+    for (int w = 0; w < 4; ++w) {
+      const __nv_bfloat162 p = __floats2bfloat162_rn(acc[2 * w], acc[2 * w + 1]);
+      ow[w] = *reinterpret_cast<const unsigned*>(&p);
     }
-    PoolBwdRow ra, rb, rc;                 // window rows y-1, y, y+1
-    pool_bwd_load(dp, do_cs, ip, C, img0, x, crop, y0 - 1, ra);
-    pool_bwd_load(dp, do_cs, ip, C, img0, x, crop, y0, rb);
-    for (int y = y0; y < y1; ++y) {
-      pool_bwd_load(dp, do_cs, ip, C, img0, x, crop, y + 1, rc);
-      uint4 zraw = make_uint4(0u, 0u, 0u, 0u);
-      if (STATS) zraw = *reinterpret_cast<const uint4*>(z + (img0 + (int64_t)y * crop + x) * C + cg * 8);
-      float acc[8];
-#pragma unroll
-      for (int e = 0; e < 8; ++e) acc[e] = 0.0f;
-      // same summation order as the gather formulation: dy = -1 (window row y+1), 0, +1 (window row y-1); dx = -1, 0, +1
-      pool_bwd_acc(rc, -1, acc);
-      pool_bwd_acc(rb, 0, acc);
-      pool_bwd_acc(ra, 1, acc);
-      uint4 o;
-      unsigned* ow = reinterpret_cast<unsigned*>(&o);
-#pragma unroll
-      for (int w = 0; w < 4; ++w) {
-        const __nv_bfloat162 p = __floats2bfloat162_rn(acc[2 * w], acc[2 * w + 1]);
-        ow[w] = *reinterpret_cast<const unsigned*>(&p);
-      }
-      *reinterpret_cast<uint4*>(din + (img0 + (int64_t)y * crop + x) * di_cs + di_co + cg * 8) = o;
-      if (STATS) {
-        const unsigned* zw = reinterpret_cast<const unsigned*>(&zraw);
-#pragma unroll
-        for (int e = 0; e < 8; ++e) {
-          const unsigned gw = ow[e >> 1], zz = zw[e >> 1];
-          float g = __uint_as_float((e & 1) ? (gw & 0xFFFF0000u) : (gw << 16));          // the rounded dIn, as stored
-          const float zf = __uint_as_float((e & 1) ? (zz & 0xFFFF0000u) : (zz << 16));
-          const float xh = (zf - mu[e]) * is[e];
-          if (act == ACT_RELU) g = xh > 0.0f ? g : 0.0f;
-          else if (act == ACT_LRELU) g = xh > 0.0f ? g : 0.1f * g;
-          s0[e] += g;
-          s1[e] = fmaf(g, xh, s1[e]);
-        }
-      }
-      ra = rb;
-      rb = rc;
-    }
+    *reinterpret_cast<uint4*>(din + (img0 + (int64_t)y * crop + x) * di_cs + di_co + cg * 8) = o;
+    ra = rb;
+    rb = rc;
   }
-  if (!STATS) return;
-  __shared__ float s_red[16][256 + 1];
-#pragma unroll
-  for (int e = 0; e < 8; ++e) {
-    s_red[e][threadIdx.x] = s0[e];
-    s_red[8 + e][threadIdx.x] = s1[e];
-  }
-  __syncthreads();
-  // threads of this block that hold channel group g: t = t0 + r*cv with t0 = (g - first_gid) mod cv
-  const int first = (int)(((int64_t)blockIdx.x * blockDim.x) % cv);
-  for (int i = threadIdx.x; i < 2 * C; i += 256) {
-    const int which = i / C, rem = i - which * C;
-    const int e = rem / cv, g = rem - e * cv;
-    int t0 = g - first;
-    if (t0 < 0) t0 += cv;
-    float a = 0.0f;
-    for (int t = t0; t < 256; t += cv) a += s_red[which * 8 + e][t];
-    const long long q = __double2ll_rn((double)a * fin.fx_scale);
-    atomicAdd(bn_acc_mine(fin) + which * C + g * 8 + e, static_cast<unsigned long long>(q));
-  }
-  __shared__ bool s_last;
-  __threadfence();
-  __syncthreads();
-  if (threadIdx.x == 0) s_last = (atomicAdd(fin.counter, 1u) == gridDim.x - 1);
-  __syncthreads();
-  if (!s_last) return;
-  __threadfence();
-  const double inv_scale = 1.0 / fin.fx_scale;
-  for (int i = threadIdx.x; i < 2 * C; i += 256) {
-    const double a = (double)bn_acc_take(fin, i) * inv_scale;
-    fin.sums[i] = (float)a;
-  }
-  if (threadIdx.x == 0) *fin.counter = 0u;
 }
 
 #include "pool_train.cuh"
@@ -575,6 +378,8 @@ static bool pool_lean_enabled() {
   return on;
 }
 
+// idx != nullptr: training (winner codes, normalise + activation of the winner with bn_mean / bn_inv_std / act);
+// otherwise inference (plain max).
 template <typename T>
 static void launch_maxpool3_fwd(Handle* h, const T* in, int in_cs, int in_co, T* out, int out_cs, int out_co, uint8_t* idx, int C,
                                 int B, int crop, const float* bn_mean = nullptr, const float* bn_inv_std = nullptr, int act = 0) {
@@ -584,27 +389,18 @@ static void launch_maxpool3_fwd(Handle* h, const T* in, int in_cs, int in_co, T*
   nseg = (int)ceil_div(crop, seg);
   const int64_t total = base * nseg;
   const unsigned nb = (unsigned)ceil_div(total, 256);
-  if (idx && ElemTag<T>::v == ET_BF16 && bn_mean && pool_lean_enabled()) {
+  if (idx && ElemTag<T>::v == ET_BF16 && pool_lean_enabled()) {
     auto k = act == ACT_RELU ? pool_lean::fwd_kernel<ACT_RELU> : act == ACT_LRELU ? pool_lean::fwd_kernel<ACT_LRELU> : pool_lean::fwd_kernel<ACT_NONE>;
     launch_pdl(h, k, dim3(nb), dim3(256), 0, (const __nv_bfloat16*)in, in_cs, in_co, (__nv_bfloat16*)out, out_cs, out_co, idx, C, B, crop, seg, nseg, bn_mean, bn_inv_std);
-  } else if (idx && ElemTag<T>::v == ET_BF16 && !getenv("DRS_NO_POOL_PIPELINE"))
+  } else if (idx && ElemTag<T>::v == ET_BF16)
     maxpool3_fwd_train_bf16_pipelined_kernel<<<nb, 256, 0, h->stream>>>((const __nv_bfloat16*)in, in_cs, in_co, (__nv_bfloat16*)out, out_cs, out_co, idx, C, B, crop, seg, nseg, bn_mean, bn_inv_std, act);
-  else if (idx && ElemTag<T>::v == ET_BF16)
-    maxpool3_fwd_train_bf16_kernel<<<nb, 256, 0, h->stream>>>((const __nv_bfloat16*)in, in_cs, in_co, (__nv_bfloat16*)out, out_cs, out_co, idx, C, B, crop, seg, nseg, bn_mean, bn_inv_std, act);
-  else if (idx && bn_mean) maxpool3_fwd_kernel<T, true, true><<<nb, 256, 0, h->stream>>>(in, in_cs, in_co, out, out_cs, out_co, idx, C, B, crop, seg, nseg, bn_mean, bn_inv_std, act);
-  else if (idx) maxpool3_fwd_kernel<T, true, false><<<nb, 256, 0, h->stream>>>(in, in_cs, in_co, out, out_cs, out_co, idx, C, B, crop, seg, nseg, nullptr, nullptr, 0);
-  else if (bn_mean) maxpool3_fwd_kernel<T, false, true><<<nb, 256, 0, h->stream>>>(in, in_cs, in_co, out, out_cs, out_co, nullptr, C, B, crop, seg, nseg, bn_mean, bn_inv_std, act);
+  else if (idx) maxpool3_fwd_kernel<T><<<nb, 256, 0, h->stream>>>(in, in_cs, in_co, out, out_cs, out_co, idx, C, B, crop, seg, nseg, bn_mean, bn_inv_std, act);
   else {
-    static const int variant = getenv("DRS_POOL_INFER") ? atoi(getenv("DRS_POOL_INFER")) : 2;   // 1: one column per thread
-    if (variant == 2) {
-      const int64_t base2 = (int64_t)B * ((crop + 1) / 2) * (C / 8);
-      int nseg2 = (int)std::min<int64_t>(std::max<int64_t>(1, ceil_div((int64_t)h->sm_count * 2048, base2)), std::max(1, crop / 4));
-      const int seg2 = (int)ceil_div(crop, nseg2);
-      nseg2 = (int)ceil_div(crop, seg2);
-      maxpool3_fwd_packed2_kernel<T><<<(unsigned)ceil_div(base2 * nseg2, 256), 256, 0, h->stream>>>(in, in_cs, in_co, out, out_cs, out_co, C, B, crop, seg2, nseg2);
-    } else {
-      maxpool3_fwd_packed_kernel<T><<<nb, 256, 0, h->stream>>>(in, in_cs, in_co, out, out_cs, out_co, C, B, crop, seg, nseg);
-    }
+    const int64_t base2 = (int64_t)B * ((crop + 1) / 2) * (C / 8);
+    int nseg2 = (int)std::min<int64_t>(std::max<int64_t>(1, ceil_div((int64_t)h->sm_count * 2048, base2)), std::max(1, crop / 4));
+    const int seg2 = (int)ceil_div(crop, nseg2);
+    nseg2 = (int)ceil_div(crop, seg2);
+    maxpool3_fwd_packed2_kernel<T><<<(unsigned)ceil_div(base2 * nseg2, 256), 256, 0, h->stream>>>(in, in_cs, in_co, out, out_cs, out_co, C, B, crop, seg2, nseg2);
   }
   LAUNCH_CHECK(h);
 }
@@ -651,8 +447,7 @@ __global__ void maxpool3_bwd_kernel(const T* __restrict__ dout, int do_cs, int d
 
 template <typename T>
 static void launch_maxpool3_bwd(Handle* h, const T* dout, int do_cs, int do_co, const uint8_t* idx, T* din, int di_cs, int di_co,
-                                int C, int B, int crop, const BnFinish* stats = nullptr, const T* stats_z = nullptr,
-                                const float* stats_mean = nullptr, const float* stats_inv_std = nullptr, int stats_act = 0) {
+                                int C, int B, int crop) {
   const int64_t M = (int64_t)B * crop * crop;
   if (ElemTag<T>::v == ET_BF16) {
     const int64_t base = (int64_t)B * crop * (C / 8);
@@ -660,25 +455,12 @@ static void launch_maxpool3_bwd(Handle* h, const T* dout, int do_cs, int do_co, 
     const int seg = (int)ceil_div(crop, nseg);
     nseg = (int)ceil_div(crop, seg);
     const unsigned nb = (unsigned)ceil_div(base * nseg, 256);
-    if (pool_lean_enabled()) {
-      if (stats) {
-        auto k = stats_act == ACT_RELU ? pool_lean::bwd_kernel<ACT_RELU, true>
-                 : stats_act == ACT_LRELU ? pool_lean::bwd_kernel<ACT_LRELU, true> : pool_lean::bwd_kernel<ACT_NONE, true>;
-        launch_pdl(h, k, dim3(nb), dim3(256), 0, (const __nv_bfloat16*)dout, do_cs, do_co, idx, (__nv_bfloat16*)din, di_cs, di_co, C, B, crop, seg,
-                   nseg, (const __nv_bfloat16*)stats_z, stats_mean, stats_inv_std, *stats);
-      } else {
-        launch_pdl(h, pool_lean::bwd_kernel<ACT_NONE, false>, dim3(nb), dim3(256), 0, (const __nv_bfloat16*)dout, do_cs, do_co, idx,
-                   (__nv_bfloat16*)din, di_cs, di_co, C, B, crop, seg, nseg, (const __nv_bfloat16*)nullptr, (const float*)nullptr,
-                   (const float*)nullptr, BnFinish{});
-      }
-    } else if (stats)
-      maxpool3_bwd_bf16_kernel<true><<<(unsigned)ceil_div(base * nseg, 256), 256, 0, h->stream>>>(
-          (const __nv_bfloat16*)dout, do_cs, do_co, idx, (__nv_bfloat16*)din, di_cs, di_co, C, B, crop, seg, nseg,
-          (const __nv_bfloat16*)stats_z, stats_mean, stats_inv_std, stats_act, *stats);
+    if (pool_lean_enabled())
+      launch_pdl(h, pool_lean::bwd_kernel, dim3(nb), dim3(256), 0, (const __nv_bfloat16*)dout, do_cs, do_co, idx, (__nv_bfloat16*)din,
+                 di_cs, di_co, C, B, crop, seg, nseg);
     else
-      maxpool3_bwd_bf16_kernel<false><<<(unsigned)ceil_div(base * nseg, 256), 256, 0, h->stream>>>(
-          (const __nv_bfloat16*)dout, do_cs, do_co, idx, (__nv_bfloat16*)din, di_cs, di_co, C, B, crop, seg, nseg, nullptr, nullptr,
-          nullptr, 0, BnFinish{});
+      maxpool3_bwd_bf16_kernel<<<nb, 256, 0, h->stream>>>((const __nv_bfloat16*)dout, do_cs, do_co, idx, (__nv_bfloat16*)din, di_cs,
+                                                          di_co, C, B, crop, seg, nseg);
   } else {
     maxpool3_bwd_kernel<T><<<(unsigned)ceil_div(M * (C / 8), 256), 256, 0, h->stream>>>(dout, do_cs, do_co, idx, din, di_cs, di_co, C, M, crop);
   }
@@ -1044,20 +826,17 @@ static void launch_classifier_fwd(Handle* h, const T* x, int x_cs, int x_co, int
                                   float* logits, uint8_t* pred, int64_t M) {
   DRS_CHECK(Ci % 64 == 0, "classifier: Ci=%d must be a multiple of 64", Ci);
   auto smem_of = [&](int tile) { return (size_t)Ci * 8 * 4 + (size_t)tile * Ci * sizeof(T); };
-  static const int force_tile = getenv("DRS_CLS_TILE") ? atoi(getenv("DRS_CLS_TILE")) : 0;
-  if (force_tile == 64) launch_classifier_fwd_t<T, 64>(h, x, x_cs, x_co, Ci, w, b, K, logits, pred, M, smem_of(64));
-  else if (smem_of(128) <= 112 * 1024) launch_classifier_fwd_t<T, 128>(h, x, x_cs, x_co, Ci, w, b, K, logits, pred, M, smem_of(128));
+  if (smem_of(128) <= 112 * 1024) launch_classifier_fwd_t<T, 128>(h, x, x_cs, x_co, Ci, w, b, K, logits, pred, M, smem_of(128));
   else if (smem_of(64) <= 112 * 1024 || smem_of(128) > 220 * 1024) launch_classifier_fwd_t<T, 64>(h, x, x_cs, x_co, Ci, w, b, K, logits, pred, M, smem_of(64));
   else launch_classifier_fwd_t<T, 128>(h, x, x_cs, x_co, Ci, w, b, K, logits, pred, M, smem_of(128));
 }
 
 // Inference: the LAST 3x3 max-pool and the classifier (1x1 convolution Ci -> K, isprs:779-786) in one pass.  The pooled
 // activations of the last layer feed nothing but the classifier, so they are neither written nor read back: the kernel
-// reads the last convolution's output once (M*Ci*2 B) and writes M*K logits.  Same thread layout as
-// maxpool3_fwd_packed_kernel -- a thread owns (image, row segment, column, 8 channels) and walks down its rows -- so the
-// CV = Ci/8 lanes that hold one pixel are neighbours in a warp: each lane multiplies its 8 pooled channels (exactly the
-// values the unfused kernel would have stored) with its 8 x K weights held in registers, and the K partial sums are combined
-// by a transposing butterfly (4 + 2 + 1 shuffles halve the number of classes a lane carries, the remaining steps add one
+// reads the last convolution's output once (M*Ci*2 B) and writes M*K logits.  A thread owns (image, row segment, two
+// columns, 8 channels) and walks down its rows, so the CV = Ci/8 lanes that hold one pixel are neighbours in a warp: each
+// lane multiplies its 8 pooled channels (exactly the values the unfused kernel would have stored) with its 8 x K weights
+// held in registers, and the K partial sums are combined by a transposing butterfly (4 + 2 + 1 shuffles halve the number of classes a lane carries, the remaining steps add one
 // value), after which the lanes with (lane % (CV/8)) == 0 hold one class each.  The order of the additions is the same for
 // every pixel wherever it sits, so patch-wise and scene-wise inference and every stripe agree bit for bit.
 // K partial class sums per lane -> one class per lane (see the kernel's header comment); every lane of the CV-lane group calls it
@@ -1197,13 +976,9 @@ maxpool3_classifier_kernel(const T* __restrict__ in, int in_cs, int in_co, int B
   }
 }
 
-static inline bool pool_classifier_fused_enabled() {
-  static const bool on = !getenv("DRS_NO_POOL_CLS_FUSE");
-  return on;
-}
 template <typename T>
 static inline bool pool_classifier_fused_supported(int Ci) {
-  return ElemTag<T>::v != ET_F32 && (Ci == 64 || Ci == 128 || Ci == 256) && pool_classifier_fused_enabled();
+  return ElemTag<T>::v != ET_F32 && (Ci == 64 || Ci == 128 || Ci == 256);
 }
 template <typename T>
 static void launch_maxpool3_classifier(Handle* h, const T* in, int in_cs, int in_co, int Ci, int B, int crop, const float* w,

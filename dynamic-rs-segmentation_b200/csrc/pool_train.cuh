@@ -13,8 +13,6 @@
 //     widened once per load into fp16 bit patterns 0x44cc (distinct normal numbers), so HSETP2 compares two channels per
 //     instruction; no masks, no byte permutes, no shifts per tap.  Rows are walked bottom-up with the windows right to left:
 //     that is the summation order of the gather kernels (dy = -1, 0, +1; dx = -1, 0, +1), so results are bit-identical.
-//   * the backward can also reduce the two batch-norm backward sums of the layer below (STATS): with the instruction diet
-//     this costs less than a separate pass over Z and dIn.
 #pragma once
 
 namespace pool_lean {
@@ -203,13 +201,8 @@ __device__ __forceinline__ void bwd_scatter(const BwdRow& r, float (&up)[8], flo
   }
 }
 
-// rounds and stores a finished row, clears its accumulators; STATS: adds the row to the batch-norm backward sums
-//   s0 = sum g, s1 = sum g * xh,  g = dIn * act'(xh), xh = (z - mean) * inv_std, over the rounded dIn as stored
-template <int ACT, bool STATS>
-__device__ __forceinline__ void bwd_emit(float (&acc)[8], __nv_bfloat16* __restrict__ pd, const __nv_bfloat16* __restrict__ pz,
-                                         const float (&mu)[8], const float (&is)[8], float (&s0)[8], float (&s1)[8]) {
-  uint4 zraw = make_uint4(0u, 0u, 0u, 0u);
-  if (STATS) zraw = *reinterpret_cast<const uint4*>(pz);
+// rounds and stores a finished row, clears its accumulators
+__device__ __forceinline__ void bwd_emit(float (&acc)[8], __nv_bfloat16* __restrict__ pd) {
   uint4 o;
   unsigned* ow = reinterpret_cast<unsigned*>(&o);
 #pragma unroll
@@ -220,122 +213,56 @@ __device__ __forceinline__ void bwd_emit(float (&acc)[8], __nv_bfloat16* __restr
     acc[2 * w + 1] = 0.0f;
   }
   *reinterpret_cast<uint4*>(pd) = o;
-  if (STATS) {
-    const unsigned* zw = reinterpret_cast<const unsigned*>(&zraw);
-#pragma unroll
-    for (int e = 0; e < 8; ++e) {
-      const unsigned gw = ow[e >> 1], zz = zw[e >> 1];
-      float g = __uint_as_float((e & 1) ? (gw & 0xFFFF0000u) : (gw << 16));
-      const float zf = __uint_as_float((e & 1) ? (zz & 0xFFFF0000u) : (zz << 16));
-      const float xh = (zf - mu[e]) * is[e];
-      if (ACT == ACT_RELU) g = xh > 0.0f ? g : 0.0f;
-      else if (ACT == ACT_LRELU) g = xh > 0.0f ? g : 0.1f * g;
-      s0[e] += g;
-      s1[e] = fmaf(g, xh, s1[e]);
-    }
-  }
 }
 
-template <int ACT, bool STATS>
 __global__ void __launch_bounds__(256, DRS_POOL_MINBLK)
 bwd_kernel(const __nv_bfloat16* __restrict__ dout, int do_cs, int do_co, const uint8_t* __restrict__ idx,
-           __nv_bfloat16* __restrict__ din, int di_cs, int di_co, int C, int B, int crop, int seg, int nseg,
-           const __nv_bfloat16* __restrict__ z, const float* __restrict__ mean, const float* __restrict__ inv_std, BnFinish fin) {
+           __nv_bfloat16* __restrict__ din, int di_cs, int di_co, int C, int B, int crop, int seg, int nseg) {
   pdl_sync();
   const int cv = C >> 3;
   const int64_t gid = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  const bool live = gid < (int64_t)B * nseg * crop * cv;
-  if (!STATS && !live) return;
+  if (gid >= (int64_t)B * nseg * crop * cv) return;
   const int cg = (int)(gid % cv);
-  float s0[8], s1[8], mu[8], is[8];
+  int64_t t = gid / cv;
+  const int x = (int)(t % crop);
+  t /= crop;
+  const int sg = (int)(t % nseg);
+  const int b = (int)(t / nseg);
+  const int y0 = sg * seg, y1 = min(crop, y0 + seg);
+  const int64_t pix0 = (int64_t)b * crop * crop + x;
+  const bool xl = x > 0, xr = x + 1 < crop;
+  const __nv_bfloat16* pg = dout + pix0 * do_cs + do_co + cg * 8;
+  const uint8_t* pk = idx + pix0 * C + cg * 8;
+  const int64_t gs = (int64_t)crop * do_cs, ks = (int64_t)crop * C;
+  __nv_bfloat16* pd = din + (pix0 + (int64_t)(y1 - 1) * crop) * di_cs + di_co + cg * 8;
+  const int64_t ds = (int64_t)crop * di_cs;
+  float a0[8], a1[8], a2[8];
 #pragma unroll
-  for (int e = 0; e < 8; ++e) { s0[e] = 0.0f; s1[e] = 0.0f; mu[e] = 0.0f; is[e] = 1.0f; }
-  if (live) {
-    int64_t t = gid / cv;
-    const int x = (int)(t % crop);
-    t /= crop;
-    const int sg = (int)(t % nseg);
-    const int b = (int)(t / nseg);
-    const int y0 = sg * seg, y1 = min(crop, y0 + seg);
-    const int64_t pix0 = (int64_t)b * crop * crop + x;
-    const bool xl = x > 0, xr = x + 1 < crop;
-    const __nv_bfloat16* pg = dout + pix0 * do_cs + do_co + cg * 8;
-    const uint8_t* pk = idx + pix0 * C + cg * 8;
-    const int64_t gs = (int64_t)crop * do_cs, ks = (int64_t)crop * C;
-    __nv_bfloat16* pd = din + (pix0 + (int64_t)(y1 - 1) * crop) * di_cs + di_co + cg * 8;
-    const int64_t ds = (int64_t)crop * di_cs;
-    const __nv_bfloat16* pz = nullptr;
-    int64_t zs = 0;
-    if (STATS) {
-      pz = z + (pix0 + (int64_t)(y1 - 1) * crop) * C + cg * 8;
-      zs = (int64_t)crop * C;
-#pragma unroll
-      for (int e = 0; e < 8; ++e) { mu[e] = mean[cg * 8 + e]; is[e] = inv_std[cg * 8 + e]; }
-    }
-    float a0[8], a1[8], a2[8];
-#pragma unroll
-    for (int e = 0; e < 8; ++e) { a0[e] = 0.0f; a1[e] = 0.0f; a2[e] = 0.0f; }
-    BwdRow r;
-    // Bottom-up: position row y is complete once window rows y+1, y, y-1 have been scattered, in that order (the gather
-    // kernels' dy = -1, 0, +1).  Prologue: window row y1 reaches only row y1-1 of this segment, window row y1-1 rows y1-1
-    // and y1-2; contributions to rows outside [y0, y1) belong to other threads and are not computed.
-    bwd_load(pg, gs, do_cs, pk, ks, C, y1, crop, xl, xr, r);
-    bwd_scatter<true, false, false>(r, a0, a1, a2);
-    bwd_load(pg, gs, do_cs, pk, ks, C, y1 - 1, crop, xl, xr, r);
-    bwd_scatter<true, true, false>(r, a1, a0, a2);
-    // step for position row y: ACC_Y = row y (window rows y+1 and y already in), ACC_1 = row y-1, ACC_2 = row y-2 (zero)
+  for (int e = 0; e < 8; ++e) { a0[e] = 0.0f; a1[e] = 0.0f; a2[e] = 0.0f; }
+  BwdRow r;
+  // Bottom-up: position row y is complete once window rows y+1, y, y-1 have been scattered, in that order (the gather
+  // kernels' dy = -1, 0, +1).  Prologue: window row y1 reaches only row y1-1 of this segment, window row y1-1 rows y1-1
+  // and y1-2; contributions to rows outside [y0, y1) belong to other threads and are not computed.
+  bwd_load(pg, gs, do_cs, pk, ks, C, y1, crop, xl, xr, r);
+  bwd_scatter<true, false, false>(r, a0, a1, a2);
+  bwd_load(pg, gs, do_cs, pk, ks, C, y1 - 1, crop, xl, xr, r);
+  bwd_scatter<true, true, false>(r, a1, a0, a2);
+  // step for position row y: ACC_Y = row y (window rows y+1 and y already in), ACC_1 = row y-1, ACC_2 = row y-2 (zero)
 #define DRS_POOL_BWD_STEP(ACC_Y, ACC_1, ACC_2)                                                   \
   {                                                                                               \
     bwd_load(pg, gs, do_cs, pk, ks, C, y - 1, crop, xl, xr, r);                                   \
     if (y > y0) bwd_scatter<true, true, true>(r, ACC_2, ACC_1, ACC_Y);                            \
     else bwd_scatter<false, false, true>(r, ACC_2, ACC_1, ACC_Y);                                 \
-    bwd_emit<ACT, STATS>(ACC_Y, pd, pz, mu, is, s0, s1);                                          \
+    bwd_emit(ACC_Y, pd);                                                                          \
     pd -= ds;                                                                                     \
-    if (STATS) pz -= zs;                                                                          \
     if (--y < y0) break;                                                                          \
   }
-    for (int y = y1 - 1;;) {
-      DRS_POOL_BWD_STEP(a0, a1, a2)
-      DRS_POOL_BWD_STEP(a1, a2, a0)
-      DRS_POOL_BWD_STEP(a2, a0, a1)
-    }
+  for (int y = y1 - 1;;) {
+    DRS_POOL_BWD_STEP(a0, a1, a2)
+    DRS_POOL_BWD_STEP(a1, a2, a0)
+    DRS_POOL_BWD_STEP(a2, a0, a1)
+  }
 #undef DRS_POOL_BWD_STEP
-  }
-  if (!STATS) return;
-  // per-thread sums -> fixed-order block sums in shared memory -> 64-bit fixed point -> integer atomics (order-independent);
-  // the last block publishes them (same protocol as bn_partial_kernel)
-  __shared__ float s_red[16][256 + 1];
-#pragma unroll
-  for (int e = 0; e < 8; ++e) {
-    s_red[e][threadIdx.x] = s0[e];
-    s_red[8 + e][threadIdx.x] = s1[e];
-  }
-  __syncthreads();
-  // threads of this block that hold channel group g: t = t0 + r*cv with t0 = (g - first_gid) mod cv
-  const int first = (int)(((int64_t)blockIdx.x * blockDim.x) % cv);
-  for (int i = threadIdx.x; i < 2 * C; i += 256) {
-    const int which = i / C, rem = i - which * C;
-    const int e = rem / cv, g = rem - e * cv;
-    int t0 = g - first;
-    if (t0 < 0) t0 += cv;
-    float a = 0.0f;
-    for (int t = t0; t < 256; t += cv) a += s_red[which * 8 + e][t];
-    const long long q = __double2ll_rn((double)a * fin.fx_scale);
-    atomicAdd(bn_acc_mine(fin) + which * C + g * 8 + e, static_cast<unsigned long long>(q));
-  }
-  __shared__ bool s_last;
-  __threadfence();
-  __syncthreads();
-  if (threadIdx.x == 0) s_last = (atomicAdd(fin.counter, 1u) == gridDim.x - 1);
-  __syncthreads();
-  if (!s_last) return;
-  __threadfence();
-  const double inv_scale = 1.0 / fin.fx_scale;
-  for (int i = threadIdx.x; i < 2 * C; i += 256) {
-    const double a = (double)bn_acc_take(fin, i) * inv_scale;
-    fin.sums[i] = (float)a;
-  }
-  if (threadIdx.x == 0) *fin.counter = 0u;
 }
 
 // ------------------------------------------------------------------------------------------------ backward + BN backward

@@ -17,16 +17,15 @@ DENSE = [("d2", 5, 1, 32, 32), ("d3", 4, 2, 64, 64), ("d4", 4, 2, 128, 64), ("d5
 
 
 def word(spec):
-    """'-1' production default; otherwise tokens m<mode> k<K blocks per stage> i1 (instrumented) s1 (dual MMA warps, experiment)
+    """'-1' production default; otherwise tokens m<mode> k<K blocks per stage> i1 (instrumented)
     p1 / p2 (force single 128-pixel units / pairs of units per filter slice), e.g. k2 or k2m10i1 or p1."""
     import re
     if re.fullmatch(r"-?\d+", spec):
         return int(spec)
     w = 0
-    for key, val in re.findall(r"([mkisp])(\d+)", spec):
+    for key, val in re.findall(r"([mkip])(\d+)", spec):
         val = int(val)
-        w |= val if key == "m" else (val << 12 if key == "k" else ((val & 1) << 16 if key == "i" else
-                                      ((val & 3) << 20 if key == "p" else (val & 1) << 18)))
+        w |= val if key == "m" else (val << 12 if key == "k" else ((val & 1) << 16 if key == "i" else (val & 3) << 20))
     return w
 
 
@@ -64,7 +63,7 @@ def main():
             ins = (C.c_uint32 * 10)()
             L.check(lib.drs_bench_conv(s._h, B, crop, k, rate, ci, co, L.PREC[prec], m, reps, C.byref(ms), ins))
             fl = 2.0 * B * crop * crop * k * k * ci * co
-            tag = "prod" if m < 0 else "m%d%s%s" % (m & 0xff, "k%d" % ((m >> 12) & 0xf) if (m >> 12) & 0xf else "", "dual" if (m >> 18) & 1 else "")
+            tag = "prod" if m < 0 else "m%d%s" % (m & 0xff, "k%d" % ((m >> 12) & 0xf) if (m >> 12) & 0xf else "")
             txt = "%s %.0fus %.0fTF" % (tag, ms.value * 1e3, fl / ms.value / 1e9)
             if m >= 0 and (m >> 16) & 1:
                 v = list(ins)
