@@ -386,38 +386,3 @@ static bool launch_wgrad_conv1(Handle* h, const float* x, int C, const TG* dy, i
   LAUNCH_CHECK(h);
   return true;
 }
-
-// ------------------------------------------------------------------------------------------------
-// weight packing: master fp32 HWIO -> operand matrices
-// ------------------------------------------------------------------------------------------------
-// fprop operand  Wf[co][tap*ci + c] = W[tap][c][co]
-template <typename T>
-__global__ void pack_fprop_kernel(const float* __restrict__ w, T* __restrict__ out, int taps, int ci, int co) {
-  const int64_t n = (int64_t)taps * ci * co;
-  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= n) return;
-  const int o = (int)(i / ((int64_t)taps * ci));
-  const int kk = (int)(i - (int64_t)o * taps * ci);
-  out[i] = from_f32<T>(w[(int64_t)kk * co + o]);
-}
-// dgrad operand  Wd[c][tap'*co + o] = W[taps-1-tap'][c][o]   (K-major for the tensor-core path)
-template <typename T>
-__global__ void pack_dgrad_kernel(const float* __restrict__ w, T* __restrict__ out, int taps, int ci, int co) {
-  const int64_t n = (int64_t)taps * ci * co;
-  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= n) return;
-  const int c = (int)(i / ((int64_t)taps * co));
-  const int r = (int)(i - (int64_t)c * taps * co);
-  const int tp = r / co, o = r - tp * co;
-  out[i] = from_f32<T>(w[((int64_t)(taps - 1 - tp) * ci + c) * co + o]);
-}
-// dgrad operand for the SIMT path: HWIO-like [tap'*co + o][c] fp32
-__global__ void pack_dgrad_simt_kernel(const float* __restrict__ w, float* __restrict__ out, int taps, int ci, int co) {
-  const int64_t n = (int64_t)taps * ci * co;
-  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= n) return;
-  const int c = (int)(i % ci);
-  const int r = (int)(i / ci);
-  const int tp = r / co, o = r - tp * co;
-  out[i] = w[((int64_t)(taps - 1 - tp) * ci + c) * co + o];
-}

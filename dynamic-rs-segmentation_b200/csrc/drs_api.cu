@@ -152,108 +152,19 @@ static void build_net(NetDesc& n, const drs_config& cfg) {
 extern "C" const char* drs_last_error(void) { return g_drs_err; }
 extern "C" int drs_version(void) { return DRS_VERSION; }
 
-struct InferLane {
-  cudaStream_t stream = nullptr;
-  Arena arena;
-  float* x = nullptr;
-  float* lg = nullptr;
-  size_t x_cap = 0, lg_cap = 0;
-  cudaEvent_t fwd_done = nullptr, acc_done = nullptr;
-};
-
-// One captured training step (CUDA graph) per (batch, patch size, buffers, learning rate): the step is ~65 small
-// dependent launches, so replaying it as a graph removes the launch gaps between them.
-struct TrainGraphKey {
-  int B, crop, ignore_label, profiling;
-  const void *x, *y, *mask, *acc_mask, *pred, *cm;
-  uint64_t lr_bits;
-  uint64_t arena_epoch;
-  bool operator<(const TrainGraphKey& o) const { return memcmp(this, &o, sizeof(*this)) < 0; }
-};
-struct TrainGraph {
-  cudaGraphExec_t exec = nullptr;
-  int64_t launches = 0, conv_launches = 0;
-  double conv_flops = 0;
-  std::vector<std::pair<cudaEvent_t, cudaEvent_t>> events;   // external event-record nodes around the tensor-core launches
-};
-
-constexpr int RESULT_STRIDE = 64 + MAX_CLASSES * MAX_CLASSES;   // floats per pinned result slot: loss, then K*K+1 counts
-struct HandleExtra {
-  // persistent scene-pass buffers (score map, occurrence counts, cell tables, label map ...): cudaMalloc / cudaFree of
-  // gigabyte-sized buffers per call costs hundreds of milliseconds, so each named slot only ever grows
-  // the label map of the last scene pass stays in slot 4 for drs_scene_confusion
-  int last_scene = -1, last_row_begin = 0, last_rows = 0, last_W = 0;
-  void* slot_ptr[8] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
-  size_t slot_cap[8] = {0, 0, 0, 0, 0, 0, 0, 0};
-  std::map<TrainGraphKey, TrainGraph> graphs;
-  std::map<TrainGraphKey, int> graph_seen;
-  TrainGraph* capturing = nullptr;   // non-null while a training step is being captured
-  cudaStream_t side_stream = nullptr;     // filter gradients run here, overlapped with the backward's HBM-bound kernels
-  cudaEvent_t ev_dz[2] = {nullptr, nullptr}, ev_wgrad[2] = {nullptr, nullptr};
-  // data-parallel exchange of the late layers' gradients, overlapped with the rest of the backward
-  cudaStream_t comm_stream = nullptr;
-  cudaEvent_t ev_bucket_ready = nullptr, ev_bucket_done = nullptr;
-  cudaEvent_t ev_x8 = nullptr;          // conv1's padded input is ready: the side stream builds the im2col matrix under the forward
-  bool use_graphs = false;          // opt-in (DRS_GRAPHS=1): measured 6-9 % per step in steady state, see DESIGN.md
-  double conv_ms_acc = 0;            // device time of profiled launches already read back
-  InferLane lane;                 // scene-inference lane (drs_scene_api.cuh)
-  cudaEvent_t lane_ready = nullptr;
-  // streamed scene upload (drs_scene_infer_host): copy stream + "rows uploaded" event
-  cudaStream_t copy_stream = nullptr;
-  cudaEvent_t up_ev[1] = {nullptr};
-  uint8_t* is_weight = nullptr;   // [n_trainable] 1 for `weights` variables
-  SceneTable table;               // host copy of the device scene table
-  // training scratch kept between calls
-  float* mean = nullptr;          // [sum co] batch mean of the last train step (per layer, same offsets as mm_off/2)
-  float* inv_std = nullptr;
-  float* sums = nullptr;          // [2*256]
-  float* loss_dev = nullptr;      // [4]: ce, l2, count, spare
-  unsigned int* cm_dev = nullptr; // [K*K+1]
-  unsigned int* count_dev = nullptr;
-  unsigned int* bn_counter = nullptr;   // last-block-done counter of bn_partial_kernel (self-resetting)
-  long long* bn_acc = nullptr;          // [BN_ACC_REPLICAS][2*512] fixed-point accumulators of bn_partial_kernel (self-clearing)
-  float* ones = nullptr;          // [512]
-  float* zeros = nullptr;         // [512]
-  float* cls_w_eval = nullptr;
-  // profiling
-  double conv_flops = 0;
-  int64_t conv_launches = 0;
-  // pipelined training loop (drs_gather_plan_dev / drs_train_step_async / drs_train_result): the plan of step i+1 is
-  // uploaded on plan_stream into a two-slot device staging ring while step i runs; loss + confusion counts of each step
-  // land in a ring of pinned result slots behind an event, so the host never blocks on the step it has just enqueued
-  void* nccl = nullptr;             // ncclComm_t of drs_comm_init (drs_comm.cuh); null: single process or callback exchange
-  int rank = 0;
-  cudaStream_t plan_stream = nullptr;
-  void* plan_stage[2] = {nullptr, nullptr};
-  size_t plan_stage_cap[2] = {0, 0};
-  cudaEvent_t plan_uploaded[2] = {nullptr, nullptr}, plan_consumed[2] = {nullptr, nullptr};
-  bool plan_consumed_valid[2] = {false, false};
-  int64_t plan_calls = 0;
-  static constexpr int RESULT_RING = 8;
-  float* result_host = nullptr;     // pinned [RESULT_RING][RESULT_STRIDE]
-  cudaEvent_t result_ev[RESULT_RING] = {};
-  int64_t next_ticket = 0;
-  // DRS_DEBUG_KEEP=1: fp32 copies of backward intermediates ("dz:<scope>", "da:<scope>")
-  std::vector<float*> keep;
-  bool debug_keep = false;
-};
-static std::map<Handle*, HandleExtra*> g_extra;
-static HandleExtra* X(Handle* h) { return g_extra[h]; }
 static void* slot_buf(Handle* h, int slot, size_t bytes) {
-  HandleExtra* x = X(h);
   if (bytes == 0) bytes = 16;
-  if (x->slot_cap[slot] < bytes) {
+  if (h->slot_cap[slot] < bytes) {
     CUDA_CHECK(cudaStreamSynchronize(h->stream));
-    if (x->slot_ptr[slot]) CUDA_CHECK(cudaFree(x->slot_ptr[slot]));
-    x->slot_ptr[slot] = nullptr;
-    x->slot_cap[slot] = 0;
-    CUDA_CHECK(cudaMalloc(&x->slot_ptr[slot], bytes));
-    x->slot_cap[slot] = bytes;
+    if (h->slot_ptr[slot]) CUDA_CHECK(cudaFree(h->slot_ptr[slot]));
+    h->slot_ptr[slot] = nullptr;
+    h->slot_cap[slot] = 0;
+    CUDA_CHECK(cudaMalloc(&h->slot_ptr[slot], bytes));
+    h->slot_cap[slot] = bytes;
   }
-  return x->slot_ptr[slot];
+  return h->slot_ptr[slot];
 }
 static void lane_release(Handle* h);
-static void pass_geometry_release(Handle* h);
 
 static void free_packed(Handle* h) {
   for (auto& c : h->net.convs) {
@@ -278,8 +189,6 @@ extern "C" int drs_create(drs_handle_t* out, const drs_config* cfg) {
   CUDA_CHECK(cudaGetDeviceProperties(&prop, cfg->device));
   DRS_CHECK(prop.major == 10, "drs_create: device %s is sm_%d%d; libdrs is built for sm_100a only", prop.name, prop.major, prop.minor);
   Handle* h = new Handle();
-  HandleExtra* x = new HandleExtra();
-  g_extra[h] = x;
   h->cfg = *cfg;
   h->sm_count = prop.multiProcessorCount;
   CUDA_CHECK(cudaDriverGetVersion(&h->driver_version));
@@ -294,7 +203,7 @@ extern "C" int drs_create(drs_handle_t* out, const drs_config* cfg) {
   CUDA_CHECK(cudaMemset(h->params, 0, nt * 4));
   CUDA_CHECK(cudaMemset(h->grads, 0, (nt + 1024) * 4));
   CUDA_CHECK(cudaMemset(h->moms, 0, nt * 4));
-  CUDA_CHECK(cudaMalloc(&x->is_weight, nt));
+  CUDA_CHECK(cudaMalloc(&h->is_weight, nt));
   {
     std::vector<uint8_t> isw(nt, 0);
     for (auto& c : h->net.convs)
@@ -304,31 +213,31 @@ extern "C" int drs_create(drs_handle_t* out, const drs_config* cfg) {
       for (int64_t i = sb.w1_off; i < sb.b1_off; ++i) isw[i] = 1;
       for (int64_t i = sb.w2_off; i < sb.b2_off; ++i) isw[i] = 1;
     }
-    CUDA_CHECK(cudaMemcpy(x->is_weight, isw.data(), nt, cudaMemcpyHostToDevice));
+    CUDA_CHECK(cudaMemcpy(h->is_weight, isw.data(), nt, cudaMemcpyHostToDevice));
     // moving_mean = 0, moving_variance = 1 (Appendix B.3)
     std::vector<float> bn(h->net.n_bnstat, 0.0f);
     for (auto& c : h->net.convs)
       for (int i = 0; i < c.co; ++i) bn[c.mv_off + i] = 1.0f;
     CUDA_CHECK(cudaMemcpy(h->bnstat, bn.data(), bn.size() * 4, cudaMemcpyHostToDevice));
   }
-  CUDA_CHECK(cudaMalloc(&x->mean, h->net.n_bnstat * 4));
-  CUDA_CHECK(cudaMalloc(&x->inv_std, h->net.n_bnstat * 4));
-  CUDA_CHECK(cudaMalloc(&x->sums, 2 * 512 * 4));
-  CUDA_CHECK(cudaMalloc(&x->loss_dev, 16 * 4));
-  CUDA_CHECK(cudaMalloc(&x->cm_dev, (MAX_CLASSES * MAX_CLASSES + 1) * 4));
-  CUDA_CHECK(cudaMalloc(&x->count_dev, 16));
-  CUDA_CHECK(cudaMemset(x->count_dev, 0, 16));
-  x->bn_counter = x->count_dev + 2;
-  CUDA_CHECK(cudaMalloc(&x->bn_acc, (size_t)BN_ACC_REPLICAS * BN_ACC_STRIDE * 8));
-  CUDA_CHECK(cudaMemset(x->bn_acc, 0, (size_t)BN_ACC_REPLICAS * BN_ACC_STRIDE * 8));
-  CUDA_CHECK(cudaMalloc(&x->ones, 512 * 4));
-  CUDA_CHECK(cudaMalloc(&x->zeros, 512 * 4));
-  CUDA_CHECK(cudaMemset(x->zeros, 0, 512 * 4));
+  CUDA_CHECK(cudaMalloc(&h->mean, h->net.n_bnstat * 4));
+  CUDA_CHECK(cudaMalloc(&h->inv_std, h->net.n_bnstat * 4));
+  CUDA_CHECK(cudaMalloc(&h->sums, 2 * 512 * 4));
+  CUDA_CHECK(cudaMalloc(&h->loss_dev, 16 * 4));
+  CUDA_CHECK(cudaMalloc(&h->cm_dev, (MAX_CLASSES * MAX_CLASSES + 1) * 4));
+  CUDA_CHECK(cudaMalloc(&h->count_dev, 16));
+  CUDA_CHECK(cudaMemset(h->count_dev, 0, 16));
+  h->bn_counter = h->count_dev + 2;
+  CUDA_CHECK(cudaMalloc(&h->bn_acc, (size_t)BN_ACC_REPLICAS * BN_ACC_STRIDE * 8));
+  CUDA_CHECK(cudaMemset(h->bn_acc, 0, (size_t)BN_ACC_REPLICAS * BN_ACC_STRIDE * 8));
+  CUDA_CHECK(cudaMalloc(&h->ones, 512 * 4));
+  CUDA_CHECK(cudaMalloc(&h->zeros, 512 * 4));
+  CUDA_CHECK(cudaMemset(h->zeros, 0, 512 * 4));
   {
     std::vector<float> o(512, 1.0f);
-    CUDA_CHECK(cudaMemcpy(x->ones, o.data(), 512 * 4, cudaMemcpyHostToDevice));
+    CUDA_CHECK(cudaMemcpy(h->ones, o.data(), 512 * 4, cudaMemcpyHostToDevice));
   }
-  memset(&x->table, 0, sizeof(x->table));
+  memset(&h->table, 0, sizeof(h->table));
   CUDA_CHECK(cudaHostAlloc(&h->diag_host, 64, cudaHostAllocMapped));
   memset(h->diag_host, 0, 64);
   CUDA_CHECK(cudaHostGetDevicePointer((void**)&h->diag_dev, h->diag_host, 0));
@@ -350,22 +259,22 @@ extern "C" int drs_create(drs_handle_t* out, const drs_config* cfg) {
   h->eval_dirty = true;
   // whole-step CUDA graphs per (batch, patch size, buffers, lr): on by default (DRS_GRAPHS=0 turns them off); the drop-in
   // loops pre-capture the patch-size interval at start-up (drs_train_prepare), like TF building its graph before the loop
-  x->use_graphs = getenv("DRS_GRAPHS") == nullptr || atoi(getenv("DRS_GRAPHS")) != 0;
-  CUDA_CHECK(cudaStreamCreateWithFlags(&x->plan_stream, cudaStreamNonBlocking));
+  h->use_graphs = getenv("DRS_GRAPHS") == nullptr || atoi(getenv("DRS_GRAPHS")) != 0;
+  CUDA_CHECK(cudaStreamCreateWithFlags(&h->plan_stream, cudaStreamNonBlocking));
   for (int i = 0; i < 2; ++i) {
-    CUDA_CHECK(cudaEventCreateWithFlags(&x->plan_uploaded[i], cudaEventDisableTiming));
-    CUDA_CHECK(cudaEventCreateWithFlags(&x->plan_consumed[i], cudaEventDisableTiming));
+    CUDA_CHECK(cudaEventCreateWithFlags(&h->plan_uploaded[i], cudaEventDisableTiming));
+    CUDA_CHECK(cudaEventCreateWithFlags(&h->plan_consumed[i], cudaEventDisableTiming));
   }
-  CUDA_CHECK(cudaHostAlloc((void**)&x->result_host, (size_t)HandleExtra::RESULT_RING * RESULT_STRIDE * 4, cudaHostAllocDefault));
-  for (int i = 0; i < HandleExtra::RESULT_RING; ++i) CUDA_CHECK(cudaEventCreateWithFlags(&x->result_ev[i], cudaEventDisableTiming));
-  CUDA_CHECK(cudaStreamCreateWithFlags(&x->side_stream, cudaStreamNonBlocking));
-  CUDA_CHECK(cudaStreamCreateWithFlags(&x->comm_stream, cudaStreamNonBlocking));
-  CUDA_CHECK(cudaEventCreateWithFlags(&x->ev_bucket_ready, cudaEventDisableTiming));
-  CUDA_CHECK(cudaEventCreateWithFlags(&x->ev_x8, cudaEventDisableTiming));
-  CUDA_CHECK(cudaEventCreateWithFlags(&x->ev_bucket_done, cudaEventDisableTiming));
+  CUDA_CHECK(cudaHostAlloc((void**)&h->result_host, (size_t)Handle::RESULT_RING * RESULT_STRIDE * 4, cudaHostAllocDefault));
+  for (int i = 0; i < Handle::RESULT_RING; ++i) CUDA_CHECK(cudaEventCreateWithFlags(&h->result_ev[i], cudaEventDisableTiming));
+  CUDA_CHECK(cudaStreamCreateWithFlags(&h->side_stream, cudaStreamNonBlocking));
+  CUDA_CHECK(cudaStreamCreateWithFlags(&h->comm_stream, cudaStreamNonBlocking));
+  CUDA_CHECK(cudaEventCreateWithFlags(&h->ev_bucket_ready, cudaEventDisableTiming));
+  CUDA_CHECK(cudaEventCreateWithFlags(&h->ev_x8, cudaEventDisableTiming));
+  CUDA_CHECK(cudaEventCreateWithFlags(&h->ev_bucket_done, cudaEventDisableTiming));
   for (int i = 0; i < 2; ++i) {
-    CUDA_CHECK(cudaEventCreateWithFlags(&x->ev_dz[i], cudaEventDisableTiming));
-    CUDA_CHECK(cudaEventCreateWithFlags(&x->ev_wgrad[i], cudaEventDisableTiming));
+    CUDA_CHECK(cudaEventCreateWithFlags(&h->ev_dz[i], cudaEventDisableTiming));
+    CUDA_CHECK(cudaEventCreateWithFlags(&h->ev_wgrad[i], cudaEventDisableTiming));
   }
   *out = h;
   API_END
@@ -376,38 +285,33 @@ extern "C" int drs_destroy(drs_handle_t h) {
   if (!h) return 0;
   cudaSetDevice(h->cfg.device);
   cudaStreamSynchronize(h->stream);
-  HandleExtra* x = X(h);
-  if (x) {
-    if (x->nccl) { drs_comm_destroy(h); }
-    pass_geometry_release(h);
-    if (x->side_stream) { cudaStreamSynchronize(x->side_stream); cudaStreamDestroy(x->side_stream); }
-    if (x->comm_stream) { cudaStreamSynchronize(x->comm_stream); cudaStreamDestroy(x->comm_stream); }
-    if (x->ev_bucket_ready) cudaEventDestroy(x->ev_bucket_ready);
-    if (x->ev_x8) cudaEventDestroy(x->ev_x8);
-    if (x->ev_bucket_done) cudaEventDestroy(x->ev_bucket_done);
-    if (x->copy_stream) { cudaStreamSynchronize(x->copy_stream); cudaStreamDestroy(x->copy_stream); }
-    if (x->plan_stream) { cudaStreamSynchronize(x->plan_stream); cudaStreamDestroy(x->plan_stream); }
-    for (int i = 0; i < 2; ++i) {
-      if (x->plan_uploaded[i]) cudaEventDestroy(x->plan_uploaded[i]);
-      if (x->plan_consumed[i]) cudaEventDestroy(x->plan_consumed[i]);
-      if (x->plan_stage[i]) cudaFree(x->plan_stage[i]);
-    }
-    for (int i = 0; i < HandleExtra::RESULT_RING; ++i)
-      if (x->result_ev[i]) cudaEventDestroy(x->result_ev[i]);
-    if (x->result_host) cudaFreeHost(x->result_host);
-    if (x->up_ev[0]) cudaEventDestroy(x->up_ev[0]);
-    for (int i = 0; i < 2; ++i) {
-      if (x->ev_dz[i]) cudaEventDestroy(x->ev_dz[i]);
-      if (x->ev_wgrad[i]) cudaEventDestroy(x->ev_wgrad[i]);
-    }
-    lane_release(h);
-    for (int i = 0; i < 8; ++i)
-      if (x->slot_ptr[i]) cudaFree(x->slot_ptr[i]);
-    for (auto& kv : x->graphs) {
-      if (kv.second.exec) cudaGraphExecDestroy(kv.second.exec);
-      for (auto& pr : kv.second.events) { cudaEventDestroy(pr.first); cudaEventDestroy(pr.second); }
-    }
-    x->graphs.clear();
+  if (h->nccl) { drs_comm_destroy(h); }
+  if (h->side_stream) { cudaStreamSynchronize(h->side_stream); cudaStreamDestroy(h->side_stream); }
+  if (h->comm_stream) { cudaStreamSynchronize(h->comm_stream); cudaStreamDestroy(h->comm_stream); }
+  if (h->ev_bucket_ready) cudaEventDestroy(h->ev_bucket_ready);
+  if (h->ev_x8) cudaEventDestroy(h->ev_x8);
+  if (h->ev_bucket_done) cudaEventDestroy(h->ev_bucket_done);
+  if (h->copy_stream) { cudaStreamSynchronize(h->copy_stream); cudaStreamDestroy(h->copy_stream); }
+  if (h->plan_stream) { cudaStreamSynchronize(h->plan_stream); cudaStreamDestroy(h->plan_stream); }
+  for (int i = 0; i < 2; ++i) {
+    if (h->plan_uploaded[i]) cudaEventDestroy(h->plan_uploaded[i]);
+    if (h->plan_consumed[i]) cudaEventDestroy(h->plan_consumed[i]);
+    if (h->plan_stage[i]) cudaFree(h->plan_stage[i]);
+  }
+  for (int i = 0; i < Handle::RESULT_RING; ++i)
+    if (h->result_ev[i]) cudaEventDestroy(h->result_ev[i]);
+  if (h->result_host) cudaFreeHost(h->result_host);
+  if (h->up_ev[0]) cudaEventDestroy(h->up_ev[0]);
+  for (int i = 0; i < 2; ++i) {
+    if (h->ev_dz[i]) cudaEventDestroy(h->ev_dz[i]);
+    if (h->ev_wgrad[i]) cudaEventDestroy(h->ev_wgrad[i]);
+  }
+  lane_release(h);
+  for (int i = 0; i < 8; ++i)
+    if (h->slot_ptr[i]) cudaFree(h->slot_ptr[i]);
+  for (auto& kv : h->graphs) {
+    if (kv.second.exec) cudaGraphExecDestroy(kv.second.exec);
+    for (auto& pr : kv.second.events) { cudaEventDestroy(pr.first); cudaEventDestroy(pr.second); }
   }
   free_packed(h);
   for (auto& kv : h->scenes) {
@@ -419,12 +323,8 @@ extern "C" int drs_destroy(drs_handle_t h) {
   if (h->dstage) cudaFree(h->dstage);
   if (h->pinned) cudaFreeHost(h->pinned);
   if (h->diag_host) cudaFreeHost(h->diag_host);
-  if (x) {
-    cudaFree(x->is_weight); cudaFree(x->mean); cudaFree(x->inv_std); cudaFree(x->sums); cudaFree(x->loss_dev);
-    cudaFree(x->cm_dev); cudaFree(x->count_dev); cudaFree(x->bn_acc); cudaFree(x->ones); cudaFree(x->zeros);
-    delete x;
-    g_extra.erase(h);
-  }
+  cudaFree(h->is_weight); cudaFree(h->mean); cudaFree(h->inv_std); cudaFree(h->sums); cudaFree(h->loss_dev);
+  cudaFree(h->cm_dev); cudaFree(h->count_dev); cudaFree(h->bn_acc); cudaFree(h->ones); cudaFree(h->zeros);
   for (auto& pr : h->conv_events) { cudaEventDestroy(pr.first); cudaEventDestroy(pr.second); }
   cudaEventDestroy(h->ev_a); cudaEventDestroy(h->ev_b);
   cudaStreamDestroy(h->own_stream);
@@ -765,6 +665,17 @@ __global__ void repack_kernel(const __grid_constant__ RepackTable t) {
   else reinterpret_cast<__nv_bfloat16*>(s.out)[i] = __float2bfloat16_rn(v);
 }
 
+// one filter's operand matrix of the given kind, exactly as refresh_packed builds a layer's
+static void repack_filter(Handle* h, const float* w, void* out, int taps, int ci, int co, int kind, int etype) {
+  RepackTable t;
+  memset(&t, 0, sizeof(t));
+  t.etype = etype;
+  t.seg[t.n++] = RepackSeg{w, out, taps, ci, co, kind, 0};
+  t.total = (long long)taps * ci * co;
+  repack_kernel<<<nblk(t.total, 256), 256, 0, h->stream>>>(t);
+  LAUNCH_CHECK(h);
+}
+
 // training needs only the layer operands; inference additionally the folded eval-mode BN and conv1's tensor-core operand
 static void refresh_packed(Handle* h, bool training) {
   const int et = act_type(h);
@@ -823,14 +734,21 @@ static void refresh_packed(Handle* h, bool training) {
 // ------------------------------------------------------------------------------------------------
 struct ActBuf { void* p; int cs; int co; };   // pointer, channel stride, channel offset
 
+// the shape of one convolution outside a network (the unit-test entry points), SAME-padded as build_net pads a layer
+static ConvLayer conv_shape(int k, int rate, int ci, int co) {
+  ConvLayer c;
+  c.k = k; c.rate = rate; c.ci = ci; c.co = co;
+  c.pad_b = (k - 1) * rate / 2; c.pad_a = (k - 1) * rate - c.pad_b;
+  return c;
+}
+
 static void prof_begin(Handle* h, cudaEvent_t* a, cudaEvent_t* b) {
   if (!h->time_convs) return;
-  HandleExtra* x = X(h);
-  if (x->capturing) {
+  if (h->capturing) {
     cudaEvent_t e0, e1;
     CUDA_CHECK(cudaEventCreate(&e0));
     CUDA_CHECK(cudaEventCreate(&e1));
-    x->capturing->events.push_back({e0, e1});
+    h->capturing->events.push_back({e0, e1});
     *a = e0; *b = e1;
     CUDA_CHECK(cudaEventRecordWithFlags(e0, h->stream, cudaEventRecordExternal));
     return;
@@ -848,7 +766,7 @@ static void prof_begin(Handle* h, cudaEvent_t* a, cudaEvent_t* b) {
 }
 static void prof_end(Handle* h, cudaEvent_t b) {
   if (!h->time_convs) return;
-  if (X(h)->capturing) { CUDA_CHECK(cudaEventRecordWithFlags(b, h->stream, cudaEventRecordExternal)); return; }
+  if (h->capturing) { CUDA_CHECK(cudaEventRecordWithFlags(b, h->stream, cudaEventRecordExternal)); return; }
   CUDA_CHECK(cudaEventRecord(b, h->stream));
 }
 
@@ -884,20 +802,47 @@ static void run_conv(Handle* h, const ActBuf& in, int ci, const float* w_simt, c
     launch_conv_tc(h, a);
   }
   prof_end(h, eb);
-  X(h)->conv_flops += 2.0 * (double)B * crop * crop * k * k * ci * co;
-  X(h)->conv_launches += nsplit;
+  h->conv_flops += 2.0 * (double)B * crop * crop * k * k * ci * co;
+  h->conv_launches += nsplit;
 }
 
 // ------------------------------------------------------------------------------------------------
 // inference forward (eval-mode BN folded into the conv epilogue)
 // ------------------------------------------------------------------------------------------------
-static size_t forward_eval_workspace(Handle* h, int B, int crop) {
-  const int64_t M = (int64_t)B * crop * crop;
-  const size_t es = h->cfg.precision == DRS_PREC_FP32 ? 4 : 2;
-  const int nbuf = h->net.dense ? 1 : 3;
-  size_t se_bytes = 0;
-  for (auto& sb : h->net.se) se_bytes = std::max(se_bytes, ((size_t)B * (3 * sb.c + sb.r)) * 4 + 4096);
-  return nbuf * ((size_t)M * h->net.feat_stride * es + 4096) + (size_t)M * h->net.classes * 4 + (size_t)M * 32 * es + se_bytes + 65536;
+// Every buffer the inference forward takes from the arena, in one place (see TrainWs in drs_train.cuh)
+template <typename TA>
+struct EvalWs {
+  TA* bufs[3] = {nullptr, nullptr, nullptr};   // feature buffers (dense nets: one concatenated buffer)
+  float* logits = nullptr;                     // when the caller passes no buffer
+  float* se = nullptr;                         // SE gate scratch of the widest gate: sums, means, gate, hidden
+  TA* x8 = nullptr;                            // conv1 on the tensor cores: input padded to 8 channels
+
+  void layout(const Handle* h, WsAlloc& a, int B, int crop) {
+    const NetDesc& n = h->net;
+    const int64_t M = (int64_t)B * crop * crop;
+    for (int i = 0; i < (n.dense ? 1 : 3); ++i) bufs[i] = a.take<TA>((size_t)M * n.feat_stride * sizeof(TA));
+    logits = a.take<float>((size_t)M * n.classes * 4);
+    size_t se_floats = 0;
+    for (auto& sb : n.se) se_floats = std::max(se_floats, (size_t)B * (3 * sb.c + sb.r));
+    if (se_floats) se = a.take<float>(se_floats * 4);
+    const ConvLayer& c0 = n.convs[0];
+    if (ElemTag<TA>::v != ET_F32 && conv1_tc_supported(c0.k, c0.rate, c0.ci, c0.co)) x8 = a.take<TA>((size_t)M * 8 * sizeof(TA));
+  }
+};
+
+// the bytes workspace layout W takes from the arena: a counting run of W::layout
+template <typename W>
+static size_t layout_bytes(const Handle* h, int B, int crop) {
+  WsAlloc count;
+  W().layout(h, count, B, crop);
+  return count.used;
+}
+static size_t eval_arena_bytes(const Handle* h, int B, int crop) {
+  switch (act_type(h)) {
+    case ET_F32: return layout_bytes<EvalWs<float>>(h, B, crop);
+    case ET_F16: return layout_bytes<EvalWs<__half>>(h, B, crop);
+    default: return layout_bytes<EvalWs<__nv_bfloat16>>(h, B, crop);
+  }
 }
 
 template <typename TA>
@@ -906,19 +851,14 @@ static void forward_eval_t(Handle* h, const float* x_dev, int B, int crop, float
   const int64_t M = (int64_t)B * crop * crop;
   refresh_packed(h, false);
   const int fs = n.feat_stride;
-  const size_t buf_bytes = (size_t)M * fs * sizeof(TA);
-  const int nbuf = n.dense ? 1 : 3;
-  ensure_arena(h, forward_eval_workspace(h, B, crop));
+  ensure_arena(h, layout_bytes<EvalWs<TA>>(h, B, crop));
   h->arena.reset();
-  TA* bufs[3] = {nullptr, nullptr, nullptr};
-  for (int i = 0; i < nbuf; ++i) bufs[i] = (TA*)arena_take(h, buf_bytes);
-  float* logits = logits_dev ? logits_dev : (float*)arena_take(h, (size_t)M * n.classes * 4);
-  float* se_scratch = nullptr;
+  EvalWs<TA> ws;
   {
-    size_t se_floats = 0;
-    for (auto& sb : n.se) se_floats = std::max(se_floats, (size_t)B * (3 * sb.c + sb.r));
-    if (se_floats) se_scratch = (float*)arena_take(h, se_floats * 4);
+    WsAlloc carve{&h->arena};
+    ws.layout(h, carve, B, crop);
   }
+  float* logits = logits_dev ? logits_dev : ws.logits;
   h->taps.clear();
 
   ActBuf cur{nullptr, 0, 0};
@@ -928,23 +868,22 @@ static void forward_eval_t(Handle* h, const float* x_dev, int B, int crop, float
     ConvLayer& c = n.convs[l];
     ActBuf out;
     const int sq_part = (n.squeeze && l >= 1) ? (int)((l - 1) % 3) : -1;    // 0: _s1, 1: _s2_1, 2: _s2_2 (isprs:726-742)
-    if (n.dense) out = {bufs[0], fs, c.out_coff};
-    else if (sq_part == 0) { sq_s = (xi + 1) % 3; sq_c = (xi + 2) % 3; out = {bufs[sq_s], fs, 0}; }
-    else if (sq_part >= 1) { cur = {bufs[sq_s], fs, 0}; out = {bufs[sq_c], fs, c.out_coff}; }
-    else out = {bufs[(xi + 1) % 3], fs, 0};
-    if (l == 0 && ElemTag<TA>::v != ET_F32 && c.w_fprop && conv1_tc_supported(c.k, c.rate, c.ci, c.co)) {
-      TA* x8 = (TA*)arena_take(h, (size_t)M * 8 * sizeof(TA));
-      pad_cast8_kernel<TA><<<nblk(M, 256), 256, 0, h->stream>>>(x_dev, x8, c.ci, M);
+    if (n.dense) out = {ws.bufs[0], fs, c.out_coff};
+    else if (sq_part == 0) { sq_s = (xi + 1) % 3; sq_c = (xi + 2) % 3; out = {ws.bufs[sq_s], fs, 0}; }
+    else if (sq_part >= 1) { cur = {ws.bufs[sq_s], fs, 0}; out = {ws.bufs[sq_c], fs, c.out_coff}; }
+    else out = {ws.bufs[(xi + 1) % 3], fs, 0};
+    if (l == 0 && ws.x8 && c.w_fprop) {
+      pad_cast8_kernel<TA><<<nblk(M, 256), 256, 0, h->stream>>>(x_dev, ws.x8, c.ci, M);
       LAUNCH_CHECK(h);
       cudaEvent_t ea = nullptr, eb = nullptr;
       prof_begin(h, &ea, &eb);
       Conv1TcArgs a1;
-      a1.x8 = x8; a1.wpack = c.w_fprop; a1.out = out.p; a1.out_cstride = out.cs; a1.out_coff = out.co; a1.co = c.co;
+      a1.x8 = ws.x8; a1.wpack = c.w_fprop; a1.out = out.p; a1.out_cstride = out.cs; a1.out_coff = out.co; a1.co = c.co;
       a1.B = B; a1.crop = crop; a1.scale = c.fold_scale; a1.shift = c.fold_shift; a1.act = n.act; a1.etype = ElemTag<TA>::v;
       launch_conv1_tc(h, a1);
       prof_end(h, eb);
-      X(h)->conv_flops += 2.0 * (double)M * c.k * c.k * c.ci * c.co;   // algorithmic FLOPs: the real C channels
-      X(h)->conv_launches += 1;
+      h->conv_flops += 2.0 * (double)M * c.k * c.k * c.ci * c.co;   // algorithmic FLOPs: the real C channels
+      h->conv_launches += 1;
     } else if (l == 0) {
       launch_conv_simt<float, TA>(h, x_dev, n.channels, 0, n.channels, h->params + c.w_off, (TA*)out.p, out.cs, out.co, c.co,
                                   B, crop, c.k, c.rate, c.pad_b, c.fold_scale, c.fold_shift, n.act);
@@ -958,19 +897,19 @@ static void forward_eval_t(Handle* h, const float* x_dev, int B, int crop, float
                                      h->params + n.cls_b_off, n.classes, logits, pred_dev);
       return;
     } else if (n.pool) {
-      ActBuf pout{bufs[(xi + 2) % 3], fs, 0};
+      ActBuf pout{ws.bufs[(xi + 2) % 3], fs, 0};
       launch_maxpool3_fwd<TA>(h, (const TA*)out.p, out.cs, out.co, (TA*)pout.p, pout.cs, pout.co, nullptr, c.co, B, crop);
       cur = pout;
       xi = (xi + 2) % 3;
     } else if (c.post == 1) {
-      ActBuf pout{bufs[(xi + 2) % 3], fs, 0};
+      ActBuf pout{ws.bufs[(xi + 2) % 3], fs, 0};
       launch_avgpool_fwd<TA>(h, (const TA*)out.p, out.cs, out.co, (TA*)pout.p, pout.cs, pout.co, c.co, B, crop, c.post_k);
       cur = pout;
       xi = (xi + 2) % 3;
     } else if (c.post == 2) {
       // squeeze-and-excitation gate, in place (per-image statistics: the result depends on the patch, as in the reference)
       const SeBlock& sb = n.se[c.se];
-      float* sum = se_scratch;
+      float* sum = ws.se;
       float* sv = sum + (size_t)B * sb.c;
       float* ev = sv + (size_t)B * sb.c;
       float* hv = ev + (size_t)B * sb.c;
@@ -987,9 +926,9 @@ static void forward_eval_t(Handle* h, const float* x_dev, int B, int crop, float
       xi = (xi + 1) % 3;
     } else if (sq_part >= 0) {
       if (sq_part == 0) cur = out;                       // S: read by the two expand convolutions
-      else if (sq_part == 2) { cur = {bufs[sq_c], fs, 0}; xi = sq_c; }    // the module's concatenated output
+      else if (sq_part == 2) { cur = {ws.bufs[sq_c], fs, 0}; xi = sq_c; }    // the module's concatenated output
     } else if (n.dense) {
-      cur = {bufs[0], fs, 0};
+      cur = {ws.bufs[0], fs, 0};
     } else {
       cur = out;
       xi = (xi + 1) % 3;
@@ -1051,22 +990,20 @@ extern "C" int drs_forward_host(drs_handle_t h, const float* x_host, int32_t B, 
 
 template <typename T>
 static void debug_keep(Handle* h, const std::string& name, const T* ptr, int cs, int co, int C, int64_t M) {
-  HandleExtra* x = X(h);
-  if (!x->debug_keep) return;
+  if (!h->debug_keep) return;
   float* buf = nullptr;
   CUDA_CHECK(cudaMalloc(&buf, M * C * 4));
-  x->keep.push_back(buf);
+  h->keep.push_back(buf);
   slice_to_f32_kernel<T><<<nblk(M * C, 256), 256, 0, h->stream>>>(ptr, cs, co, C, M, buf);
   LAUNCH_CHECK(h);
   h->taps[name] = {buf, ET_F32, C, 0, C, M};
 }
 static void debug_keep_reset(Handle* h) {
-  HandleExtra* x = X(h);
-  x->debug_keep = getenv("DRS_DEBUG_KEEP") != nullptr;
-  if (x->keep.empty()) return;
+  h->debug_keep = getenv("DRS_DEBUG_KEEP") != nullptr;
+  if (h->keep.empty()) return;
   cudaStreamSynchronize(h->stream);
-  for (float* p : x->keep) cudaFree(p);
-  x->keep.clear();
+  for (float* p : h->keep) cudaFree(p);
+  h->keep.clear();
 }
 
 #include "drs_train.cuh"

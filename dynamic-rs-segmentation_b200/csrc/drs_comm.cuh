@@ -78,14 +78,13 @@ extern "C" int drs_comm_init(drs_handle_t h, const uint8_t* id128, int32_t rank,
   DRS_CHECK(h && id128, "null argument");
   DRS_CHECK(world >= 1 && rank >= 0 && rank < world, "comm_init: bad rank %d of %d", rank, world);
   CUDA_CHECK(cudaSetDevice(h->cfg.device));
-  HandleExtra* x = X(h);
-  if (x->nccl) { NCCL_CHECK(nccl_api()->CommDestroy((drs_ncclComm_t)x->nccl)); x->nccl = nullptr; }
+  if (h->nccl) { NCCL_CHECK(nccl_api()->CommDestroy((drs_ncclComm_t)h->nccl)); h->nccl = nullptr; }
   drs_ncclUniqueId id;
   memcpy(id.internal, id128, 128);
   drs_ncclComm_t comm = nullptr;
   NCCL_CHECK(nccl_api()->CommInitRank(&comm, world, id, rank));
-  x->nccl = comm;
-  x->rank = rank;
+  h->nccl = comm;
+  h->rank = rank;
   h->world = world;
   h->sync_bn = sync_bn ? 1 : 0;
   h->allreduce = nullptr;
@@ -96,13 +95,12 @@ extern "C" int drs_comm_init(drs_handle_t h, const uint8_t* id128, int32_t rank,
 extern "C" int drs_comm_destroy(drs_handle_t h) {
   API_BEGIN
   DRS_CHECK(h, "null handle");
-  HandleExtra* x = X(h);
-  if (x->nccl) {
+  if (h->nccl) {
     CUDA_CHECK(cudaSetDevice(h->cfg.device));
     cudaStreamSynchronize(h->stream);
-    if (x->comm_stream) cudaStreamSynchronize(x->comm_stream);
-    NCCL_CHECK(nccl_api()->CommDestroy((drs_ncclComm_t)x->nccl));
-    x->nccl = nullptr;
+    if (h->comm_stream) cudaStreamSynchronize(h->comm_stream);
+    NCCL_CHECK(nccl_api()->CommDestroy((drs_ncclComm_t)h->nccl));
+    h->nccl = nullptr;
     h->world = 1;
   }
   API_END
@@ -112,10 +110,9 @@ extern "C" int drs_comm_destroy(drs_handle_t h) {
 static void do_allreduce(Handle* h, float* buf, int64_t count, cudaStream_t on_stream = (cudaStream_t)(uintptr_t)1) {
   if (h->world <= 1) return;
   h->pdl_prev = false;
-  HandleExtra* x = X(h);
   const cudaStream_t st = on_stream == (cudaStream_t)(uintptr_t)1 ? h->stream : on_stream;
-  if (x->nccl) {
-    NCCL_CHECK(nccl_api()->AllReduce(buf, buf, (size_t)count, DRS_NCCL_FLOAT32, DRS_NCCL_SUM, (drs_ncclComm_t)x->nccl, st));
+  if (h->nccl) {
+    NCCL_CHECK(nccl_api()->AllReduce(buf, buf, (size_t)count, DRS_NCCL_FLOAT32, DRS_NCCL_SUM, (drs_ncclComm_t)h->nccl, st));
     return;
   }
   if (!h->allreduce) return;
@@ -131,20 +128,19 @@ extern "C" int drs_scene_gather_labels(drs_handle_t h, int32_t H, int32_t W, con
   API_BEGIN
   DRS_CHECK(h && row_cuts, "null argument");
   CUDA_CHECK(cudaSetDevice(h->cfg.device));
-  HandleExtra* x = X(h);
-  DRS_CHECK(x->nccl, "scene_gather_labels: drs_comm_init has not been called");
-  const int world = h->world, rank = x->rank;
-  DRS_CHECK(x->last_scene >= 0 && x->last_W == W && x->last_row_begin == row_cuts[rank] &&
-                x->last_rows == row_cuts[rank + 1] - row_cuts[rank],
-            "scene_gather_labels: the last scene pass covered rows [%d,%d), not this rank's stripe [%d,%d)", x->last_row_begin,
-            x->last_row_begin + x->last_rows, row_cuts[rank], row_cuts[rank + 1]);
+  DRS_CHECK(h->nccl, "scene_gather_labels: drs_comm_init has not been called");
+  const int world = h->world, rank = h->rank;
+  DRS_CHECK(h->last_scene >= 0 && h->last_W == W && h->last_row_begin == row_cuts[rank] &&
+                h->last_rows == row_cuts[rank + 1] - row_cuts[rank],
+            "scene_gather_labels: the last scene pass covered rows [%d,%d), not this rank's stripe [%d,%d)", h->last_row_begin,
+            h->last_row_begin + h->last_rows, row_cuts[rank], row_cuts[rank + 1]);
   DRS_CHECK(labels_out_host || (rank != 0 && !all_ranks), "scene_gather_labels: this rank needs the output buffer");
-  const uint8_t* mine = (const uint8_t*)x->slot_ptr[4];
+  const uint8_t* mine = (const uint8_t*)h->slot_ptr[4];
   NcclApi* n = nccl_api();
-  drs_ncclComm_t comm = (drs_ncclComm_t)x->nccl;
+  drs_ncclComm_t comm = (drs_ncclComm_t)h->nccl;
   uint8_t* full = (rank == 0 || all_ranks) ? (uint8_t*)slot_buf(h, 7, (size_t)H * W) : nullptr;
   if (rank != 0) {
-    if (x->last_rows > 0) NCCL_CHECK(n->Send(mine, (size_t)x->last_rows * W, DRS_NCCL_UINT8, 0, comm, h->stream));
+    if (h->last_rows > 0) NCCL_CHECK(n->Send(mine, (size_t)h->last_rows * W, DRS_NCCL_UINT8, 0, comm, h->stream));
   } else {
     NCCL_CHECK(n->GroupStart());
     for (int r = 1; r < world; ++r) {
@@ -152,7 +148,7 @@ extern "C" int drs_scene_gather_labels(drs_handle_t h, int32_t H, int32_t W, con
       if (rows > 0) NCCL_CHECK(n->Recv(full + (size_t)row_cuts[r] * W, (size_t)rows * W, DRS_NCCL_UINT8, r, comm, h->stream));
     }
     NCCL_CHECK(n->GroupEnd());
-    CUDA_CHECK(cudaMemcpyAsync(full + (size_t)row_cuts[0] * W, mine, (size_t)x->last_rows * W, cudaMemcpyDeviceToDevice, h->stream));
+    CUDA_CHECK(cudaMemcpyAsync(full + (size_t)row_cuts[0] * W, mine, (size_t)h->last_rows * W, cudaMemcpyDeviceToDevice, h->stream));
   }
   if (all_ranks) NCCL_CHECK(n->Broadcast(full, full, (size_t)H * W, DRS_NCCL_UINT8, 0, comm, h->stream));
   if (labels_out_host && full) CUDA_CHECK(cudaMemcpyAsync(labels_out_host, full, (size_t)H * W, cudaMemcpyDeviceToHost, h->stream));

@@ -99,6 +99,19 @@ struct Scene {
   int row0 = 0, rows = 0;   // resident rows [row0, row0+rows) of the H-row scene (a rank keeps only its stripe + halo)
 };
 
+constexpr int MAX_SCENES = 64;
+struct SceneDesc {
+  const void* data;       // rows [row0, row0 + rows) of the scene
+  const uint8_t* labels;
+  int H, W, C, dtype;
+  int row0, rows;
+};
+struct SceneTable {
+  SceneDesc s[MAX_SCENES];
+};
+
+constexpr int MAX_CLASSES = 8;
+
 struct Arena {
   char* base = nullptr;
   size_t cap = 0, used = 0;
@@ -110,6 +123,45 @@ struct Arena {
     return base + off;
   }
 };
+
+struct InferLane {
+  cudaStream_t stream = nullptr;
+  Arena arena;
+  float* x = nullptr;
+  float* lg = nullptr;
+  size_t x_cap = 0, lg_cap = 0;
+  cudaEvent_t fwd_done = nullptr, acc_done = nullptr;
+};
+
+// One captured training step (CUDA graph) per (batch, patch size, buffers, learning rate): the step is ~65 small
+// dependent launches, so replaying it as a graph removes the launch gaps between them.
+struct TrainGraphKey {
+  int B, crop, ignore_label, profiling;
+  const void *x, *y, *mask, *acc_mask, *pred, *cm;
+  uint64_t lr_bits;
+  uint64_t arena_epoch;
+  bool operator<(const TrainGraphKey& o) const { return memcmp(this, &o, sizeof(*this)) < 0; }
+};
+struct TrainGraph {
+  cudaGraphExec_t exec = nullptr;
+  int64_t launches = 0, conv_launches = 0;
+  double conv_flops = 0;
+  std::vector<std::pair<cudaEvent_t, cudaEvent_t>> events;   // external event-record nodes around the tensor-core launches
+};
+
+// cell tables of an ordered position list (host)
+struct CellTables {
+  int nh, nw, stride;
+  std::vector<int32_t> off, seq;
+};
+// a scene pass's visiting order and cell tables, memoised per geometry (drs_scene_api.cuh: pass_geometry)
+struct PassGeometry {
+  int key[8];
+  std::vector<int32_t> pos, inst;
+  CellTables ct;
+};
+
+constexpr int RESULT_STRIDE = 64 + MAX_CLASSES * MAX_CLASSES;   // floats per pinned result slot: loss, then K*K+1 counts
 
 typedef CUresult (*PFN_encodeTiled)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
                                     const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
@@ -185,6 +237,63 @@ struct drs_handle_s {
   PFN_encodeTiled encodeTiled = nullptr;
   PFN_encodeIm2col encodeIm2col = nullptr;
   std::map<TmKey, CUtensorMap> tm_cache;
+
+  // persistent scene-pass buffers (score map, occurrence counts, cell tables, label map ...): cudaMalloc / cudaFree of
+  // gigabyte-sized buffers per call costs hundreds of milliseconds, so each named slot only ever grows
+  // the label map of the last scene pass stays in slot 4 for drs_scene_confusion
+  int last_scene = -1, last_row_begin = 0, last_rows = 0, last_W = 0;
+  void* slot_ptr[8] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
+  size_t slot_cap[8] = {0, 0, 0, 0, 0, 0, 0, 0};
+  std::vector<PassGeometry> pass_geometry;   // the last few scene-pass geometries, oldest first
+  std::map<TrainGraphKey, TrainGraph> graphs;
+  TrainGraph* capturing = nullptr;   // non-null while a training step is being captured
+  cudaStream_t side_stream = nullptr;     // filter gradients run here, overlapped with the backward's HBM-bound kernels
+  cudaEvent_t ev_dz[2] = {nullptr, nullptr}, ev_wgrad[2] = {nullptr, nullptr};
+  // data-parallel exchange of the late layers' gradients, overlapped with the rest of the backward
+  cudaStream_t comm_stream = nullptr;
+  cudaEvent_t ev_bucket_ready = nullptr, ev_bucket_done = nullptr;
+  cudaEvent_t ev_x8 = nullptr;          // conv1's padded input is ready: the side stream builds the im2col matrix under the forward
+  bool use_graphs = true;           // DRS_GRAPHS=0 turns the whole-step CUDA graphs off (drs_create)
+  double conv_ms_acc = 0;            // device time of profiled launches already read back
+  InferLane lane;                 // scene-inference lane (drs_scene_api.cuh)
+  cudaEvent_t lane_ready = nullptr;
+  // streamed scene upload (drs_scene_infer_host): copy stream + "rows uploaded" event
+  cudaStream_t copy_stream = nullptr;
+  cudaEvent_t up_ev[1] = {nullptr};
+  uint8_t* is_weight = nullptr;   // [n_trainable] 1 for `weights` variables
+  SceneTable table;               // host copy of the device scene table
+  // training scratch kept between calls
+  float* mean = nullptr;          // [sum co] batch mean of the last train step (per layer, same offsets as mm_off/2)
+  float* inv_std = nullptr;
+  float* sums = nullptr;          // [2*256]
+  float* loss_dev = nullptr;      // [4]: ce, l2, count, spare
+  unsigned int* cm_dev = nullptr; // [K*K+1]
+  unsigned int* count_dev = nullptr;
+  unsigned int* bn_counter = nullptr;   // last-block-done counter of bn_partial_kernel (self-resetting)
+  long long* bn_acc = nullptr;          // [BN_ACC_REPLICAS][2*512] fixed-point accumulators of bn_partial_kernel (self-clearing)
+  float* ones = nullptr;          // [512]
+  float* zeros = nullptr;         // [512]
+  // profiling
+  double conv_flops = 0;
+  int64_t conv_launches = 0;
+  // pipelined training loop (drs_gather_plan_dev / drs_train_step_async / drs_train_result): the plan of step i+1 is
+  // uploaded on plan_stream into a two-slot device staging ring while step i runs; loss + confusion counts of each step
+  // land in a ring of pinned result slots behind an event, so the host never blocks on the step it has just enqueued
+  void* nccl = nullptr;             // ncclComm_t of drs_comm_init (drs_comm.cuh); null: single process or callback exchange
+  int rank = 0;
+  cudaStream_t plan_stream = nullptr;
+  void* plan_stage[2] = {nullptr, nullptr};
+  size_t plan_stage_cap[2] = {0, 0};
+  cudaEvent_t plan_uploaded[2] = {nullptr, nullptr}, plan_consumed[2] = {nullptr, nullptr};
+  bool plan_consumed_valid[2] = {false, false};
+  int64_t plan_calls = 0;
+  static constexpr int RESULT_RING = 8;
+  float* result_host = nullptr;     // pinned [RESULT_RING][RESULT_STRIDE]
+  cudaEvent_t result_ev[RESULT_RING] = {};
+  int64_t next_ticket = 0;
+  // DRS_DEBUG_KEEP=1: fp32 copies of backward intermediates ("dz:<scope>", "da:<scope>")
+  std::vector<float*> keep;
+  bool debug_keep = false;
 };
 typedef drs_handle_s Handle;
 
@@ -204,6 +313,38 @@ static inline void* arena_take(Handle* h, size_t bytes) {
   DRS_CHECK(p != nullptr, "workspace arena exhausted (need %zu more bytes, cap %zu)", bytes, h->arena.cap);
   return p;
 }
+// What a workspace layout (TrainWs, EvalWs) runs against: with an arena it carves the buffers from it; without one it only
+// adds up what the same requests take, and that sum is what the arena is sized by.
+struct WsAlloc {
+  Arena* arena = nullptr;
+  size_t used = 0;
+  template <typename T> T* take(size_t bytes) {
+    used = round_up(used, 1024) + bytes;
+    if (!arena) return nullptr;
+    void* p = arena->take(bytes);
+    DRS_CHECK(p != nullptr, "workspace arena exhausted (need %zu more bytes, cap %zu)", bytes, arena->cap);
+    return (T*)p;
+  }
+};
+
+// Launches inside the scope go to stream `s` (and carve from `arena`, when given) if `on`; the handle's stream, arena and
+// PDL state are restored when the scope ends, also when a launch throws.  The first launch on `s` gets no programmatic
+// dependency: its predecessor on that stream is not known.
+struct StreamScope {
+  drs_handle_s* h;
+  bool on, swap_arena, pdl_prev;
+  cudaStream_t stream;
+  Arena arena;
+  StreamScope(drs_handle_s* h_, bool on_, cudaStream_t s, const Arena* a = nullptr)
+      : h(h_), on(on_), swap_arena(on_ && a), pdl_prev(h_->pdl_prev), stream(h_->stream), arena(h_->arena) {
+    if (on) { h->stream = s; h->pdl_prev = false; }
+    if (swap_arena) h->arena = *a;
+  }
+  ~StreamScope() {
+    if (on) { h->stream = stream; h->pdl_prev = pdl_prev; }
+    if (swap_arena) h->arena = arena;
+  }
+};
 static inline void ensure_pinned(Handle* h, size_t bytes) {
   if (h->pinned_cap >= bytes) return;
   CUDA_CHECK(cudaStreamSynchronize(h->stream));

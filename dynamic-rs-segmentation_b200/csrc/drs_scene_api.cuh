@@ -34,7 +34,7 @@ static void scene_upload_rows(Handle* h, int32_t scene_id, const void* rows_host
   }
   CUDA_CHECK(cudaStreamSynchronize(h->stream));
   s.H = H; s.W = W; s.C = C; s.dtype = dtype; s.row0 = row0; s.rows = rows;
-  X(h)->table.s[scene_id] = SceneDesc{s.data, s.labels, H, W, C, dtype, row0, rows};
+  h->table.s[scene_id] = SceneDesc{s.data, s.labels, H, W, C, dtype, row0, rows};
 }
 
 extern "C" int drs_scene_upload(drs_handle_t h, int32_t scene_id, const void* scene_host, int32_t H, int32_t W, int32_t C,
@@ -60,7 +60,7 @@ extern "C" int drs_scene_free(drs_handle_t h, int32_t scene_id) {
   if (it->second.data) cudaFree(it->second.data);
   if (it->second.labels) cudaFree(it->second.labels);
   h->scenes.erase(it);
-  memset(&X(h)->table.s[scene_id], 0, sizeof(SceneDesc));
+  memset(&h->table.s[scene_id], 0, sizeof(SceneDesc));
   API_END
 }
 
@@ -85,10 +85,10 @@ static void launch_gather(Handle* h, GatherParams gp, const GatherInline* il = n
   gp.fp16_patches = h->gather_fp16;
   const int64_t n = (int64_t)gp.B * gp.crop * gp.crop * gp.C;
   if (il) {
-    gather_kernel<true><<<nblk(n, 256), 256, 0, h->stream>>>(X(h)->table, gp, *il);
+    gather_kernel<true><<<nblk(n, 256), 256, 0, h->stream>>>(h->table, gp, *il);
   } else {
     static const GatherInline none = {};
-    gather_kernel<false><<<nblk(n, 256), 256, 0, h->stream>>>(X(h)->table, gp, none);
+    gather_kernel<false><<<nblk(n, 256), 256, 0, h->stream>>>(h->table, gp, none);
   }
   LAUNCH_CHECK(h);
 }
@@ -199,7 +199,6 @@ extern "C" int drs_gather_plan_dev(drs_handle_t h, const int32_t* inst_host, con
   DRS_CHECK(h && inst_host && x_out_dev, "null argument");
   DRS_CHECK(B >= 1 && crop >= 1, "gather_plan: bad B=%d crop=%d", B, crop);
   CUDA_CHECK(cudaSetDevice(h->cfg.device));
-  HandleExtra* x = X(h);
   for (int b = 0; b < B; ++b) {
     const int sid = inst_host[b * 3], r = inst_host[b * 3 + 1], c = inst_host[b * 3 + 2];
     auto it = h->scenes.find(sid);
@@ -212,22 +211,22 @@ extern "C" int drs_gather_plan_dev(drs_handle_t h, const int32_t* inst_host, con
   const size_t small = round_up((size_t)B * 12, 256) + 3 * round_up((size_t)B, 256) + round_up((size_t)B * 4, 256) +
                        round_up((size_t)B * 48, 256);
   const size_t need = small + (has_noise ? round_up((size_t)noise_count * 8, 256) : 0) + 1024;
-  const int s = (int)(x->plan_calls++ & 1);
-  if (x->plan_consumed_valid[s]) CUDA_CHECK(cudaStreamWaitEvent(x->plan_stream, x->plan_consumed[s], 0));
-  if (x->plan_stage_cap[s] < need) {
+  const int s = (int)(h->plan_calls++ & 1);
+  if (h->plan_consumed_valid[s]) CUDA_CHECK(cudaStreamWaitEvent(h->plan_stream, h->plan_consumed[s], 0));
+  if (h->plan_stage_cap[s] < need) {
     CUDA_CHECK(cudaStreamSynchronize(h->stream));
-    CUDA_CHECK(cudaStreamSynchronize(x->plan_stream));
-    if (x->plan_stage[s]) CUDA_CHECK(cudaFree(x->plan_stage[s]));
-    x->plan_stage[s] = nullptr;
-    x->plan_stage_cap[s] = 0;
+    CUDA_CHECK(cudaStreamSynchronize(h->plan_stream));
+    if (h->plan_stage[s]) CUDA_CHECK(cudaFree(h->plan_stage[s]));
+    h->plan_stage[s] = nullptr;
+    h->plan_stage_cap[s] = 0;
     const size_t want = need + (need >> 1);
-    CUDA_CHECK(cudaMalloc(&x->plan_stage[s], want));
-    x->plan_stage_cap[s] = want;
+    CUDA_CHECK(cudaMalloc(&h->plan_stage[s], want));
+    h->plan_stage_cap[s] = want;
   }
-  char* d = (char*)x->plan_stage[s];
+  char* d = (char*)h->plan_stage[s];
   auto put = [&](const void* src, size_t bytes) -> void* {
     void* dst = d;
-    CUDA_CHECK(cudaMemcpyAsync(dst, src, bytes, cudaMemcpyHostToDevice, x->plan_stream));
+    CUDA_CHECK(cudaMemcpyAsync(dst, src, bytes, cudaMemcpyHostToDevice, h->plan_stream));
     d += round_up(bytes, 256);
     return dst;
   };
@@ -244,16 +243,16 @@ extern "C" int drs_gather_plan_dev(drs_handle_t h, const int32_t* inst_host, con
     gp.noise_slot = (const int32_t*)put(noise_slot_host, (size_t)B * 4);
     gp.noise = (const double*)put(noise_host, (size_t)noise_count * 8);
   }
-  CUDA_CHECK(cudaEventRecord(x->plan_uploaded[s], x->plan_stream));
-  CUDA_CHECK(cudaStreamWaitEvent(h->stream, x->plan_uploaded[s], 0));
+  CUDA_CHECK(cudaEventRecord(h->plan_uploaded[s], h->plan_stream));
+  CUDA_CHECK(cudaStreamWaitEvent(h->stream, h->plan_uploaded[s], 0));
   gp.x_out = x_out_dev;
   gp.y_out = y_out_dev;
   gp.amask_out = amask_out_dev;
   gp.B = B;
   gp.crop = crop;
   launch_gather(h, gp);
-  CUDA_CHECK(cudaEventRecord(x->plan_consumed[s], h->stream));
-  x->plan_consumed_valid[s] = true;
+  CUDA_CHECK(cudaEventRecord(h->plan_consumed[s], h->stream));
+  h->plan_consumed_valid[s] = true;
   API_END
 }
 
@@ -272,11 +271,6 @@ extern "C" int drs_grid_positions(int32_t H, int32_t W, int32_t crop, int32_t ba
   API_END
 }
 
-// cell tables of an ordered position list (host)
-struct CellTables {
-  int nh, nw, stride;
-  std::vector<int32_t> off, seq;
-};
 static void build_cells(const std::vector<int32_t>& pos, int H, int W, int crop, CellTables& ct) {
   const int stride = crop / 2;
   ct.stride = stride;
@@ -379,8 +373,7 @@ extern "C" int drs_accumulate_argmax(drs_handle_t h, const float* logits_dev, co
 // stream, chunk after chunk, so per-pixel sums keep the script's visiting order.  The lane is kept in the handle between
 // calls (its workspace is several GB for a Potsdam tile).
 static void lane_release(Handle* h) {
-  HandleExtra* x = X(h);
-  InferLane& L = x->lane;
+  InferLane& L = h->lane;
   if (L.stream) { cudaStreamSynchronize(L.stream); cudaStreamDestroy(L.stream); }
   if (L.arena.base) cudaFree(L.arena.base);
   if (L.x) cudaFree(L.x);
@@ -388,13 +381,12 @@ static void lane_release(Handle* h) {
   if (L.fwd_done) cudaEventDestroy(L.fwd_done);
   if (L.acc_done) cudaEventDestroy(L.acc_done);
   L = InferLane();
-  if (x->lane_ready) cudaEventDestroy(x->lane_ready);
-  x->lane_ready = nullptr;
+  if (h->lane_ready) cudaEventDestroy(h->lane_ready);
+  h->lane_ready = nullptr;
 }
 static void lane_ensure(Handle* h, size_t arena_bytes, size_t x_bytes, size_t lg_bytes) {
-  HandleExtra* x = X(h);
-  if (!x->lane_ready) CUDA_CHECK(cudaEventCreateWithFlags(&x->lane_ready, cudaEventDisableTiming));
-  InferLane& L = x->lane;
+  if (!h->lane_ready) CUDA_CHECK(cudaEventCreateWithFlags(&h->lane_ready, cudaEventDisableTiming));
+  InferLane& L = h->lane;
   if (!L.stream) {
     CUDA_CHECK(cudaStreamCreateWithFlags(&L.stream, cudaStreamNonBlocking));
     CUDA_CHECK(cudaEventCreateWithFlags(&L.fwd_done, cudaEventDisableTiming));
@@ -426,7 +418,6 @@ struct HostSceneFeed {
 };
 
 static void feed_rows(Handle* h, HostSceneFeed& f, const Scene& sc, int rows_needed, cudaStream_t consumer) {
-  HandleExtra* x = X(h);
   if (rows_needed > sc.H) rows_needed = sc.H;
   bool any = false;
   const int rows_per_piece = (int)std::max<size_t>(1, ((size_t)8 << 20) / f.row_bytes);
@@ -435,17 +426,17 @@ static void feed_rows(Handle* h, HostSceneFeed& f, const Scene& sc, int rows_nee
     // Pageable source: the driver stages the piece itself (measured faster than a memcpy into our own pinned ring) and
     // returns once the source has been read; kernels already queued keep the GPU busy meanwhile.
     CUDA_CHECK(cudaMemcpyAsync((char*)sc.data + (size_t)f.uploaded * f.row_bytes, f.host + (size_t)f.uploaded * f.row_bytes,
-                               (size_t)n * f.row_bytes, cudaMemcpyHostToDevice, x->copy_stream));
+                               (size_t)n * f.row_bytes, cudaMemcpyHostToDevice, h->copy_stream));
     f.uploaded += n;
     any = true;
   }
   if (any) {
-    CUDA_CHECK(cudaEventRecord(x->up_ev[0], x->copy_stream));
+    CUDA_CHECK(cudaEventRecord(h->up_ev[0], h->copy_stream));
     f.recorded = true;
   }
   // The consumer waits for the latest "rows uploaded" event (copies on one stream complete in order, so it covers every
   // earlier piece).
-  if (f.recorded) CUDA_CHECK(cudaStreamWaitEvent(consumer, x->up_ev[0], 0));
+  if (f.recorded) CUDA_CHECK(cudaStreamWaitEvent(consumer, h->up_ev[0], 0));
 }
 
 static void scene_infer_impl(drs_handle_t h, int32_t scene_id, int32_t crop, int32_t batch, int32_t variant, int32_t row_begin,
@@ -467,7 +458,6 @@ extern "C" int drs_scene_infer_host(drs_handle_t h, int32_t scene_id, const void
   DRS_CHECK(scene_id >= 0 && scene_id < MAX_SCENES, "scene_id %d out of range [0,%d)", scene_id, MAX_SCENES);
   DRS_CHECK(dtype == DRS_SCENE_F64 || dtype == DRS_SCENE_F32, "bad scene dtype %d", dtype);
   DRS_CHECK(C == h->net.channels, "scene has %d channels, net expects %d", C, h->net.channels);
-  HandleExtra* x = X(h);
   Scene& s = h->scenes[scene_id];
   CUDA_CHECK(cudaStreamSynchronize(h->stream));
   const size_t row_bytes = (size_t)W * C * (dtype == DRS_SCENE_F64 ? 8 : 4);
@@ -480,9 +470,9 @@ extern "C" int drs_scene_infer_host(drs_handle_t h, int32_t scene_id, const void
   }
   if (s.labels) { CUDA_CHECK(cudaFree(s.labels)); s.labels = nullptr; s.labels_cap = 0; }
   s.H = H; s.W = W; s.C = C; s.dtype = dtype; s.row0 = 0; s.rows = H;
-  x->table.s[scene_id] = SceneDesc{s.data, s.labels, H, W, C, dtype, 0, H};
-  if (!x->copy_stream) CUDA_CHECK(cudaStreamCreateWithFlags(&x->copy_stream, cudaStreamNonBlocking));
-  if (!x->up_ev[0]) CUDA_CHECK(cudaEventCreateWithFlags(&x->up_ev[0], cudaEventDisableTiming));
+  h->table.s[scene_id] = SceneDesc{s.data, s.labels, H, W, C, dtype, 0, H};
+  if (!h->copy_stream) CUDA_CHECK(cudaStreamCreateWithFlags(&h->copy_stream, cudaStreamNonBlocking));
+  if (!h->up_ev[0]) CUDA_CHECK(cudaEventCreateWithFlags(&h->up_ev[0], cudaEventDisableTiming));
   HostSceneFeed feed;
   feed.host = (const char*)scene_host;
   feed.row_bytes = row_bytes;
@@ -490,16 +480,8 @@ extern "C" int drs_scene_infer_host(drs_handle_t h, int32_t scene_id, const void
   API_END
 }
 
-struct PassGeometry {
-  int key[8];
-  std::vector<int32_t> pos, inst;
-  CellTables ct;
-};
-static std::map<Handle*, std::vector<PassGeometry>> g_pass_geometry;
-static void pass_geometry_release(Handle* h) { g_pass_geometry.erase(h); }
-
 static PassGeometry& pass_geometry(Handle* h, int scene_id, int H, int W, int crop, int batch, int variant, int row_begin, int row_end) {
-  std::vector<PassGeometry>& cache = g_pass_geometry[h];
+  std::vector<PassGeometry>& cache = h->pass_geometry;
   const int key[8] = {scene_id, H, W, crop, batch, variant, row_begin, row_end};
   for (auto& g : cache)
     if (memcmp(g.key, key, sizeof(key)) == 0) return g;
@@ -549,14 +531,10 @@ static void scene_infer_impl(drs_handle_t h, int32_t scene_id, int32_t crop, int
   int chunk = (int)std::max<int64_t>(1, std::min<int64_t>(P, (target_tiles * CONV_TC_BM) / pp));
   ScenePass sp;
   int32_t* inst_dev = nullptr;
-  HandleExtra* hx = X(h);
-  cudaStream_t main_stream = h->stream;
-  Arena main_arena = h->arena;
+  const cudaStream_t main_stream = h->stream;
   auto cleanup = [&]() {
-    h->stream = main_stream;
-    h->arena = main_arena;
     cudaStreamSynchronize(main_stream);
-    if (hx->lane.stream) cudaStreamSynchronize(hx->lane.stream);
+    if (h->lane.stream) cudaStreamSynchronize(h->lane.stream);
     sp.release();
   };
   try {
@@ -565,42 +543,41 @@ static void scene_infer_impl(drs_handle_t h, int32_t scene_id, int32_t crop, int
     inst_dev = (int32_t*)slot_buf(h, 6, std::max<size_t>(inst.size(), 1) * 4);
     CUDA_CHECK(cudaMemcpyAsync(inst_dev, inst.data(), inst.size() * 4, cudaMemcpyHostToDevice, h->stream));
     refresh_packed(h, false);                       // packed weights / folded BN once, before the lane starts
-    lane_ensure(h, forward_eval_workspace(h, chunk, crop), (size_t)chunk * pp * C * 4, (size_t)chunk * pp * K * 4);
-    InferLane& L = hx->lane;
-    CUDA_CHECK(cudaEventRecord(hx->lane_ready, main_stream));
-    CUDA_CHECK(cudaStreamWaitEvent(L.stream, hx->lane_ready, 0));
+    lane_ensure(h, eval_arena_bytes(h, chunk, crop), (size_t)chunk * pp * C * 4, (size_t)chunk * pp * K * 4);
+    InferLane& L = h->lane;
+    CUDA_CHECK(cudaEventRecord(h->lane_ready, main_stream));
+    CUDA_CHECK(cudaStreamWaitEvent(L.stream, h->lane_ready, 0));
     for (int s0 = 0; s0 < P; s0 += chunk) {
       const int nb = std::min(chunk, P - s0);
-      h->stream = L.stream;
-      h->arena = L.arena;
-      if (s0 > 0) CUDA_CHECK(cudaStreamWaitEvent(L.stream, L.acc_done, 0));   // logits buffer of the previous chunk consumed
-      if (feed) {
-        // rows this chunk's patches read, plus one more chunk's worth so that the copy runs ahead of the compute
-        int need = 0;
-        const int s1 = std::min(P, s0 + 2 * chunk);
-        for (int s = s0; s < s1; ++s) need = std::max(need, pos[2 * s] + crop);
-        feed_rows(h, *feed, sc, need, L.stream);
+      {                                              // gather + forward of the chunk on the lane
+        StreamScope on_lane(h, true, L.stream, &L.arena);
+        if (s0 > 0) CUDA_CHECK(cudaStreamWaitEvent(L.stream, L.acc_done, 0));   // logits buffer of the previous chunk consumed
+        if (feed) {
+          // rows this chunk's patches read, plus one more chunk's worth so that the copy runs ahead of the compute
+          int need = 0;
+          const int s1 = std::min(P, s0 + 2 * chunk);
+          for (int s = s0; s < s1; ++s) need = std::max(need, pos[2 * s] + crop);
+          feed_rows(h, *feed, sc, need, L.stream);
+        }
+        GatherParams gp;
+        memset(&gp, 0, sizeof(gp));
+        gp.inst = inst_dev + (size_t)s0 * 3;
+        gp.x_out = L.x;
+        gp.B = nb;
+        gp.crop = crop;
+        launch_gather(h, gp);
+        forward_eval(h, L.x, nb, crop, L.lg, nullptr);
+        CUDA_CHECK(cudaEventRecord(L.fwd_done, L.stream));
       }
-      GatherParams gp;
-      memset(&gp, 0, sizeof(gp));
-      gp.inst = inst_dev + (size_t)s0 * 3;
-      gp.x_out = L.x;
-      gp.B = nb;
-      gp.crop = crop;
-      launch_gather(h, gp);
-      forward_eval(h, L.x, nb, crop, L.lg, nullptr);
-      CUDA_CHECK(cudaEventRecord(L.fwd_done, L.stream));
-      h->stream = main_stream;
-      h->arena = main_arena;
       CUDA_CHECK(cudaStreamWaitEvent(main_stream, L.fwd_done, 0));
       accumulate_chunk(h, sp, ct, L.lg, pos, s0, s0 + nb, H, W, K, crop, row_begin, row_end);
       CUDA_CHECK(cudaEventRecord(L.acc_done, main_stream));
     }
     scene_pass_finish(h, sp, rows, W, K, labels_out_host, mean_out_host);
-    hx->last_scene = scene_id; hx->last_row_begin = row_begin; hx->last_rows = rows; hx->last_W = W;
+    h->last_scene = scene_id; h->last_row_begin = row_begin; h->last_rows = rows; h->last_W = W;
     if (feed) {                                      // rows no patch reads (none for the grids of the scripts) and the tail
       feed_rows(h, *feed, sc, sc.H, main_stream);
-      CUDA_CHECK(cudaStreamSynchronize(hx->copy_stream));
+      CUDA_CHECK(cudaStreamSynchronize(h->copy_stream));
     }
   } catch (...) { cleanup(); throw; }
   cleanup();
@@ -614,21 +591,20 @@ extern "C" int drs_scene_confusion(drs_handle_t h, int32_t scene_id, int32_t K, 
   DRS_CHECK(h && cm_out_host, "null argument");
   DRS_CHECK(K >= 1 && K <= MAX_CLASSES, "K=%d out of range", K);
   CUDA_CHECK(cudaSetDevice(h->cfg.device));
-  HandleExtra* x = X(h);
   auto it = h->scenes.find(scene_id);
   DRS_CHECK(it != h->scenes.end(), "scene_confusion: scene %d not uploaded", scene_id);
   const Scene& sc = it->second;
   DRS_CHECK(sc.labels, "scene_confusion: scene %d was uploaded without labels", scene_id);
-  DRS_CHECK(x->last_scene == scene_id && x->slot_ptr[4], "scene_confusion: no label map of scene %d is resident (run drs_scene_infer first)", scene_id);
-  DRS_CHECK(x->last_W == sc.W && x->last_row_begin >= sc.row0 && x->last_row_begin + x->last_rows <= sc.row0 + sc.rows,
-            "scene_confusion: label rows [%d,%d) outside the resident ground truth", x->last_row_begin, x->last_row_begin + x->last_rows);
-  const int64_t n = (int64_t)x->last_rows * sc.W;
-  const uint8_t* truth = sc.labels + (int64_t)(x->last_row_begin - sc.row0) * sc.W;
-  CUDA_CHECK(cudaMemsetAsync(x->cm_dev, 0, (K * K + 1) * 4, h->stream));
+  DRS_CHECK(h->last_scene == scene_id && h->slot_ptr[4], "scene_confusion: no label map of scene %d is resident (run drs_scene_infer first)", scene_id);
+  DRS_CHECK(h->last_W == sc.W && h->last_row_begin >= sc.row0 && h->last_row_begin + h->last_rows <= sc.row0 + sc.rows,
+            "scene_confusion: label rows [%d,%d) outside the resident ground truth", h->last_row_begin, h->last_row_begin + h->last_rows);
+  const int64_t n = (int64_t)h->last_rows * sc.W;
+  const uint8_t* truth = sc.labels + (int64_t)(h->last_row_begin - sc.row0) * sc.W;
+  CUDA_CHECK(cudaMemsetAsync(h->cm_dev, 0, (K * K + 1) * 4, h->stream));
   const unsigned blocks = (unsigned)std::min<int64_t>(ceil_div(std::max<int64_t>(n, 1), 256), (int64_t)h->sm_count * 8);
-  confusion_kernel<<<blocks, 256, 0, h->stream>>>(truth, (const uint8_t*)x->slot_ptr[4], nullptr, n, K, ignore_label, x->cm_dev);
+  confusion_kernel<<<blocks, 256, 0, h->stream>>>(truth, (const uint8_t*)h->slot_ptr[4], nullptr, n, K, ignore_label, h->cm_dev);
   LAUNCH_CHECK(h);
-  CUDA_CHECK(cudaMemcpyAsync(cm_out_host, x->cm_dev, (K * K + 1) * 4, cudaMemcpyDeviceToHost, h->stream));
+  CUDA_CHECK(cudaMemcpyAsync(cm_out_host, h->cm_dev, (K * K + 1) * 4, cudaMemcpyDeviceToHost, h->stream));
   CUDA_CHECK(cudaStreamSynchronize(h->stream));
   API_END
 }
@@ -639,12 +615,11 @@ extern "C" int drs_confusion_dev(drs_handle_t h, const uint8_t* truth_dev, const
   DRS_CHECK(h && truth_dev && pred_dev && cm_out_host, "null argument");
   DRS_CHECK(K >= 1 && K <= MAX_CLASSES, "K=%d out of range", K);
   CUDA_CHECK(cudaSetDevice(h->cfg.device));
-  HandleExtra* x = X(h);
-  CUDA_CHECK(cudaMemsetAsync(x->cm_dev, 0, (K * K + 1) * 4, h->stream));
+  CUDA_CHECK(cudaMemsetAsync(h->cm_dev, 0, (K * K + 1) * 4, h->stream));
   const unsigned blocks = (unsigned)std::min<int64_t>(ceil_div(std::max<int64_t>(n, 1), 256), (int64_t)h->sm_count * 8);
-  confusion_kernel<<<blocks, 256, 0, h->stream>>>(truth_dev, pred_dev, mask_dev, n, K, ignore_label, x->cm_dev);
+  confusion_kernel<<<blocks, 256, 0, h->stream>>>(truth_dev, pred_dev, mask_dev, n, K, ignore_label, h->cm_dev);
   LAUNCH_CHECK(h);
-  CUDA_CHECK(cudaMemcpyAsync(cm_out_host, x->cm_dev, (K * K + 1) * 4, cudaMemcpyDeviceToHost, h->stream));
+  CUDA_CHECK(cudaMemcpyAsync(cm_out_host, h->cm_dev, (K * K + 1) * 4, cudaMemcpyDeviceToHost, h->stream));
   CUDA_CHECK(cudaStreamSynchronize(h->stream));
   API_END
 }
@@ -657,9 +632,9 @@ extern "C" int drs_set_profiling(drs_handle_t h, int32_t on) {
   DRS_CHECK(h, "null handle");
   h->time_convs = on != 0;
   h->conv_events_used = 0;
-  X(h)->conv_flops = 0;
-  X(h)->conv_launches = 0;
-  X(h)->conv_ms_acc = 0;
+  h->conv_flops = 0;
+  h->conv_launches = 0;
+  h->conv_ms_acc = 0;
   API_END
 }
 // Sum of the device time of the tensor-core convolution launches recorded since drs_set_profiling(1)
@@ -668,19 +643,19 @@ extern "C" int drs_profile_read(drs_handle_t h, float* conv_ms, int64_t* conv_la
   API_BEGIN
   DRS_CHECK(h, "null handle");
   CUDA_CHECK(cudaStreamSynchronize(h->stream));
-  float total = (float)X(h)->conv_ms_acc;
-  X(h)->conv_ms_acc = 0;
+  float total = (float)h->conv_ms_acc;
+  h->conv_ms_acc = 0;
   for (size_t i = 0; i < h->conv_events_used; ++i) {
     float ms = 0.0f;
     CUDA_CHECK(cudaEventElapsedTime(&ms, h->conv_events[i].first, h->conv_events[i].second));
     total += ms;
   }
   if (conv_ms) *conv_ms = total;
-  if (conv_launches) *conv_launches = X(h)->conv_launches;
-  if (conv_flops) *conv_flops = X(h)->conv_flops;
+  if (conv_launches) *conv_launches = h->conv_launches;
+  if (conv_flops) *conv_flops = h->conv_flops;
   h->conv_events_used = 0;
-  X(h)->conv_flops = 0;
-  X(h)->conv_launches = 0;
+  h->conv_flops = 0;
+  h->conv_launches = 0;
   API_END
 }
 extern "C" int drs_last_conv_ms(drs_handle_t h, float* ms_out) { return drs_profile_read(h, ms_out, nullptr, nullptr); }
@@ -705,7 +680,20 @@ extern "C" int drs_debug_activation(drs_handle_t h, const char* name, float* out
   API_END
 }
 
-// One convolution through the production kernels (unit tests): y = act(conv(x, w) * scale + shift)
+// One convolution through the production path (unit tests): y = act(conv(x, w) * scale + shift).  16-bit precisions cast
+// the input and pack the filter as refresh_packed packs a layer's.
+template <typename T>
+static void debug_conv_tc(Handle* h, const float* x32, const float* w32, const float* sc, const float* sh, const ConvLayer& c, int B,
+                          int crop, int act, T* xa, void* wp, T* ya, float* y32) {
+  const int64_t M = (int64_t)B * crop * crop;
+  cast_kernel<float, T><<<nblk(M * c.ci, 256), 256, 0, h->stream>>>(x32, xa, M * c.ci);
+  LAUNCH_CHECK(h);
+  repack_filter(h, w32, wp, c.k * c.k, c.ci, c.co, 0, ElemTag<T>::v);
+  run_conv<T>(h, ActBuf{xa, c.ci, 0}, c.ci, w32, wp, ActBuf{ya, c.co, 0}, c.co, B, crop, c.k, c.rate, c.pad_b, sc, sh, act);
+  cast_kernel<T, float><<<nblk(M * c.co, 256), 256, 0, h->stream>>>(ya, y32, M * c.co);
+  LAUNCH_CHECK(h);
+}
+
 extern "C" int drs_debug_conv(drs_handle_t h, const float* x_host, const float* w_host, const float* scale_host, const float* shift_host,
                               int32_t B, int32_t crop, int32_t k, int32_t rate, int32_t Ci, int32_t Co, int32_t act, int32_t precision,
                               float* y_host) {
@@ -713,9 +701,8 @@ extern "C" int drs_debug_conv(drs_handle_t h, const float* x_host, const float* 
   DRS_CHECK(h && x_host && w_host && scale_host && shift_host && y_host, "null argument");
   CUDA_CHECK(cudaSetDevice(h->cfg.device));
   const int64_t M = (int64_t)B * crop * crop;
-  const int taps = k * k;
-  const int64_t nw = (int64_t)taps * Ci * Co;
-  const int pad_b = ((k - 1) * rate) / 2;
+  const int64_t nw = (int64_t)k * k * Ci * Co;
+  const ConvLayer c = conv_shape(k, rate, Ci, Co);
   float *x32 = nullptr, *w32 = nullptr, *sc = nullptr, *sh = nullptr, *y32 = nullptr;
   void *xa = nullptr, *wp = nullptr, *ya = nullptr;
   auto cleanup = [&]() {
@@ -732,28 +719,13 @@ extern "C" int drs_debug_conv(drs_handle_t h, const float* x_host, const float* 
     CUDA_CHECK(cudaMemcpyAsync(sc, scale_host, Co * 4, cudaMemcpyHostToDevice, h->stream));
     CUDA_CHECK(cudaMemcpyAsync(sh, shift_host, Co * 4, cudaMemcpyHostToDevice, h->stream));
     if (precision == DRS_PREC_FP32) {
-      launch_conv_simt<float, float>(h, x32, Ci, 0, Ci, w32, y32, Co, 0, Co, B, crop, k, rate, pad_b, sc, sh, act);
+      run_conv<float>(h, ActBuf{x32, Ci, 0}, Ci, w32, nullptr, ActBuf{y32, Co, 0}, Co, B, crop, k, rate, c.pad_b, sc, sh, act);
     } else {
       CUDA_CHECK(cudaMalloc(&xa, M * Ci * 2));
       CUDA_CHECK(cudaMalloc(&wp, nw * 2));
       CUDA_CHECK(cudaMalloc(&ya, M * Co * 2));
-      ConvTcArgs a;
-      a.in = xa; a.in_cstride = Ci; a.in_coff = 0; a.ci = Ci; a.w = wp; a.out = ya; a.out_cstride = Co; a.out_coff = 0; a.co = Co;
-      a.B = B; a.crop = crop; a.k = k; a.rate = rate; a.pad_b = pad_b; a.scale = sc; a.shift = sh; a.act = act;
-      if (precision == DRS_PREC_F16) {
-        cast_kernel<float, __half><<<nblk(M * Ci, 256), 256, 0, h->stream>>>(x32, (__half*)xa, M * Ci);
-        pack_fprop_kernel<__half><<<nblk(nw, 256), 256, 0, h->stream>>>(w32, (__half*)wp, taps, Ci, Co);
-        a.etype = ET_F16;
-        launch_conv_tc(h, a);
-        cast_kernel<__half, float><<<nblk(M * Co, 256), 256, 0, h->stream>>>((const __half*)ya, y32, M * Co);
-      } else {
-        cast_kernel<float, __nv_bfloat16><<<nblk(M * Ci, 256), 256, 0, h->stream>>>(x32, (__nv_bfloat16*)xa, M * Ci);
-        pack_fprop_kernel<__nv_bfloat16><<<nblk(nw, 256), 256, 0, h->stream>>>(w32, (__nv_bfloat16*)wp, taps, Ci, Co);
-        a.etype = ET_BF16;
-        launch_conv_tc(h, a);
-        cast_kernel<__nv_bfloat16, float><<<nblk(M * Co, 256), 256, 0, h->stream>>>((const __nv_bfloat16*)ya, y32, M * Co);
-      }
-      h->launches += 3;
+      if (precision == DRS_PREC_F16) debug_conv_tc<__half>(h, x32, w32, sc, sh, c, B, crop, act, (__half*)xa, wp, (__half*)ya, y32);
+      else debug_conv_tc<__nv_bfloat16>(h, x32, w32, sc, sh, c, B, crop, act, (__nv_bfloat16*)xa, wp, (__nv_bfloat16*)ya, y32);
     }
     CUDA_CHECK(cudaMemcpyAsync(y_host, y32, M * Co * 4, cudaMemcpyDeviceToHost, h->stream));
     int rc = drs_synchronize(h);
@@ -827,7 +799,7 @@ extern "C" int drs_bench_conv(drs_handle_t h, int32_t B, int32_t crop, int32_t k
   API_END
 }
 
-// Filter gradient of one convolution through the production kernels (unit tests)
+// Filter gradient of one convolution through the training step's filter-gradient phase (unit tests)
 extern "C" int drs_debug_wgrad(drs_handle_t h, const float* x_host, const float* dy_host, int32_t B, int32_t crop, int32_t k,
                                int32_t rate, int32_t Ci, int32_t Co, int32_t precision, float* dw_host) {
   API_BEGIN
@@ -835,8 +807,7 @@ extern "C" int drs_debug_wgrad(drs_handle_t h, const float* x_host, const float*
   CUDA_CHECK(cudaSetDevice(h->cfg.device));
   const int64_t M = (int64_t)B * crop * crop;
   const int64_t nw = (int64_t)k * k * Ci * Co;
-  const int pad_b = ((k - 1) * rate) / 2;
-  const int max_splits = 48;
+  const ConvLayer c = conv_shape(k, rate, Ci, Co);
   float *x32 = nullptr, *dy32 = nullptr, *dw = nullptr, *part = nullptr;
   void *xa = nullptr, *dya = nullptr;
   auto cleanup = [&]() { cudaFree(x32); cudaFree(dy32); cudaFree(dw); cudaFree(part); cudaFree(xa); cudaFree(dya); };
@@ -845,12 +816,12 @@ extern "C" int drs_debug_wgrad(drs_handle_t h, const float* x_host, const float*
     CUDA_CHECK(cudaMalloc(&dy32, M * Co * 4));
     CUDA_CHECK(cudaMalloc(&dw, nw * 4));
     // (the tensor-core kernel runs 32-channel operands as 64: its split partials have the padded shape)
-    const int64_t nw_pad = (int64_t)k * k * ((Ci + 63) / 64 * 64) * ((Co + 63) / 64 * 64);
-    CUDA_CHECK(cudaMalloc(&part, nw_pad * 4 * max_splits));
+    const size_t part_cap = (size_t)k * k * ((Ci + 63) / 64 * 64) * ((Co + 63) / 64 * 64) * WGRAD_MAX_SPLITS;
+    CUDA_CHECK(cudaMalloc(&part, part_cap * 4));
     CUDA_CHECK(cudaMemcpyAsync(x32, x_host, M * Ci * 4, cudaMemcpyHostToDevice, h->stream));
     CUDA_CHECK(cudaMemcpyAsync(dy32, dy_host, M * Co * 4, cudaMemcpyHostToDevice, h->stream));
     if (precision == DRS_PREC_FP32) {
-      launch_wgrad_simt<float, float>(h, x32, Ci, 0, Ci, dy32, Co, 0, Co, dw, part, max_splits, B, crop, k, rate, pad_b);
+      filter_gradient<float>(h, c, ActBuf{x32, Ci, 0}, nullptr, nullptr, dy32, B, crop, dw, part, part_cap);
     } else {
       DRS_CHECK(precision == DRS_PREC_BF16, "debug_wgrad: precision must be FP32 or BF16");
       CUDA_CHECK(cudaMalloc(&xa, M * Ci * 2));
@@ -858,12 +829,7 @@ extern "C" int drs_debug_wgrad(drs_handle_t h, const float* x_host, const float*
       cast_kernel<float, __nv_bfloat16><<<nblk(M * Ci, 256), 256, 0, h->stream>>>(x32, (__nv_bfloat16*)xa, M * Ci);
       cast_kernel<float, __nv_bfloat16><<<nblk(M * Co, 256), 256, 0, h->stream>>>(dy32, (__nv_bfloat16*)dya, M * Co);
       h->launches += 2;
-      WgradTcArgs wa;
-      wa.x = xa; wa.in_cstride = Ci; wa.in_coff = 0; wa.ci = Ci;
-      wa.dy = dya; wa.dy_cstride = Co; wa.dy_coff = 0; wa.co = Co;
-      wa.B = B; wa.crop = crop; wa.k = k; wa.rate = rate; wa.pad_b = pad_b;
-      wa.dw = dw; wa.part = part; wa.part_capacity = (size_t)nw_pad * max_splits;
-      launch_wgrad_tc(h, wa);
+      filter_gradient<__nv_bfloat16>(h, c, ActBuf{xa, Ci, 0}, nullptr, nullptr, (const __nv_bfloat16*)dya, B, crop, dw, part, part_cap);
     }
     CUDA_CHECK(cudaMemcpyAsync(dw_host, dw, nw * 4, cudaMemcpyDeviceToHost, h->stream));
     int rc = drs_synchronize(h);

@@ -736,8 +736,6 @@ __global__ void add_slice_kernel(T* __restrict__ dst, int d_cs, int d_co, const 
 // conv_classifier (1x1, Ci -> K, bias, no BN/act)  isprs:779-786  + tf.argmax(logits, 3) isprs:1690
 // One warp per pixel: lanes stride the channels (coalesced), shuffle-reduce K partial sums.
 // ------------------------------------------------------------------------------------------------
-constexpr int MAX_CLASSES = 8;
-
 // Tile kernel: a block stages [CLS_TILE pixels x Ci] in shared memory with coalesced 16-byte loads (128B-swizzled
 // rows, so that the row-per-thread reads below are conflict-free), then thread r owns pixel r: Ci*K FMAs against
 // weights broadcast from shared memory, first-maximum argmax, one K-float row of logits out.  No shuffles.
@@ -1316,10 +1314,6 @@ template <typename TI, typename TO>
 __global__ void cast_kernel(const TI* __restrict__ in, TO* __restrict__ out, int64_t n) {
   const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i < n) out[i] = from_f32<TO>(to_f32(in[i]));
-}
-__global__ void fill_kernel(float* __restrict__ p, float v, int64_t n) {
-  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i < n) p[i] = v;
 }
 // strided 2-D slice -> dense fp32 (debug taps)
 template <typename T>

@@ -7,17 +7,6 @@
 
 #include "drs_common.cuh"
 
-constexpr int MAX_SCENES = 64;
-struct SceneDesc {
-  const void* data;       // rows [row0, row0 + rows) of the scene
-  const uint8_t* labels;
-  int H, W, C, dtype;
-  int row0, rows;
-};
-struct SceneTable {
-  SceneDesc s[MAX_SCENES];
-};
-
 constexpr int GATHER_INLINE_MAX = 256;
 // Small batches carry their instance table inside the kernel parameters: no staging copy, no host synchronisation.
 struct GatherInline {
