@@ -99,7 +99,7 @@ static void build_net(NetDesc& n, const drs_config& cfg) {
       c.post = 2; c.se = (int)n.se.size();
       n.se.push_back(sb);
     }
-    n.convs.push_back(c);
+    n.convs.push_back(std::move(c));
     if (n.dense) { feat += c.co; cin = feat; } else cin = c.co;
   }
   if (n.squeeze) {
@@ -129,7 +129,7 @@ static void build_net(NetDesc& n, const drs_config& cfg) {
         c.b_off = off; off += c.co;
         c.mm_off = boff; boff += c.co;
         c.mv_off = boff; boff += c.co;
-        n.convs.push_back(c);
+        n.convs.push_back(std::move(c));
       }
       prev_group = s1 + 1;
       prev_cs = q.out;
@@ -152,31 +152,6 @@ static void build_net(NetDesc& n, const drs_config& cfg) {
 extern "C" const char* drs_last_error(void) { return g_drs_err; }
 extern "C" int drs_version(void) { return DRS_VERSION; }
 
-static void* slot_buf(Handle* h, int slot, size_t bytes) {
-  if (bytes == 0) bytes = 16;
-  if (h->slot_cap[slot] < bytes) {
-    CUDA_CHECK(cudaStreamSynchronize(h->stream));
-    if (h->slot_ptr[slot]) CUDA_CHECK(cudaFree(h->slot_ptr[slot]));
-    h->slot_ptr[slot] = nullptr;
-    h->slot_cap[slot] = 0;
-    CUDA_CHECK(cudaMalloc(&h->slot_ptr[slot], bytes));
-    h->slot_cap[slot] = bytes;
-  }
-  return h->slot_ptr[slot];
-}
-static void lane_release(Handle* h);
-
-static void free_packed(Handle* h) {
-  for (auto& c : h->net.convs) {
-    if (c.w_fprop) cudaFree(c.w_fprop);
-    if (c.w_dgrad) cudaFree(c.w_dgrad);
-    if (c.fold_scale) cudaFree(c.fold_scale);
-    if (c.fold_shift) cudaFree(c.fold_shift);
-    c.w_fprop = c.w_dgrad = nullptr;
-    c.fold_scale = c.fold_shift = nullptr;
-  }
-}
-
 extern "C" int drs_create(drs_handle_t* out, const drs_config* cfg) {
   API_BEGIN
   DRS_CHECK(out && cfg, "drs_create: null argument");
@@ -188,22 +163,22 @@ extern "C" int drs_create(drs_handle_t* out, const drs_config* cfg) {
   cudaDeviceProp prop;
   CUDA_CHECK(cudaGetDeviceProperties(&prop, cfg->device));
   DRS_CHECK(prop.major == 10, "drs_create: device %s is sm_%d%d; libdrs is built for sm_100a only", prop.name, prop.major, prop.minor);
-  Handle* h = new Handle();
+  std::unique_ptr<Handle> h(new Handle());   // everything created below is released with it if a later step throws
   h->cfg = *cfg;
   h->sm_count = prop.multiProcessorCount;
   CUDA_CHECK(cudaDriverGetVersion(&h->driver_version));
   build_net(h->net, *cfg);
-  CUDA_CHECK(cudaStreamCreateWithFlags(&h->own_stream, cudaStreamNonBlocking));
+  h->own_stream = new_stream();
   h->stream = h->own_stream;
   const int64_t nt = h->net.n_trainable;
-  CUDA_CHECK(cudaMalloc(&h->params, nt * 4));
-  CUDA_CHECK(cudaMalloc(&h->grads, (nt + 1024) * 4));
-  CUDA_CHECK(cudaMalloc(&h->moms, nt * 4));
-  CUDA_CHECK(cudaMalloc(&h->bnstat, h->net.n_bnstat * 4));
+  h->params = DevMem<float>(nt * 4);
+  h->grads = DevMem<float>((nt + 1024) * 4);
+  h->moms = DevMem<float>(nt * 4);
+  h->bnstat = DevMem<float>(h->net.n_bnstat * 4);
   CUDA_CHECK(cudaMemset(h->params, 0, nt * 4));
   CUDA_CHECK(cudaMemset(h->grads, 0, (nt + 1024) * 4));
   CUDA_CHECK(cudaMemset(h->moms, 0, nt * 4));
-  CUDA_CHECK(cudaMalloc(&h->is_weight, nt));
+  h->is_weight = DevMem<uint8_t>(nt);
   {
     std::vector<uint8_t> isw(nt, 0);
     for (auto& c : h->net.convs)
@@ -220,25 +195,25 @@ extern "C" int drs_create(drs_handle_t* out, const drs_config* cfg) {
       for (int i = 0; i < c.co; ++i) bn[c.mv_off + i] = 1.0f;
     CUDA_CHECK(cudaMemcpy(h->bnstat, bn.data(), bn.size() * 4, cudaMemcpyHostToDevice));
   }
-  CUDA_CHECK(cudaMalloc(&h->mean, h->net.n_bnstat * 4));
-  CUDA_CHECK(cudaMalloc(&h->inv_std, h->net.n_bnstat * 4));
-  CUDA_CHECK(cudaMalloc(&h->sums, 2 * 512 * 4));
-  CUDA_CHECK(cudaMalloc(&h->loss_dev, 16 * 4));
-  CUDA_CHECK(cudaMalloc(&h->cm_dev, (MAX_CLASSES * MAX_CLASSES + 1) * 4));
-  CUDA_CHECK(cudaMalloc(&h->count_dev, 16));
+  h->mean = DevMem<float>(h->net.n_bnstat * 4);
+  h->inv_std = DevMem<float>(h->net.n_bnstat * 4);
+  h->sums = DevMem<float>(2 * 512 * 4);
+  h->loss_dev = DevMem<float>(16 * 4);
+  h->cm_dev = DevMem<unsigned int>((MAX_CLASSES * MAX_CLASSES + 1) * 4);
+  h->count_dev = DevMem<unsigned int>(16);
   CUDA_CHECK(cudaMemset(h->count_dev, 0, 16));
   h->bn_counter = h->count_dev + 2;
-  CUDA_CHECK(cudaMalloc(&h->bn_acc, (size_t)BN_ACC_REPLICAS * BN_ACC_STRIDE * 8));
+  h->bn_acc = DevMem<long long>((size_t)BN_ACC_REPLICAS * BN_ACC_STRIDE * 8);
   CUDA_CHECK(cudaMemset(h->bn_acc, 0, (size_t)BN_ACC_REPLICAS * BN_ACC_STRIDE * 8));
-  CUDA_CHECK(cudaMalloc(&h->ones, 512 * 4));
-  CUDA_CHECK(cudaMalloc(&h->zeros, 512 * 4));
+  h->ones = DevMem<float>(512 * 4);
+  h->zeros = DevMem<float>(512 * 4);
   CUDA_CHECK(cudaMemset(h->zeros, 0, 512 * 4));
   {
     std::vector<float> o(512, 1.0f);
     CUDA_CHECK(cudaMemcpy(h->ones, o.data(), 512 * 4, cudaMemcpyHostToDevice));
   }
   memset(&h->table, 0, sizeof(h->table));
-  CUDA_CHECK(cudaHostAlloc(&h->diag_host, 64, cudaHostAllocMapped));
+  h->diag_host = new_pinned<uint32_t>(64, cudaHostAllocMapped);
   memset(h->diag_host, 0, 64);
   CUDA_CHECK(cudaHostGetDevicePointer((void**)&h->diag_dev, h->diag_host, 0));
   // driver entry points for tensor-map encoding (no link-time dependency on libcuda)
@@ -253,81 +228,41 @@ extern "C" int drs_create(drs_handle_t* out, const drs_config* cfg) {
     DRS_CHECK(fn && qres == cudaDriverEntryPointSuccess, "cuTensorMapEncodeIm2col not available");
     h->encodeIm2col = (PFN_encodeIm2col)fn;
   }
-  CUDA_CHECK(cudaEventCreate(&h->ev_a));
-  CUDA_CHECK(cudaEventCreate(&h->ev_b));
   h->packed_dirty = true;
   h->eval_dirty = true;
   // whole-step CUDA graphs per (batch, patch size, buffers, lr): on by default (DRS_GRAPHS=0 turns them off); the drop-in
   // loops pre-capture the patch-size interval at start-up (drs_train_prepare), like TF building its graph before the loop
   h->use_graphs = getenv("DRS_GRAPHS") == nullptr || atoi(getenv("DRS_GRAPHS")) != 0;
-  CUDA_CHECK(cudaStreamCreateWithFlags(&h->plan_stream, cudaStreamNonBlocking));
+  h->plan_stream = new_stream();
   for (int i = 0; i < 2; ++i) {
-    CUDA_CHECK(cudaEventCreateWithFlags(&h->plan_uploaded[i], cudaEventDisableTiming));
-    CUDA_CHECK(cudaEventCreateWithFlags(&h->plan_consumed[i], cudaEventDisableTiming));
+    h->plan_uploaded[i] = new_event();
+    h->plan_consumed[i] = new_event();
   }
-  CUDA_CHECK(cudaHostAlloc((void**)&h->result_host, (size_t)Handle::RESULT_RING * RESULT_STRIDE * 4, cudaHostAllocDefault));
-  for (int i = 0; i < Handle::RESULT_RING; ++i) CUDA_CHECK(cudaEventCreateWithFlags(&h->result_ev[i], cudaEventDisableTiming));
-  CUDA_CHECK(cudaStreamCreateWithFlags(&h->side_stream, cudaStreamNonBlocking));
-  CUDA_CHECK(cudaStreamCreateWithFlags(&h->comm_stream, cudaStreamNonBlocking));
-  CUDA_CHECK(cudaEventCreateWithFlags(&h->ev_bucket_ready, cudaEventDisableTiming));
-  CUDA_CHECK(cudaEventCreateWithFlags(&h->ev_x8, cudaEventDisableTiming));
-  CUDA_CHECK(cudaEventCreateWithFlags(&h->ev_bucket_done, cudaEventDisableTiming));
+  h->result_host = new_pinned<float>((size_t)Handle::RESULT_RING * RESULT_STRIDE * 4, cudaHostAllocDefault);
+  for (int i = 0; i < Handle::RESULT_RING; ++i) h->result_ev[i] = new_event();
+  h->side_stream = new_stream();
+  h->comm_stream = new_stream();
+  h->ev_bucket_ready = new_event();
+  h->ev_x8 = new_event();
+  h->ev_bucket_done = new_event();
   for (int i = 0; i < 2; ++i) {
-    CUDA_CHECK(cudaEventCreateWithFlags(&h->ev_dz[i], cudaEventDisableTiming));
-    CUDA_CHECK(cudaEventCreateWithFlags(&h->ev_wgrad[i], cudaEventDisableTiming));
+    h->ev_dz[i] = new_event();
+    h->ev_wgrad[i] = new_event();
   }
-  *out = h;
+  *out = h.release();
   API_END
 }
 
+// Everything the handle holds is released by its members' destructors, once no stream has work left that uses it.
 extern "C" int drs_destroy(drs_handle_t h) {
   API_BEGIN
   if (!h) return 0;
   cudaSetDevice(h->cfg.device);
   cudaStreamSynchronize(h->stream);
-  if (h->nccl) { drs_comm_destroy(h); }
-  if (h->side_stream) { cudaStreamSynchronize(h->side_stream); cudaStreamDestroy(h->side_stream); }
-  if (h->comm_stream) { cudaStreamSynchronize(h->comm_stream); cudaStreamDestroy(h->comm_stream); }
-  if (h->ev_bucket_ready) cudaEventDestroy(h->ev_bucket_ready);
-  if (h->ev_x8) cudaEventDestroy(h->ev_x8);
-  if (h->ev_bucket_done) cudaEventDestroy(h->ev_bucket_done);
-  if (h->copy_stream) { cudaStreamSynchronize(h->copy_stream); cudaStreamDestroy(h->copy_stream); }
-  if (h->plan_stream) { cudaStreamSynchronize(h->plan_stream); cudaStreamDestroy(h->plan_stream); }
-  for (int i = 0; i < 2; ++i) {
-    if (h->plan_uploaded[i]) cudaEventDestroy(h->plan_uploaded[i]);
-    if (h->plan_consumed[i]) cudaEventDestroy(h->plan_consumed[i]);
-    if (h->plan_stage[i]) cudaFree(h->plan_stage[i]);
-  }
-  for (int i = 0; i < Handle::RESULT_RING; ++i)
-    if (h->result_ev[i]) cudaEventDestroy(h->result_ev[i]);
-  if (h->result_host) cudaFreeHost(h->result_host);
-  if (h->up_ev[0]) cudaEventDestroy(h->up_ev[0]);
-  for (int i = 0; i < 2; ++i) {
-    if (h->ev_dz[i]) cudaEventDestroy(h->ev_dz[i]);
-    if (h->ev_wgrad[i]) cudaEventDestroy(h->ev_wgrad[i]);
-  }
-  lane_release(h);
-  for (int i = 0; i < 8; ++i)
-    if (h->slot_ptr[i]) cudaFree(h->slot_ptr[i]);
-  for (auto& kv : h->graphs) {
-    if (kv.second.exec) cudaGraphExecDestroy(kv.second.exec);
-    for (auto& pr : kv.second.events) { cudaEventDestroy(pr.first); cudaEventDestroy(pr.second); }
-  }
-  free_packed(h);
-  for (auto& kv : h->scenes) {
-    if (kv.second.data) cudaFree(kv.second.data);
-    if (kv.second.labels) cudaFree(kv.second.labels);
-  }
-  cudaFree(h->params); cudaFree(h->grads); cudaFree(h->moms); cudaFree(h->bnstat);
-  if (h->arena.base) cudaFree(h->arena.base);
-  if (h->dstage) cudaFree(h->dstage);
-  if (h->pinned) cudaFreeHost(h->pinned);
-  if (h->diag_host) cudaFreeHost(h->diag_host);
-  cudaFree(h->is_weight); cudaFree(h->mean); cudaFree(h->inv_std); cudaFree(h->sums); cudaFree(h->loss_dev);
-  cudaFree(h->cm_dev); cudaFree(h->count_dev); cudaFree(h->bn_acc); cudaFree(h->ones); cudaFree(h->zeros);
-  for (auto& pr : h->conv_events) { cudaEventDestroy(pr.first); cudaEventDestroy(pr.second); }
-  cudaEventDestroy(h->ev_a); cudaEventDestroy(h->ev_b);
-  cudaStreamDestroy(h->own_stream);
+  for (cudaStream_t s : {h->own_stream.get(), h->side_stream.get(), h->comm_stream.get(), h->copy_stream.get(),
+                         h->plan_stream.get(), h->lane.stream.get()})
+    if (s) cudaStreamSynchronize(s);
+  if (h->nccl) drs_comm_destroy(h);
   delete h;
   API_END
 }
@@ -690,11 +625,11 @@ static void refresh_packed(Handle* h, bool training) {
       const long long n = (long long)taps * c.ci * c.co;
       const size_t es = et == ET_F32 ? 4 : 2;
       if (et != ET_F32) {
-        if (!c.w_fprop) CUDA_CHECK(cudaMalloc(&c.w_fprop, n * es));
+        c.w_fprop.grow(n * es, n * es);
         t.seg[t.n++] = RepackSeg{h->params + c.w_off, c.w_fprop, taps, c.ci, c.co, 0, off};
         off += n;
       }
-      if (!c.w_dgrad) CUDA_CHECK(cudaMalloc(&c.w_dgrad, n * es));
+      c.w_dgrad.grow(n * es, n * es);
       t.seg[t.n++] = RepackSeg{h->params + c.w_off, c.w_dgrad, taps, c.ci, c.co, et == ET_F32 ? 2 : 1, off};
       off += n;
     }
@@ -708,10 +643,8 @@ static void refresh_packed(Handle* h, bool training) {
   if (!training && h->eval_dirty) {
     for (size_t l = 0; l < h->net.convs.size(); ++l) {
       ConvLayer& c = h->net.convs[l];
-      if (!c.fold_scale) {
-        CUDA_CHECK(cudaMalloc(&c.fold_scale, c.co * 4));
-        CUDA_CHECK(cudaMalloc(&c.fold_shift, c.co * 4));
-      }
+      c.fold_scale.grow(c.co * 4, c.co * 4);
+      c.fold_shift.grow(c.co * 4, c.co * 4);
       fold_bn_kernel<<<nblk(c.co, 128), 128, 0, h->stream>>>(h->params + c.b_off, h->bnstat + c.mm_off, h->bnstat + c.mv_off,
                                                               h->cfg.bn_eps, c.fold_scale, c.fold_shift, c.co);
       LAUNCH_CHECK(h);
@@ -719,9 +652,9 @@ static void refresh_packed(Handle* h, bool training) {
       // fp32 mode run it on the CUDA-core kernel straight from the HWIO weights
       if (l == 0 && et != ET_F32 && conv1_tc_supported(c.k, c.rate, c.ci, c.co)) {
         const int n = C1_SLOTS * c.co * 8;
-        if (!c.w_fprop) CUDA_CHECK(cudaMalloc(&c.w_fprop, (size_t)n * 2));
-        if (et == ET_F16) pack_conv1_kernel<__half><<<nblk(n, 256), 256, 0, h->stream>>>(h->params + c.w_off, (__half*)c.w_fprop, c.ci, c.co);
-        else pack_conv1_kernel<__nv_bfloat16><<<nblk(n, 256), 256, 0, h->stream>>>(h->params + c.w_off, (__nv_bfloat16*)c.w_fprop, c.ci, c.co);
+        c.w_fprop.grow((size_t)n * 2, (size_t)n * 2);
+        if (et == ET_F16) pack_conv1_kernel<__half><<<nblk(n, 256), 256, 0, h->stream>>>(h->params + c.w_off, (__half*)c.w_fprop.get(), c.ci, c.co);
+        else pack_conv1_kernel<__nv_bfloat16><<<nblk(n, 256), 256, 0, h->stream>>>(h->params + c.w_off, (__nv_bfloat16*)c.w_fprop.get(), c.ci, c.co);
         LAUNCH_CHECK(h);
       }
     }
@@ -745,20 +678,14 @@ static ConvLayer conv_shape(int k, int rate, int ci, int co) {
 static void prof_begin(Handle* h, cudaEvent_t* a, cudaEvent_t* b) {
   if (!h->time_convs) return;
   if (h->capturing) {
-    cudaEvent_t e0, e1;
-    CUDA_CHECK(cudaEventCreate(&e0));
-    CUDA_CHECK(cudaEventCreate(&e1));
-    h->capturing->events.push_back({e0, e1});
-    *a = e0; *b = e1;
-    CUDA_CHECK(cudaEventRecordWithFlags(e0, h->stream, cudaEventRecordExternal));
+    h->capturing->events.emplace_back(new_event(cudaEventDefault), new_event(cudaEventDefault));
+    *a = h->capturing->events.back().first;
+    *b = h->capturing->events.back().second;
+    CUDA_CHECK(cudaEventRecordWithFlags(*a, h->stream, cudaEventRecordExternal));
     return;
   }
-  if (h->conv_events_used == h->conv_events.size()) {
-    cudaEvent_t e0, e1;
-    CUDA_CHECK(cudaEventCreate(&e0));
-    CUDA_CHECK(cudaEventCreate(&e1));
-    h->conv_events.push_back({e0, e1});
-  }
+  if (h->conv_events_used == h->conv_events.size())
+    h->conv_events.emplace_back(new_event(cudaEventDefault), new_event(cudaEventDefault));
   *a = h->conv_events[h->conv_events_used].first;
   *b = h->conv_events[h->conv_events_used].second;
   h->conv_events_used++;
@@ -852,10 +779,10 @@ static void forward_eval_t(Handle* h, const float* x_dev, int B, int crop, float
   refresh_packed(h, false);
   const int fs = n.feat_stride;
   ensure_arena(h, layout_bytes<EvalWs<TA>>(h, B, crop));
-  h->arena.reset();
+  h->arena->reset();
   EvalWs<TA> ws;
   {
-    WsAlloc carve{&h->arena};
+    WsAlloc carve{h->arena};
     ws.layout(h, carve, B, crop);
   }
   float* logits = logits_dev ? logits_dev : ws.logits;
@@ -970,7 +897,7 @@ extern "C" int drs_forward_host(drs_handle_t h, const float* x_host, int32_t B, 
   const int C = h->net.channels, K = h->net.classes;
   const size_t xb = (size_t)M * C * 4, lb = (size_t)M * K * 4;
   ensure_dstage(h, xb + lb + (size_t)M * 9 + 4096);
-  char* d = (char*)h->dstage;
+  char* d = h->dstage;
   float* x_dev = (float*)d;
   float* lg_dev = (float*)(d + round_up(xb, 256));
   long long* p64 = (long long*)((char*)lg_dev + round_up(lb, 256));
@@ -991,9 +918,8 @@ extern "C" int drs_forward_host(drs_handle_t h, const float* x_host, int32_t B, 
 template <typename T>
 static void debug_keep(Handle* h, const std::string& name, const T* ptr, int cs, int co, int C, int64_t M) {
   if (!h->debug_keep) return;
-  float* buf = nullptr;
-  CUDA_CHECK(cudaMalloc(&buf, M * C * 4));
-  h->keep.push_back(buf);
+  h->keep.emplace_back(M * C * 4);
+  float* buf = h->keep.back();
   slice_to_f32_kernel<T><<<nblk(M * C, 256), 256, 0, h->stream>>>(ptr, cs, co, C, M, buf);
   LAUNCH_CHECK(h);
   h->taps[name] = {buf, ET_F32, C, 0, C, M};
@@ -1002,7 +928,6 @@ static void debug_keep_reset(Handle* h) {
   h->debug_keep = getenv("DRS_DEBUG_KEEP") != nullptr;
   if (h->keep.empty()) return;
   cudaStreamSynchronize(h->stream);
-  for (float* p : h->keep) cudaFree(p);
   h->keep.clear();
 }
 

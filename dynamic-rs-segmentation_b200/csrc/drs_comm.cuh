@@ -120,7 +120,7 @@ static void do_allreduce(Handle* h, float* buf, int64_t count, cudaStream_t on_s
   DRS_CHECK(rc == 0, "allreduce callback failed with %d", rc);
 }
 
-// Stripe-sharded scene pass: every rank's uint8 label stripe (slot 4 of the last drs_scene_infer) goes to rank 0 over
+// Stripe-sharded scene pass: every rank's uint8 label stripe (the label map of the last drs_scene_infer) goes to rank 0 over
 // NVLink, straight from device memory; rank 0 assembles [H, W] on the device and copies it to the host once.
 //   row_cuts [world+1]: stripe r holds rows [row_cuts[r], row_cuts[r+1]) (dist.stripe_bounds)
 extern "C" int drs_scene_gather_labels(drs_handle_t h, int32_t H, int32_t W, const int32_t* row_cuts, int32_t all_ranks,
@@ -135,10 +135,10 @@ extern "C" int drs_scene_gather_labels(drs_handle_t h, int32_t H, int32_t W, con
             "scene_gather_labels: the last scene pass covered rows [%d,%d), not this rank's stripe [%d,%d)", h->last_row_begin,
             h->last_row_begin + h->last_rows, row_cuts[rank], row_cuts[rank + 1]);
   DRS_CHECK(labels_out_host || (rank != 0 && !all_ranks), "scene_gather_labels: this rank needs the output buffer");
-  const uint8_t* mine = (const uint8_t*)h->slot_ptr[4];
+  const uint8_t* mine = h->pass.labels;
   NcclApi* n = nccl_api();
   drs_ncclComm_t comm = (drs_ncclComm_t)h->nccl;
-  uint8_t* full = (rank == 0 || all_ranks) ? (uint8_t*)slot_buf(h, 7, (size_t)H * W) : nullptr;
+  uint8_t* full = (rank == 0 || all_ranks) ? pass_buf(h, h->pass.assembled, (size_t)H * W) : nullptr;
   if (rank != 0) {
     if (h->last_rows > 0) NCCL_CHECK(n->Send(mine, (size_t)h->last_rows * W, DRS_NCCL_UINT8, 0, comm, h->stream));
   } else {

@@ -9,8 +9,11 @@
 #include <stdlib.h>
 #include <string.h>
 
+#include <initializer_list>
 #include <map>
+#include <memory>
 #include <string>
+#include <utility>
 #include <vector>
 
 #include "../../include/drs.h"
@@ -40,6 +43,88 @@ struct DrsError {
 static inline int64_t ceil_div(int64_t a, int64_t b) { return (a + b - 1) / b; }
 static inline int64_t round_up(int64_t a, int64_t b) { return ceil_div(a, b) * b; }
 
+// ------------------------------------------------------------------ owned CUDA resources
+// A stream, event, graph exec or allocation that releases itself: whatever holds one (the handle, a scene, a debug entry
+// point) frees it by going away, so no list of frees has to mirror the allocations.  The destructor ignores the error of the
+// release (nothing could be done about it there); reset() returns it.
+template <typename T, auto Destroy>
+class Owner {
+ public:
+  Owner() = default;
+  explicit Owner(T p) : p_(p) {}
+  Owner(Owner&& o) noexcept : p_(o.p_) { o.p_ = nullptr; }
+  Owner& operator=(Owner&& o) noexcept {
+    if (this != &o) { reset(); p_ = o.p_; o.p_ = nullptr; }
+    return *this;
+  }
+  ~Owner() { reset(); }
+  cudaError_t reset() {
+    const cudaError_t e = p_ ? Destroy(p_) : cudaSuccess;
+    p_ = nullptr;
+    return e;
+  }
+  T get() const { return p_; }
+  operator T() const { return p_; }
+
+ private:
+  T p_ = nullptr;
+};
+using Stream = Owner<cudaStream_t, cudaStreamDestroy>;
+using Event = Owner<cudaEvent_t, cudaEventDestroy>;
+using GraphExec = Owner<cudaGraphExec_t, cudaGraphExecDestroy>;
+template <typename T> using PinnedMem = Owner<T*, cudaFreeHost>;
+
+static inline Stream new_stream() {
+  cudaStream_t s = nullptr;
+  CUDA_CHECK(cudaStreamCreateWithFlags(&s, cudaStreamNonBlocking));
+  return Stream(s);
+}
+static inline Event new_event(unsigned flags = cudaEventDisableTiming) {
+  cudaEvent_t e = nullptr;
+  CUDA_CHECK(cudaEventCreateWithFlags(&e, flags));
+  return Event(e);
+}
+template <typename T>
+static PinnedMem<T> new_pinned(size_t bytes, unsigned flags) {
+  void* p = nullptr;
+  CUDA_CHECK(cudaHostAlloc(&p, bytes, flags));
+  return PinnedMem<T>((T*)p);
+}
+
+// Device memory and its size in bytes.
+template <typename T>
+struct DevMem {
+  Owner<T*, cudaFree> p;
+  size_t cap = 0;
+
+  DevMem() = default;
+  explicit DevMem(size_t bytes) { grow(bytes, bytes); }
+  DevMem(DevMem&& o) noexcept : p(std::move(o.p)), cap(std::exchange(o.cap, 0)) {}
+  DevMem& operator=(DevMem&& o) noexcept {
+    p = std::move(o.p);
+    cap = std::exchange(o.cap, 0);
+    return *this;
+  }
+  T* get() const { return p; }
+  operator T*() const { return p; }
+  // Makes room for `need` bytes.  A smaller buffer is freed, once the streams in `sync` (whose queued work may still use it)
+  // have drained, and replaced by `want` >= need bytes.  Returns whether it was.
+  bool grow(size_t need, size_t want, std::initializer_list<cudaStream_t> sync = {}) {
+    if (cap >= need) return false;
+    for (cudaStream_t s : sync) CUDA_CHECK(cudaStreamSynchronize(s));
+    reset();
+    void* q = nullptr;
+    CUDA_CHECK(cudaMalloc(&q, want));
+    p = Owner<T*, cudaFree>((T*)q);
+    cap = want;
+    return true;
+  }
+  void reset() {
+    cap = 0;
+    CUDA_CHECK(p.reset());
+  }
+};
+
 // ------------------------------------------------------------------ network description
 enum { ACT_NONE = 0, ACT_RELU = 1, ACT_LRELU = 2 };
 
@@ -54,11 +139,10 @@ struct ConvLayer {
   // offsets into the flat BN-statistics buffer
   int64_t mm_off, mv_off;
   // packed low-precision operand matrices
-  void* w_fprop = nullptr;   // [co][k*k*ci]  (K index = tap*ci + c)
-  void* w_dgrad = nullptr;   // [ci][k*k*co]  (flipped taps)
-  float* fold_scale = nullptr;  // [co] eval-mode BN folded: y = act(conv*scale + shift)
-  float* fold_shift = nullptr;
-  float* raw_scale = nullptr;   // [co] ones
+  DevMem<void> w_fprop;      // [co][k*k*ci]  (K index = tap*ci + c)
+  DevMem<void> w_dgrad;      // [ci][k*k*co]  (flipped taps)
+  DevMem<float> fold_scale;  // [co] eval-mode BN folded: y = act(conv*scale + shift)
+  DevMem<float> fold_shift;
   // structural variants (variants.cuh): a post-op behind the activation, and explicit buffer routing for the squeeze modules
   int post = 0;           // 0 none, 1 SAME average pooling post_k x post_k (isprs:753-758), 2 squeeze-and-excitation gate
   int post_k = 0;
@@ -92,10 +176,9 @@ struct NetDesc {
 };
 
 struct Scene {
-  void* data = nullptr;   // [H,W,C] f64 or f32
-  uint8_t* labels = nullptr;
+  DevMem<void> data;       // [H,W,C] f64 or f32 (re-uploads of the same shape reuse the buffers)
+  DevMem<uint8_t> labels;
   int H = 0, W = 0, C = 0, dtype = 0;
-  size_t data_cap = 0, labels_cap = 0;   // allocation sizes (re-uploads of the same shape reuse the buffers)
   int row0 = 0, rows = 0;   // resident rows [row0, row0+rows) of the H-row scene (a rank keeps only its stripe + halo)
 };
 
@@ -113,24 +196,22 @@ struct SceneTable {
 constexpr int MAX_CLASSES = 8;
 
 struct Arena {
-  char* base = nullptr;
-  size_t cap = 0, used = 0;
+  DevMem<char> mem;
+  size_t used = 0;
   void reset() { used = 0; }
   void* take(size_t bytes) {
     size_t off = (used + 1023) & ~size_t(1023);
-    if (off + bytes > cap) return nullptr;
+    if (off + bytes > mem.cap) return nullptr;
     used = off + bytes;
-    return base + off;
+    return mem.get() + off;
   }
 };
 
 struct InferLane {
-  cudaStream_t stream = nullptr;
+  Stream stream;
   Arena arena;
-  float* x = nullptr;
-  float* lg = nullptr;
-  size_t x_cap = 0, lg_cap = 0;
-  cudaEvent_t fwd_done = nullptr, acc_done = nullptr;
+  DevMem<float> x, lg;
+  Event fwd_done, acc_done;
 };
 
 // One captured training step (CUDA graph) per (batch, patch size, buffers, learning rate): the step is ~65 small
@@ -143,10 +224,10 @@ struct TrainGraphKey {
   bool operator<(const TrainGraphKey& o) const { return memcmp(this, &o, sizeof(*this)) < 0; }
 };
 struct TrainGraph {
-  cudaGraphExec_t exec = nullptr;
+  std::vector<std::pair<Event, Event>> events;   // external event-record nodes around the tensor-core launches
+  GraphExec exec;                                // (declared after the events: destroyed before them)
   int64_t launches = 0, conv_launches = 0;
   double conv_flops = 0;
-  std::vector<std::pair<cudaEvent_t, cudaEvent_t>> events;   // external event-record nodes around the tensor-core launches
 };
 
 // cell tables of an ordered position list (host)
@@ -183,7 +264,7 @@ struct drs_handle_s {
   NetDesc net;
   int sm_count = 148;
   int driver_version = 0;
-  cudaStream_t own_stream = nullptr;
+  Stream own_stream;
   cudaStream_t stream = nullptr;
   int64_t launches = 0;
   // Programmatic dependent launch (training step, main stream): pdl_on = the step allows it, pdl_prev = the last operation
@@ -191,26 +272,23 @@ struct drs_handle_s {
   bool pdl_on = false, pdl_prev = false;
 
   // variables
-  float* params = nullptr;   // flat trainables: all weights & biases
-  float* grads = nullptr;
-  float* moms = nullptr;
-  float* bnstat = nullptr;   // moving_mean / moving_variance
+  DevMem<float> params;      // flat trainables: all weights & biases
+  DevMem<float> grads;
+  DevMem<float> moms;
+  DevMem<float> bnstat;      // moving_mean / moving_variance
   int64_t global_step = 0;
   int ignore_label = -1;     // contest: label excluded from loss / confusion when no mask is passed
   bool packed_dirty = true;  // packed operand matrices need refresh
   bool eval_dirty = true;    // folded eval-mode BN / conv1 tensor-core operand need refresh
 
-  // workspace
-  Arena arena;
+  // workspace: launches carve from *arena, the handle's own arena or, inside its StreamScope, the scene lane's
+  Arena own_arena;
+  Arena* arena = &own_arena;
   uint64_t arena_epoch = 0;
-  // pinned staging for *_host entry points
-  void* pinned = nullptr;
-  size_t pinned_cap = 0;
-  void* dstage = nullptr;    // device staging for host entry points
-  size_t dstage_cap = 0;
+  DevMem<char> dstage;       // device staging for host entry points
 
   // host-mapped diagnostics written by bounded waits
-  uint32_t* diag_host = nullptr;
+  PinnedMem<uint32_t> diag_host;
   uint32_t* diag_dev = nullptr;
 
   // scenes
@@ -225,8 +303,7 @@ struct drs_handle_s {
   int sync_bn = 0;
 
   // timing of conv kernels
-  cudaEvent_t ev_a = nullptr, ev_b = nullptr;
-  std::vector<std::pair<cudaEvent_t, cudaEvent_t>> conv_events;
+  std::vector<std::pair<Event, Event>> conv_events;
   size_t conv_events_used = 0;
   bool time_convs = false;
 
@@ -238,41 +315,47 @@ struct drs_handle_s {
   PFN_encodeIm2col encodeIm2col = nullptr;
   std::map<TmKey, CUtensorMap> tm_cache;
 
-  // persistent scene-pass buffers (score map, occurrence counts, cell tables, label map ...): cudaMalloc / cudaFree of
-  // gigabyte-sized buffers per call costs hundreds of milliseconds, so each named slot only ever grows
-  // the label map of the last scene pass stays in slot 4 for drs_scene_confusion
+  // persistent scene-pass buffers: cudaMalloc / cudaFree of gigabyte-sized buffers per call costs hundreds of milliseconds,
+  // so each only ever grows.  The label map of the last pass stays for drs_scene_confusion and drs_scene_gather_labels.
   int last_scene = -1, last_row_begin = 0, last_rows = 0, last_W = 0;
-  void* slot_ptr[8] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
-  size_t slot_cap[8] = {0, 0, 0, 0, 0, 0, 0, 0};
+  struct {
+    DevMem<float> prob;                   // score map [rows][W][K]
+    DevMem<uint32_t> occur;               // occurrence counts [rows][W]
+    DevMem<int32_t> cell_off, cell_seq;   // cell tables of the visiting order
+    DevMem<uint8_t> labels;               // label map [rows][W]
+    DevMem<double> mean;                  // mean score map [rows][W][K]
+    DevMem<int32_t> inst;                 // (scene, row, col) of every patch of the pass
+    DevMem<uint8_t> assembled;            // [H][W] label map assembled from every rank's stripe
+  } pass;
   std::vector<PassGeometry> pass_geometry;   // the last few scene-pass geometries, oldest first
   std::map<TrainGraphKey, TrainGraph> graphs;
   TrainGraph* capturing = nullptr;   // non-null while a training step is being captured
-  cudaStream_t side_stream = nullptr;     // filter gradients run here, overlapped with the backward's HBM-bound kernels
-  cudaEvent_t ev_dz[2] = {nullptr, nullptr}, ev_wgrad[2] = {nullptr, nullptr};
+  Stream side_stream;                // filter gradients run here, overlapped with the backward's HBM-bound kernels
+  Event ev_dz[2], ev_wgrad[2];
   // data-parallel exchange of the late layers' gradients, overlapped with the rest of the backward
-  cudaStream_t comm_stream = nullptr;
-  cudaEvent_t ev_bucket_ready = nullptr, ev_bucket_done = nullptr;
-  cudaEvent_t ev_x8 = nullptr;          // conv1's padded input is ready: the side stream builds the im2col matrix under the forward
+  Stream comm_stream;
+  Event ev_bucket_ready, ev_bucket_done;
+  Event ev_x8;                       // conv1's padded input is ready: the side stream builds the im2col matrix under the forward
   bool use_graphs = true;           // DRS_GRAPHS=0 turns the whole-step CUDA graphs off (drs_create)
   double conv_ms_acc = 0;            // device time of profiled launches already read back
   InferLane lane;                 // scene-inference lane (drs_scene_api.cuh)
-  cudaEvent_t lane_ready = nullptr;
+  Event lane_ready;
   // streamed scene upload (drs_scene_infer_host): copy stream + "rows uploaded" event
-  cudaStream_t copy_stream = nullptr;
-  cudaEvent_t up_ev[1] = {nullptr};
-  uint8_t* is_weight = nullptr;   // [n_trainable] 1 for `weights` variables
+  Stream copy_stream;
+  Event up_ev;
+  DevMem<uint8_t> is_weight;      // [n_trainable] 1 for `weights` variables
   SceneTable table;               // host copy of the device scene table
   // training scratch kept between calls
-  float* mean = nullptr;          // [sum co] batch mean of the last train step (per layer, same offsets as mm_off/2)
-  float* inv_std = nullptr;
-  float* sums = nullptr;          // [2*256]
-  float* loss_dev = nullptr;      // [4]: ce, l2, count, spare
-  unsigned int* cm_dev = nullptr; // [K*K+1]
-  unsigned int* count_dev = nullptr;
+  DevMem<float> mean;             // [sum co] batch mean of the last train step (per layer, same offsets as mm_off/2)
+  DevMem<float> inv_std;
+  DevMem<float> sums;             // [2*256]
+  DevMem<float> loss_dev;         // [4]: ce, l2, count, spare
+  DevMem<unsigned int> cm_dev;    // [K*K+1]
+  DevMem<unsigned int> count_dev;
   unsigned int* bn_counter = nullptr;   // last-block-done counter of bn_partial_kernel (self-resetting)
-  long long* bn_acc = nullptr;          // [BN_ACC_REPLICAS][2*512] fixed-point accumulators of bn_partial_kernel (self-clearing)
-  float* ones = nullptr;          // [512]
-  float* zeros = nullptr;         // [512]
+  DevMem<long long> bn_acc;             // [BN_ACC_REPLICAS][2*512] fixed-point accumulators of bn_partial_kernel (self-clearing)
+  DevMem<float> ones;             // [512]
+  DevMem<float> zeros;            // [512]
   // profiling
   double conv_flops = 0;
   int64_t conv_launches = 0;
@@ -281,36 +364,28 @@ struct drs_handle_s {
   // land in a ring of pinned result slots behind an event, so the host never blocks on the step it has just enqueued
   void* nccl = nullptr;             // ncclComm_t of drs_comm_init (drs_comm.cuh); null: single process or callback exchange
   int rank = 0;
-  cudaStream_t plan_stream = nullptr;
-  void* plan_stage[2] = {nullptr, nullptr};
-  size_t plan_stage_cap[2] = {0, 0};
-  cudaEvent_t plan_uploaded[2] = {nullptr, nullptr}, plan_consumed[2] = {nullptr, nullptr};
+  Stream plan_stream;
+  DevMem<char> plan_stage[2];
+  Event plan_uploaded[2], plan_consumed[2];
   bool plan_consumed_valid[2] = {false, false};
   int64_t plan_calls = 0;
   static constexpr int RESULT_RING = 8;
-  float* result_host = nullptr;     // pinned [RESULT_RING][RESULT_STRIDE]
-  cudaEvent_t result_ev[RESULT_RING] = {};
+  PinnedMem<float> result_host;     // [RESULT_RING][RESULT_STRIDE]
+  Event result_ev[RESULT_RING];
   int64_t next_ticket = 0;
   // DRS_DEBUG_KEEP=1: fp32 copies of backward intermediates ("dz:<scope>", "da:<scope>")
-  std::vector<float*> keep;
+  std::vector<DevMem<float>> keep;
   bool debug_keep = false;
 };
 typedef drs_handle_s Handle;
 
 static inline void ensure_arena(Handle* h, size_t bytes) {
-  if (h->arena.cap >= bytes) return;
-  CUDA_CHECK(cudaStreamSynchronize(h->stream));
-  if (h->arena.base) CUDA_CHECK(cudaFree(h->arena.base));
-  h->arena.base = nullptr;
-  h->arena.cap = 0;
-  h->arena_epoch++;          // cached CUDA graphs hold pointers into the old arena
-  size_t want = bytes + (bytes >> 3) + (size_t(1) << 20);
-  CUDA_CHECK(cudaMalloc(&h->arena.base, want));
-  h->arena.cap = want;
+  if (h->arena->mem.grow(bytes, bytes + (bytes >> 3) + (size_t(1) << 20), {h->stream}))
+    h->arena_epoch++;          // cached CUDA graphs hold pointers into the old arena
 }
 static inline void* arena_take(Handle* h, size_t bytes) {
-  void* p = h->arena.take(bytes);
-  DRS_CHECK(p != nullptr, "workspace arena exhausted (need %zu more bytes, cap %zu)", bytes, h->arena.cap);
+  void* p = h->arena->take(bytes);
+  DRS_CHECK(p != nullptr, "workspace arena exhausted (need %zu more bytes, cap %zu)", bytes, h->arena->mem.cap);
   return p;
 }
 // What a workspace layout (TrainWs, EvalWs) runs against: with an arena it carves the buffers from it; without one it only
@@ -322,7 +397,7 @@ struct WsAlloc {
     used = round_up(used, 1024) + bytes;
     if (!arena) return nullptr;
     void* p = arena->take(bytes);
-    DRS_CHECK(p != nullptr, "workspace arena exhausted (need %zu more bytes, cap %zu)", bytes, arena->cap);
+    DRS_CHECK(p != nullptr, "workspace arena exhausted (need %zu more bytes, cap %zu)", bytes, arena->mem.cap);
     return (T*)p;
   }
 };
@@ -332,36 +407,26 @@ struct WsAlloc {
 // dependency: its predecessor on that stream is not known.
 struct StreamScope {
   drs_handle_s* h;
-  bool on, swap_arena, pdl_prev;
+  bool on, pdl_prev;
   cudaStream_t stream;
-  Arena arena;
-  StreamScope(drs_handle_s* h_, bool on_, cudaStream_t s, const Arena* a = nullptr)
-      : h(h_), on(on_), swap_arena(on_ && a), pdl_prev(h_->pdl_prev), stream(h_->stream), arena(h_->arena) {
+  Arena* arena;
+  StreamScope(drs_handle_s* h_, bool on_, cudaStream_t s, Arena* a = nullptr)
+      : h(h_), on(on_), pdl_prev(h_->pdl_prev), stream(h_->stream), arena(h_->arena) {
     if (on) { h->stream = s; h->pdl_prev = false; }
-    if (swap_arena) h->arena = *a;
+    if (on && a) h->arena = a;
   }
   ~StreamScope() {
     if (on) { h->stream = stream; h->pdl_prev = pdl_prev; }
-    if (swap_arena) h->arena = arena;
+    h->arena = arena;
   }
 };
-static inline void ensure_pinned(Handle* h, size_t bytes) {
-  if (h->pinned_cap >= bytes) return;
-  CUDA_CHECK(cudaStreamSynchronize(h->stream));
-  if (h->pinned) CUDA_CHECK(cudaFreeHost(h->pinned));
-  h->pinned = nullptr;
-  size_t want = bytes + (bytes >> 2) + 4096;
-  CUDA_CHECK(cudaHostAlloc(&h->pinned, want, cudaHostAllocDefault));
-  h->pinned_cap = want;
-}
-static inline void ensure_dstage(Handle* h, size_t bytes) {
-  if (h->dstage_cap >= bytes) return;
-  CUDA_CHECK(cudaStreamSynchronize(h->stream));
-  if (h->dstage) CUDA_CHECK(cudaFree(h->dstage));
-  h->dstage = nullptr;
-  size_t want = bytes + (bytes >> 2) + 4096;
-  CUDA_CHECK(cudaMalloc(&h->dstage, want));
-  h->dstage_cap = want;
+static inline void ensure_dstage(Handle* h, size_t bytes) { h->dstage.grow(bytes, bytes + (bytes >> 2) + 4096, {h->stream}); }
+// a scene-pass buffer of the handle, grown to exactly `bytes` (an empty table still gets an address)
+template <typename T>
+static T* pass_buf(Handle* h, DevMem<T>& b, size_t bytes) {
+  if (bytes == 0) bytes = 16;
+  b.grow(bytes, bytes, {h->stream});
+  return b;
 }
 
 // Train-mode BN statistics: what the last block of a statistics-producing kernel (bn_partial_kernel, or the conv epilogue)

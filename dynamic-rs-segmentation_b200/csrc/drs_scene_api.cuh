@@ -13,24 +13,13 @@ static void scene_upload_rows(Handle* h, int32_t scene_id, const void* rows_host
   Scene& s = h->scenes[scene_id];
   CUDA_CHECK(cudaStreamSynchronize(h->stream));
   const size_t bytes = (size_t)rows * W * C * (dtype == DRS_SCENE_F64 ? 8 : 4);
-  if (s.data_cap < bytes) {
-    if (s.data) CUDA_CHECK(cudaFree(s.data));
-    s.data = nullptr; s.data_cap = 0;
-    CUDA_CHECK(cudaMalloc(&s.data, bytes));
-    s.data_cap = bytes;
-  }
+  s.data.grow(bytes, bytes);
   CUDA_CHECK(cudaMemcpyAsync(s.data, rows_host, bytes, cudaMemcpyHostToDevice, h->stream));
   if (labels_rows_host) {
-    if (s.labels_cap < (size_t)rows * W) {
-      if (s.labels) CUDA_CHECK(cudaFree(s.labels));
-      s.labels = nullptr; s.labels_cap = 0;
-      CUDA_CHECK(cudaMalloc(&s.labels, (size_t)rows * W));
-      s.labels_cap = (size_t)rows * W;
-    }
+    s.labels.grow((size_t)rows * W, (size_t)rows * W);
     CUDA_CHECK(cudaMemcpyAsync(s.labels, labels_rows_host, (size_t)rows * W, cudaMemcpyHostToDevice, h->stream));
-  } else if (s.labels) {
-    CUDA_CHECK(cudaFree(s.labels));
-    s.labels = nullptr; s.labels_cap = 0;
+  } else {
+    s.labels.reset();
   }
   CUDA_CHECK(cudaStreamSynchronize(h->stream));
   s.H = H; s.W = W; s.C = C; s.dtype = dtype; s.row0 = row0; s.rows = rows;
@@ -57,8 +46,6 @@ extern "C" int drs_scene_free(drs_handle_t h, int32_t scene_id) {
   auto it = h->scenes.find(scene_id);
   if (it == h->scenes.end()) return 0;
   CUDA_CHECK(cudaStreamSynchronize(h->stream));
-  if (it->second.data) cudaFree(it->second.data);
-  if (it->second.labels) cudaFree(it->second.labels);
   h->scenes.erase(it);
   memset(&h->table.s[scene_id], 0, sizeof(SceneDesc));
   API_END
@@ -135,7 +122,7 @@ static void gather_dev_impl(drs_handle_t h, const int32_t* inst_host, const uint
   if (noise_host) need += round_up((size_t)pp * C * 8, 256);
   if (over_x_host) need += round_up((size_t)pp * C * 8, 256) + round_up((size_t)pp, 256);
   ensure_dstage(h, need + 1024);
-  char* d = (char*)h->dstage;
+  char* d = h->dstage;
   GatherParams gp;
   memset(&gp, 0, sizeof(gp));
   auto put = [&](const void* src, size_t bytes) -> void* {
@@ -213,17 +200,8 @@ extern "C" int drs_gather_plan_dev(drs_handle_t h, const int32_t* inst_host, con
   const size_t need = small + (has_noise ? round_up((size_t)noise_count * 8, 256) : 0) + 1024;
   const int s = (int)(h->plan_calls++ & 1);
   if (h->plan_consumed_valid[s]) CUDA_CHECK(cudaStreamWaitEvent(h->plan_stream, h->plan_consumed[s], 0));
-  if (h->plan_stage_cap[s] < need) {
-    CUDA_CHECK(cudaStreamSynchronize(h->stream));
-    CUDA_CHECK(cudaStreamSynchronize(h->plan_stream));
-    if (h->plan_stage[s]) CUDA_CHECK(cudaFree(h->plan_stage[s]));
-    h->plan_stage[s] = nullptr;
-    h->plan_stage_cap[s] = 0;
-    const size_t want = need + (need >> 1);
-    CUDA_CHECK(cudaMalloc(&h->plan_stage[s], want));
-    h->plan_stage_cap[s] = want;
-  }
-  char* d = (char*)h->plan_stage[s];
+  h->plan_stage[s].grow(need, need + (need >> 1), {h->stream, h->plan_stream});
+  char* d = h->plan_stage[s];
   auto put = [&](const void* src, size_t bytes) -> void* {
     void* dst = d;
     CUDA_CHECK(cudaMemcpyAsync(dst, src, bytes, cudaMemcpyHostToDevice, h->plan_stream));
@@ -296,15 +274,7 @@ static void build_cells(const std::vector<int32_t>& pos, int H, int W, int crop,
   for (int64_t p = 0; p < P; ++p) ct.seq[fill[cell_of[p]]++] = (int32_t)p;   // ascending visit order per cell
 }
 
-struct ScenePass {
-  float* prob = nullptr;
-  uint32_t* occur = nullptr;
-  int32_t* cell_off = nullptr;
-  int32_t* cell_seq = nullptr;
-  void release() { prob = nullptr; occur = nullptr; cell_off = cell_seq = nullptr; }   // buffers live in the handle's slots
-};
-
-static void accumulate_chunk(Handle* h, const ScenePass& sp, const CellTables& ct, const float* logits, const std::vector<int32_t>& pos,
+static void accumulate_chunk(Handle* h, const CellTables& ct, const float* logits, const std::vector<int32_t>& pos,
                              int seq0, int seq1, int H, int W, int K, int crop, int row_begin, int row_end) {
   int y_lo = H, y_hi = 0;
   for (int s = seq0; s < seq1; ++s) {
@@ -315,7 +285,7 @@ static void accumulate_chunk(Handle* h, const ScenePass& sp, const CellTables& c
   y_hi = std::min(y_hi, row_end);
   if (y_hi <= y_lo) return;
   AccumParams ap;
-  ap.logits = logits; ap.cell_off = sp.cell_off; ap.cell_seq = sp.cell_seq; ap.prob = sp.prob; ap.occur = sp.occur;
+  ap.logits = logits; ap.cell_off = h->pass.cell_off; ap.cell_seq = h->pass.cell_seq; ap.prob = h->pass.prob; ap.occur = h->pass.occur;
   ap.H = H; ap.W = W; ap.K = K; ap.crop = crop; ap.stride = ct.stride; ap.nh = ct.nh; ap.nw = ct.nw;
   ap.row_begin = row_begin; ap.row_end = row_end; ap.y_lo = y_lo; ap.y_hi = y_hi; ap.seq0 = seq0; ap.seq1 = seq1;
   ap.overflow = h->diag_dev + 15;
@@ -324,22 +294,22 @@ static void accumulate_chunk(Handle* h, const ScenePass& sp, const CellTables& c
   LAUNCH_CHECK(h);
 }
 
-static void scene_pass_begin(Handle* h, ScenePass& sp, const CellTables& ct, int rows, int W, int K) {
-  sp.prob = (float*)slot_buf(h, 0, (size_t)rows * W * K * 4);
-  sp.occur = (uint32_t*)slot_buf(h, 1, (size_t)rows * W * 4);
-  sp.cell_off = (int32_t*)slot_buf(h, 2, ct.off.size() * 4);
-  sp.cell_seq = (int32_t*)slot_buf(h, 3, std::max<size_t>(ct.seq.size(), 1) * 4);
-  CUDA_CHECK(cudaMemsetAsync(sp.prob, 0, (size_t)rows * W * K * 4, h->stream));
-  CUDA_CHECK(cudaMemsetAsync(sp.occur, 0, (size_t)rows * W * 4, h->stream));
-  CUDA_CHECK(cudaMemcpyAsync(sp.cell_off, ct.off.data(), ct.off.size() * 4, cudaMemcpyHostToDevice, h->stream));
-  if (!ct.seq.empty()) CUDA_CHECK(cudaMemcpyAsync(sp.cell_seq, ct.seq.data(), ct.seq.size() * 4, cudaMemcpyHostToDevice, h->stream));
+static void scene_pass_begin(Handle* h, const CellTables& ct, int rows, int W, int K) {
+  float* prob = pass_buf(h, h->pass.prob, (size_t)rows * W * K * 4);
+  uint32_t* occur = pass_buf(h, h->pass.occur, (size_t)rows * W * 4);
+  int32_t* cell_off = pass_buf(h, h->pass.cell_off, ct.off.size() * 4);
+  int32_t* cell_seq = pass_buf(h, h->pass.cell_seq, std::max<size_t>(ct.seq.size(), 1) * 4);
+  CUDA_CHECK(cudaMemsetAsync(prob, 0, (size_t)rows * W * K * 4, h->stream));
+  CUDA_CHECK(cudaMemsetAsync(occur, 0, (size_t)rows * W * 4, h->stream));
+  CUDA_CHECK(cudaMemcpyAsync(cell_off, ct.off.data(), ct.off.size() * 4, cudaMemcpyHostToDevice, h->stream));
+  if (!ct.seq.empty()) CUDA_CHECK(cudaMemcpyAsync(cell_seq, ct.seq.data(), ct.seq.size() * 4, cudaMemcpyHostToDevice, h->stream));
 }
 
-static void scene_pass_finish(Handle* h, ScenePass& sp, int rows, int W, int K, uint8_t* labels_host, double* mean_host) {
+static void scene_pass_finish(Handle* h, int rows, int W, int K, uint8_t* labels_host, double* mean_host) {
   const int64_t npix = (int64_t)rows * W;
-  uint8_t* lab_dev = (uint8_t*)slot_buf(h, 4, npix);
-  double* mean_dev = mean_host ? (double*)slot_buf(h, 5, npix * K * 8) : nullptr;
-  scene_argmax_kernel<<<nblk(npix, 256), 256, 0, h->stream>>>(sp.prob, sp.occur, npix, K, lab_dev, mean_dev);
+  uint8_t* lab_dev = pass_buf(h, h->pass.labels, npix);
+  double* mean_dev = mean_host ? pass_buf(h, h->pass.mean, npix * K * 8) : nullptr;
+  scene_argmax_kernel<<<nblk(npix, 256), 256, 0, h->stream>>>(h->pass.prob, h->pass.occur, npix, K, lab_dev, mean_dev);
   LAUNCH_CHECK(h);
   if (labels_host) CUDA_CHECK(cudaMemcpyAsync(labels_host, lab_dev, npix, cudaMemcpyDeviceToHost, h->stream));
   if (mean_host) CUDA_CHECK(cudaMemcpyAsync(mean_host, mean_dev, npix * K * 8, cudaMemcpyDeviceToHost, h->stream));
@@ -359,52 +329,26 @@ extern "C" int drs_accumulate_argmax(drs_handle_t h, const float* logits_dev, co
   std::vector<int32_t> pos(pos_host, pos_host + (size_t)P * 2);
   CellTables ct;
   build_cells(pos, H, W, crop, ct);
-  ScenePass sp;
-  try {
-    scene_pass_begin(h, sp, ct, H, W, K);
-    accumulate_chunk(h, sp, ct, logits_dev, pos, 0, P, H, W, K, crop, 0, H);
-    scene_pass_finish(h, sp, H, W, K, labels_out_host, mean_out_host);
-  } catch (...) { sp.release(); throw; }
-  sp.release();
+  scene_pass_begin(h, ct, H, W, K);
+  accumulate_chunk(h, ct, logits_dev, pos, 0, P, H, W, K, crop, 0, H);
+  scene_pass_finish(h, H, W, K, labels_out_host, mean_out_host);
   API_END
 }
 
 // The chunks of a scene run on a lane of their own (stream + workspace); the ordered accumulation stays on the handle's
 // stream, chunk after chunk, so per-pixel sums keep the script's visiting order.  The lane is kept in the handle between
 // calls (its workspace is several GB for a Potsdam tile).
-static void lane_release(Handle* h) {
-  InferLane& L = h->lane;
-  if (L.stream) { cudaStreamSynchronize(L.stream); cudaStreamDestroy(L.stream); }
-  if (L.arena.base) cudaFree(L.arena.base);
-  if (L.x) cudaFree(L.x);
-  if (L.lg) cudaFree(L.lg);
-  if (L.fwd_done) cudaEventDestroy(L.fwd_done);
-  if (L.acc_done) cudaEventDestroy(L.acc_done);
-  L = InferLane();
-  if (h->lane_ready) cudaEventDestroy(h->lane_ready);
-  h->lane_ready = nullptr;
-}
 static void lane_ensure(Handle* h, size_t arena_bytes, size_t x_bytes, size_t lg_bytes) {
-  if (!h->lane_ready) CUDA_CHECK(cudaEventCreateWithFlags(&h->lane_ready, cudaEventDisableTiming));
+  if (!h->lane_ready) h->lane_ready = new_event();
   InferLane& L = h->lane;
   if (!L.stream) {
-    CUDA_CHECK(cudaStreamCreateWithFlags(&L.stream, cudaStreamNonBlocking));
-    CUDA_CHECK(cudaEventCreateWithFlags(&L.fwd_done, cudaEventDisableTiming));
-    CUDA_CHECK(cudaEventCreateWithFlags(&L.acc_done, cudaEventDisableTiming));
+    L.stream = new_stream();
+    L.fwd_done = new_event();
+    L.acc_done = new_event();
   }
-  if (L.arena.cap < arena_bytes || L.x_cap < x_bytes || L.lg_cap < lg_bytes) {
-    CUDA_CHECK(cudaStreamSynchronize(L.stream));
-    if (L.arena.base) cudaFree(L.arena.base);
-    if (L.x) cudaFree(L.x);
-    if (L.lg) cudaFree(L.lg);
-    L.arena = Arena(); L.x = L.lg = nullptr; L.x_cap = L.lg_cap = 0;
-    CUDA_CHECK(cudaMalloc(&L.arena.base, arena_bytes));
-    L.arena.cap = arena_bytes;
-    CUDA_CHECK(cudaMalloc(&L.x, x_bytes));
-    L.x_cap = x_bytes;
-    CUDA_CHECK(cudaMalloc(&L.lg, lg_bytes));
-    L.lg_cap = lg_bytes;
-  }
+  L.arena.mem.grow(arena_bytes, arena_bytes, {L.stream});
+  L.x.grow(x_bytes, x_bytes, {L.stream});
+  L.lg.grow(lg_bytes, lg_bytes, {L.stream});
 }
 
 // Streamed upload of a host scene during a scene pass: rows are copied on a separate stream, in ~8 MB pieces, just ahead of
@@ -414,7 +358,7 @@ struct HostSceneFeed {
   const char* host = nullptr;    // [H,W,C] in the scene dtype, row-major
   size_t row_bytes = 0;
   int uploaded = 0;              // rows [0, uploaded) are enqueued
-  bool recorded = false;         // up_ev[0] has been recorded at least once during this pass
+  bool recorded = false;         // up_ev has been recorded at least once during this pass
 };
 
 static void feed_rows(Handle* h, HostSceneFeed& f, const Scene& sc, int rows_needed, cudaStream_t consumer) {
@@ -425,18 +369,18 @@ static void feed_rows(Handle* h, HostSceneFeed& f, const Scene& sc, int rows_nee
     const int n = std::min(rows_per_piece, rows_needed - f.uploaded);
     // Pageable source: the driver stages the piece itself (measured faster than a memcpy into our own pinned ring) and
     // returns once the source has been read; kernels already queued keep the GPU busy meanwhile.
-    CUDA_CHECK(cudaMemcpyAsync((char*)sc.data + (size_t)f.uploaded * f.row_bytes, f.host + (size_t)f.uploaded * f.row_bytes,
+    CUDA_CHECK(cudaMemcpyAsync((char*)sc.data.get() + (size_t)f.uploaded * f.row_bytes, f.host + (size_t)f.uploaded * f.row_bytes,
                                (size_t)n * f.row_bytes, cudaMemcpyHostToDevice, h->copy_stream));
     f.uploaded += n;
     any = true;
   }
   if (any) {
-    CUDA_CHECK(cudaEventRecord(h->up_ev[0], h->copy_stream));
+    CUDA_CHECK(cudaEventRecord(h->up_ev, h->copy_stream));
     f.recorded = true;
   }
   // The consumer waits for the latest "rows uploaded" event (copies on one stream complete in order, so it covers every
   // earlier piece).
-  if (f.recorded) CUDA_CHECK(cudaStreamWaitEvent(consumer, h->up_ev[0], 0));
+  if (f.recorded) CUDA_CHECK(cudaStreamWaitEvent(consumer, h->up_ev, 0));
 }
 
 static void scene_infer_impl(drs_handle_t h, int32_t scene_id, int32_t crop, int32_t batch, int32_t variant, int32_t row_begin,
@@ -462,17 +406,12 @@ extern "C" int drs_scene_infer_host(drs_handle_t h, int32_t scene_id, const void
   CUDA_CHECK(cudaStreamSynchronize(h->stream));
   const size_t row_bytes = (size_t)W * C * (dtype == DRS_SCENE_F64 ? 8 : 4);
   const size_t bytes = row_bytes * H;
-  if (s.data_cap < bytes) {
-    if (s.data) CUDA_CHECK(cudaFree(s.data));
-    s.data = nullptr; s.data_cap = 0;
-    CUDA_CHECK(cudaMalloc(&s.data, bytes));
-    s.data_cap = bytes;
-  }
-  if (s.labels) { CUDA_CHECK(cudaFree(s.labels)); s.labels = nullptr; s.labels_cap = 0; }
+  s.data.grow(bytes, bytes);
+  s.labels.reset();
   s.H = H; s.W = W; s.C = C; s.dtype = dtype; s.row0 = 0; s.rows = H;
   h->table.s[scene_id] = SceneDesc{s.data, s.labels, H, W, C, dtype, 0, H};
-  if (!h->copy_stream) CUDA_CHECK(cudaStreamCreateWithFlags(&h->copy_stream, cudaStreamNonBlocking));
-  if (!h->up_ev[0]) CUDA_CHECK(cudaEventCreateWithFlags(&h->up_ev[0], cudaEventDisableTiming));
+  if (!h->copy_stream) h->copy_stream = new_stream();
+  if (!h->up_ev) h->up_ev = new_event();
   HostSceneFeed feed;
   feed.host = (const char*)scene_host;
   feed.row_bytes = row_bytes;
@@ -529,18 +468,15 @@ static void scene_infer_impl(drs_handle_t h, int32_t scene_id, int32_t crop, int
   const int waves = getenv("DRS_CHUNK_WAVES") ? std::max(1, atoi(getenv("DRS_CHUNK_WAVES"))) : 40;
   const int64_t target_tiles = (int64_t)h->sm_count * waves;
   int chunk = (int)std::max<int64_t>(1, std::min<int64_t>(P, (target_tiles * CONV_TC_BM) / pp));
-  ScenePass sp;
-  int32_t* inst_dev = nullptr;
   const cudaStream_t main_stream = h->stream;
   auto cleanup = [&]() {
     cudaStreamSynchronize(main_stream);
     if (h->lane.stream) cudaStreamSynchronize(h->lane.stream);
-    sp.release();
   };
   try {
-    scene_pass_begin(h, sp, ct, rows, W, K);
+    scene_pass_begin(h, ct, rows, W, K);
     const std::vector<int32_t>& inst = pg.inst;
-    inst_dev = (int32_t*)slot_buf(h, 6, std::max<size_t>(inst.size(), 1) * 4);
+    int32_t* inst_dev = pass_buf(h, h->pass.inst, std::max<size_t>(inst.size(), 1) * 4);
     CUDA_CHECK(cudaMemcpyAsync(inst_dev, inst.data(), inst.size() * 4, cudaMemcpyHostToDevice, h->stream));
     refresh_packed(h, false);                       // packed weights / folded BN once, before the lane starts
     lane_ensure(h, eval_arena_bytes(h, chunk, crop), (size_t)chunk * pp * C * 4, (size_t)chunk * pp * K * 4);
@@ -570,10 +506,10 @@ static void scene_infer_impl(drs_handle_t h, int32_t scene_id, int32_t crop, int
         CUDA_CHECK(cudaEventRecord(L.fwd_done, L.stream));
       }
       CUDA_CHECK(cudaStreamWaitEvent(main_stream, L.fwd_done, 0));
-      accumulate_chunk(h, sp, ct, L.lg, pos, s0, s0 + nb, H, W, K, crop, row_begin, row_end);
+      accumulate_chunk(h, ct, L.lg, pos, s0, s0 + nb, H, W, K, crop, row_begin, row_end);
       CUDA_CHECK(cudaEventRecord(L.acc_done, main_stream));
     }
-    scene_pass_finish(h, sp, rows, W, K, labels_out_host, mean_out_host);
+    scene_pass_finish(h, rows, W, K, labels_out_host, mean_out_host);
     h->last_scene = scene_id; h->last_row_begin = row_begin; h->last_rows = rows; h->last_W = W;
     if (feed) {                                      // rows no patch reads (none for the grids of the scripts) and the tail
       feed_rows(h, *feed, sc, sc.H, main_stream);
@@ -595,14 +531,14 @@ extern "C" int drs_scene_confusion(drs_handle_t h, int32_t scene_id, int32_t K, 
   DRS_CHECK(it != h->scenes.end(), "scene_confusion: scene %d not uploaded", scene_id);
   const Scene& sc = it->second;
   DRS_CHECK(sc.labels, "scene_confusion: scene %d was uploaded without labels", scene_id);
-  DRS_CHECK(h->last_scene == scene_id && h->slot_ptr[4], "scene_confusion: no label map of scene %d is resident (run drs_scene_infer first)", scene_id);
+  DRS_CHECK(h->last_scene == scene_id && h->pass.labels, "scene_confusion: no label map of scene %d is resident (run drs_scene_infer first)", scene_id);
   DRS_CHECK(h->last_W == sc.W && h->last_row_begin >= sc.row0 && h->last_row_begin + h->last_rows <= sc.row0 + sc.rows,
             "scene_confusion: label rows [%d,%d) outside the resident ground truth", h->last_row_begin, h->last_row_begin + h->last_rows);
   const int64_t n = (int64_t)h->last_rows * sc.W;
   const uint8_t* truth = sc.labels + (int64_t)(h->last_row_begin - sc.row0) * sc.W;
   CUDA_CHECK(cudaMemsetAsync(h->cm_dev, 0, (K * K + 1) * 4, h->stream));
   const unsigned blocks = (unsigned)std::min<int64_t>(ceil_div(std::max<int64_t>(n, 1), 256), (int64_t)h->sm_count * 8);
-  confusion_kernel<<<blocks, 256, 0, h->stream>>>(truth, (const uint8_t*)h->slot_ptr[4], nullptr, n, K, ignore_label, h->cm_dev);
+  confusion_kernel<<<blocks, 256, 0, h->stream>>>(truth, h->pass.labels, nullptr, n, K, ignore_label, h->cm_dev);
   LAUNCH_CHECK(h);
   CUDA_CHECK(cudaMemcpyAsync(cm_out_host, h->cm_dev, (K * K + 1) * 4, cudaMemcpyDeviceToHost, h->stream));
   CUDA_CHECK(cudaStreamSynchronize(h->stream));
@@ -667,16 +603,13 @@ extern "C" int drs_debug_activation(drs_handle_t h, const char* name, float* out
   DRS_CHECK(it != h->taps.end(), "no activation recorded for scope '%s'", name);
   const Handle::Tap& t = it->second;
   DRS_CHECK(count == t.pixels * t.co, "activation '%s' has %lld elements, got %lld", name, (long long)(t.pixels * t.co), (long long)count);
-  float* tmp = nullptr;
-  CUDA_CHECK(cudaMalloc(&tmp, count * 4));
+  DevMem<float> tmp(count * 4);
   if (t.type == ET_F32) slice_to_f32_kernel<float><<<nblk(count, 256), 256, 0, h->stream>>>((const float*)t.ptr, t.cstride, t.coff, t.co, t.pixels, tmp);
   else if (t.type == ET_F16) slice_to_f32_kernel<__half><<<nblk(count, 256), 256, 0, h->stream>>>((const __half*)t.ptr, t.cstride, t.coff, t.co, t.pixels, tmp);
   else slice_to_f32_kernel<__nv_bfloat16><<<nblk(count, 256), 256, 0, h->stream>>>((const __nv_bfloat16*)t.ptr, t.cstride, t.coff, t.co, t.pixels, tmp);
   h->launches++;
-  cudaError_t e = cudaMemcpyAsync(out_host, tmp, count * 4, cudaMemcpyDeviceToHost, h->stream);
-  if (e == cudaSuccess) e = cudaStreamSynchronize(h->stream);
-  cudaFree(tmp);
-  CUDA_CHECK(e);
+  CUDA_CHECK(cudaMemcpyAsync(out_host, tmp, count * 4, cudaMemcpyDeviceToHost, h->stream));
+  CUDA_CHECK(cudaStreamSynchronize(h->stream));
   API_END
 }
 
@@ -703,35 +636,24 @@ extern "C" int drs_debug_conv(drs_handle_t h, const float* x_host, const float* 
   const int64_t M = (int64_t)B * crop * crop;
   const int64_t nw = (int64_t)k * k * Ci * Co;
   const ConvLayer c = conv_shape(k, rate, Ci, Co);
-  float *x32 = nullptr, *w32 = nullptr, *sc = nullptr, *sh = nullptr, *y32 = nullptr;
-  void *xa = nullptr, *wp = nullptr, *ya = nullptr;
-  auto cleanup = [&]() {
-    cudaFree(x32); cudaFree(w32); cudaFree(sc); cudaFree(sh); cudaFree(y32); cudaFree(xa); cudaFree(wp); cudaFree(ya);
-  };
-  try {
-    CUDA_CHECK(cudaMalloc(&x32, M * Ci * 4));
-    CUDA_CHECK(cudaMalloc(&w32, nw * 4));
-    CUDA_CHECK(cudaMalloc(&sc, Co * 4));
-    CUDA_CHECK(cudaMalloc(&sh, Co * 4));
-    CUDA_CHECK(cudaMalloc(&y32, M * Co * 4));
-    CUDA_CHECK(cudaMemcpyAsync(x32, x_host, M * Ci * 4, cudaMemcpyHostToDevice, h->stream));
-    CUDA_CHECK(cudaMemcpyAsync(w32, w_host, nw * 4, cudaMemcpyHostToDevice, h->stream));
-    CUDA_CHECK(cudaMemcpyAsync(sc, scale_host, Co * 4, cudaMemcpyHostToDevice, h->stream));
-    CUDA_CHECK(cudaMemcpyAsync(sh, shift_host, Co * 4, cudaMemcpyHostToDevice, h->stream));
-    if (precision == DRS_PREC_FP32) {
-      run_conv<float>(h, ActBuf{x32, Ci, 0}, Ci, w32, nullptr, ActBuf{y32, Co, 0}, Co, B, crop, k, rate, c.pad_b, sc, sh, act);
-    } else {
-      CUDA_CHECK(cudaMalloc(&xa, M * Ci * 2));
-      CUDA_CHECK(cudaMalloc(&wp, nw * 2));
-      CUDA_CHECK(cudaMalloc(&ya, M * Co * 2));
-      if (precision == DRS_PREC_F16) debug_conv_tc<__half>(h, x32, w32, sc, sh, c, B, crop, act, (__half*)xa, wp, (__half*)ya, y32);
-      else debug_conv_tc<__nv_bfloat16>(h, x32, w32, sc, sh, c, B, crop, act, (__nv_bfloat16*)xa, wp, (__nv_bfloat16*)ya, y32);
-    }
-    CUDA_CHECK(cudaMemcpyAsync(y_host, y32, M * Co * 4, cudaMemcpyDeviceToHost, h->stream));
-    int rc = drs_synchronize(h);
-    if (rc) throw DrsError{rc};
-  } catch (...) { cleanup(); throw; }
-  cleanup();
+  DevMem<float> x32(M * Ci * 4), w32(nw * 4), sc(Co * 4), sh(Co * 4), y32(M * Co * 4);
+  DevMem<void> xa, wp, ya;   // 16-bit operands; like the rest freed on return, after the synchronize
+  CUDA_CHECK(cudaMemcpyAsync(x32, x_host, M * Ci * 4, cudaMemcpyHostToDevice, h->stream));
+  CUDA_CHECK(cudaMemcpyAsync(w32, w_host, nw * 4, cudaMemcpyHostToDevice, h->stream));
+  CUDA_CHECK(cudaMemcpyAsync(sc, scale_host, Co * 4, cudaMemcpyHostToDevice, h->stream));
+  CUDA_CHECK(cudaMemcpyAsync(sh, shift_host, Co * 4, cudaMemcpyHostToDevice, h->stream));
+  if (precision == DRS_PREC_FP32) {
+    run_conv<float>(h, ActBuf{x32, Ci, 0}, Ci, w32, nullptr, ActBuf{y32, Co, 0}, Co, B, crop, k, rate, c.pad_b, sc, sh, act);
+  } else {
+    xa = DevMem<void>(M * Ci * 2);
+    wp = DevMem<void>(nw * 2);
+    ya = DevMem<void>(M * Co * 2);
+    if (precision == DRS_PREC_F16) debug_conv_tc<__half>(h, x32, w32, sc, sh, c, B, crop, act, (__half*)xa.get(), wp, (__half*)ya.get(), y32);
+    else debug_conv_tc<__nv_bfloat16>(h, x32, w32, sc, sh, c, B, crop, act, (__nv_bfloat16*)xa.get(), wp, (__nv_bfloat16*)ya.get(), y32);
+  }
+  CUDA_CHECK(cudaMemcpyAsync(y_host, y32, M * Co * 4, cudaMemcpyDeviceToHost, h->stream));
+  int rc = drs_synchronize(h);
+  if (rc) return rc;
   API_END
 }
 
@@ -754,48 +676,34 @@ extern "C" int drs_bench_conv(drs_handle_t h, int32_t B, int32_t crop, int32_t k
   const int64_t M = (int64_t)B * crop * crop;
   const int64_t nw = (int64_t)k * k * Ci * Co;
   const int pad_b = ((k - 1) * rate) / 2;
-  void *xa = nullptr, *wp = nullptr, *ya = nullptr;
-  float* sc = nullptr;
-  cudaEvent_t e0 = nullptr, e1 = nullptr;
-  auto cleanup = [&]() {
-    cudaFree(xa); cudaFree(wp); cudaFree(ya); cudaFree(sc);
-    if (e0) cudaEventDestroy(e0);
-    if (e1) cudaEventDestroy(e1);
-    g_conv_exp_mode = -1;
-  };
-  try {
-    const int bf = precision == DRS_PREC_BF16;
-    CUDA_CHECK(cudaMalloc(&xa, M * Ci * 2));
-    CUDA_CHECK(cudaMalloc(&wp, nw * 2));
-    CUDA_CHECK(cudaMalloc(&ya, M * Co * 2));
-    CUDA_CHECK(cudaMalloc(&sc, 2 * 256 * 4));
-    bench_fill_kernel<<<1024, 256, 0, h->stream>>>((uint16_t*)xa, M * Ci, 1u, bf);
-    bench_fill_kernel<<<256, 256, 0, h->stream>>>((uint16_t*)wp, nw, 2u, bf);
-    {
-      std::vector<float> one_zero(512, 0.0f);
-      for (int i = 0; i < 256; ++i) one_zero[i] = 1.0f;
-      CUDA_CHECK(cudaMemcpy(sc, one_zero.data(), 512 * 4, cudaMemcpyHostToDevice));
-    }
-    CUDA_CHECK(cudaEventCreate(&e0));
-    CUDA_CHECK(cudaEventCreate(&e1));
-    ConvTcArgs a;
-    a.in = xa; a.in_cstride = Ci; a.in_coff = 0; a.ci = Ci; a.w = wp; a.out = ya; a.out_cstride = Co; a.out_coff = 0; a.co = Co;
-    a.B = B; a.crop = crop; a.k = k; a.rate = rate; a.pad_b = pad_b; a.scale = sc; a.shift = sc + 256; a.act = ACT_RELU;
-    a.etype = bf ? ET_BF16 : ET_F16;
-    g_conv_exp_mode = exp_mode;
-    launch_conv_tc(h, a);                       // warm-up (tensor maps, module load)
-    CUDA_CHECK(cudaEventRecord(e0, h->stream));
-    for (int r = 0; r < reps; ++r) launch_conv_tc(h, a);
-    CUDA_CHECK(cudaEventRecord(e1, h->stream));
-    int rc = drs_synchronize(h);
-    if (rc) throw DrsError{rc};
-    float ms = 0.0f;
-    CUDA_CHECK(cudaEventElapsedTime(&ms, e0, e1));
-    *ms_out = ms / reps;
-    // instrumented launches (exp_mode bit 16): cycle counters of CTA 0's last launch
-    if (instr_out) for (int i = 0; i < 10; ++i) instr_out[i] = h->diag_host[4 + i];
-  } catch (...) { cleanup(); throw; }
-  cleanup();
+  struct ExpModeReset { ~ExpModeReset() { g_conv_exp_mode = -1; } } exp_mode_reset;   // on every way out
+  const int bf = precision == DRS_PREC_BF16;
+  DevMem<uint16_t> xa(M * Ci * 2), wp(nw * 2), ya(M * Co * 2);
+  DevMem<float> sc(2 * 256 * 4);
+  bench_fill_kernel<<<1024, 256, 0, h->stream>>>(xa, M * Ci, 1u, bf);
+  bench_fill_kernel<<<256, 256, 0, h->stream>>>(wp, nw, 2u, bf);
+  {
+    std::vector<float> one_zero(512, 0.0f);
+    for (int i = 0; i < 256; ++i) one_zero[i] = 1.0f;
+    CUDA_CHECK(cudaMemcpy(sc, one_zero.data(), 512 * 4, cudaMemcpyHostToDevice));
+  }
+  Event e0 = new_event(cudaEventDefault), e1 = new_event(cudaEventDefault);
+  ConvTcArgs a;
+  a.in = xa; a.in_cstride = Ci; a.in_coff = 0; a.ci = Ci; a.w = wp; a.out = ya; a.out_cstride = Co; a.out_coff = 0; a.co = Co;
+  a.B = B; a.crop = crop; a.k = k; a.rate = rate; a.pad_b = pad_b; a.scale = sc; a.shift = sc + 256; a.act = ACT_RELU;
+  a.etype = bf ? ET_BF16 : ET_F16;
+  g_conv_exp_mode = exp_mode;
+  launch_conv_tc(h, a);                       // warm-up (tensor maps, module load)
+  CUDA_CHECK(cudaEventRecord(e0, h->stream));
+  for (int r = 0; r < reps; ++r) launch_conv_tc(h, a);
+  CUDA_CHECK(cudaEventRecord(e1, h->stream));
+  int rc = drs_synchronize(h);
+  if (rc) return rc;
+  float ms = 0.0f;
+  CUDA_CHECK(cudaEventElapsedTime(&ms, e0, e1));
+  *ms_out = ms / reps;
+  // instrumented launches (exp_mode bit 16): cycle counters of CTA 0's last launch
+  if (instr_out) for (int i = 0; i < 10; ++i) instr_out[i] = h->diag_host[4 + i];
   API_END
 }
 
@@ -808,33 +716,25 @@ extern "C" int drs_debug_wgrad(drs_handle_t h, const float* x_host, const float*
   const int64_t M = (int64_t)B * crop * crop;
   const int64_t nw = (int64_t)k * k * Ci * Co;
   const ConvLayer c = conv_shape(k, rate, Ci, Co);
-  float *x32 = nullptr, *dy32 = nullptr, *dw = nullptr, *part = nullptr;
-  void *xa = nullptr, *dya = nullptr;
-  auto cleanup = [&]() { cudaFree(x32); cudaFree(dy32); cudaFree(dw); cudaFree(part); cudaFree(xa); cudaFree(dya); };
-  try {
-    CUDA_CHECK(cudaMalloc(&x32, M * Ci * 4));
-    CUDA_CHECK(cudaMalloc(&dy32, M * Co * 4));
-    CUDA_CHECK(cudaMalloc(&dw, nw * 4));
-    // (the tensor-core kernel runs 32-channel operands as 64: its split partials have the padded shape)
-    const size_t part_cap = (size_t)k * k * ((Ci + 63) / 64 * 64) * ((Co + 63) / 64 * 64) * WGRAD_MAX_SPLITS;
-    CUDA_CHECK(cudaMalloc(&part, part_cap * 4));
-    CUDA_CHECK(cudaMemcpyAsync(x32, x_host, M * Ci * 4, cudaMemcpyHostToDevice, h->stream));
-    CUDA_CHECK(cudaMemcpyAsync(dy32, dy_host, M * Co * 4, cudaMemcpyHostToDevice, h->stream));
-    if (precision == DRS_PREC_FP32) {
-      filter_gradient<float>(h, c, ActBuf{x32, Ci, 0}, nullptr, nullptr, dy32, B, crop, dw, part, part_cap);
-    } else {
-      DRS_CHECK(precision == DRS_PREC_BF16, "debug_wgrad: precision must be FP32 or BF16");
-      CUDA_CHECK(cudaMalloc(&xa, M * Ci * 2));
-      CUDA_CHECK(cudaMalloc(&dya, M * Co * 2));
-      cast_kernel<float, __nv_bfloat16><<<nblk(M * Ci, 256), 256, 0, h->stream>>>(x32, (__nv_bfloat16*)xa, M * Ci);
-      cast_kernel<float, __nv_bfloat16><<<nblk(M * Co, 256), 256, 0, h->stream>>>(dy32, (__nv_bfloat16*)dya, M * Co);
-      h->launches += 2;
-      filter_gradient<__nv_bfloat16>(h, c, ActBuf{xa, Ci, 0}, nullptr, nullptr, (const __nv_bfloat16*)dya, B, crop, dw, part, part_cap);
-    }
-    CUDA_CHECK(cudaMemcpyAsync(dw_host, dw, nw * 4, cudaMemcpyDeviceToHost, h->stream));
-    int rc = drs_synchronize(h);
-    if (rc) throw DrsError{rc};
-  } catch (...) { cleanup(); throw; }
-  cleanup();
+  // (the tensor-core kernel runs 32-channel operands as 64: its split partials have the padded shape)
+  const size_t part_cap = (size_t)k * k * ((Ci + 63) / 64 * 64) * ((Co + 63) / 64 * 64) * WGRAD_MAX_SPLITS;
+  DevMem<float> x32(M * Ci * 4), dy32(M * Co * 4), dw(nw * 4), part(part_cap * 4);
+  DevMem<__nv_bfloat16> xa, dya;   // bf16 operands; like the rest freed on return, after the synchronize
+  CUDA_CHECK(cudaMemcpyAsync(x32, x_host, M * Ci * 4, cudaMemcpyHostToDevice, h->stream));
+  CUDA_CHECK(cudaMemcpyAsync(dy32, dy_host, M * Co * 4, cudaMemcpyHostToDevice, h->stream));
+  if (precision == DRS_PREC_FP32) {
+    filter_gradient<float>(h, c, ActBuf{x32, Ci, 0}, nullptr, nullptr, dy32, B, crop, dw, part, part_cap);
+  } else {
+    DRS_CHECK(precision == DRS_PREC_BF16, "debug_wgrad: precision must be FP32 or BF16");
+    xa = DevMem<__nv_bfloat16>(M * Ci * 2);
+    dya = DevMem<__nv_bfloat16>(M * Co * 2);
+    cast_kernel<float, __nv_bfloat16><<<nblk(M * Ci, 256), 256, 0, h->stream>>>(x32, xa, M * Ci);
+    cast_kernel<float, __nv_bfloat16><<<nblk(M * Co, 256), 256, 0, h->stream>>>(dy32, dya, M * Co);
+    h->launches += 2;
+    filter_gradient<__nv_bfloat16>(h, c, ActBuf{xa, Ci, 0}, nullptr, nullptr, dya, B, crop, dw, part, part_cap);
+  }
+  CUDA_CHECK(cudaMemcpyAsync(dw_host, dw, nw * 4, cudaMemcpyDeviceToHost, h->stream));
+  int rc = drs_synchronize(h);
+  if (rc) return rc;
   API_END
 }

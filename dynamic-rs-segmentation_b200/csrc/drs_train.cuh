@@ -322,10 +322,10 @@ static void train_step_t(Handle* h, const float* x_dev, const float* y_dev, cons
   refresh_packed(h, true);
 
   ensure_arena(h, layout_bytes<TrainWs<TA>>(h, B, crop));
-  h->arena.reset();
+  h->arena->reset();
   TrainWs<TA> ws;
   {
-    WsAlloc carve{&h->arena};
+    WsAlloc carve{h->arena};
     ws.layout(h, carve, B, crop);
   }
   uint8_t* pred = pred_out_dev ? pred_out_dev : ws.pred;
@@ -368,8 +368,8 @@ static void train_step_t(Handle* h, const float* x_dev, const float* y_dev, cons
     if (l == 0 && ws.x8) {
       // conv1 on the tensor cores as in inference (conv1_tc.cuh): input and filter rounded to bf16 like every other layer's
       // operands; the filter is re-packed every step (13 K elements).  The filter gradient keeps the fp32 input.
-      if (!c.w_fprop) CUDA_CHECK(cudaMalloc(&c.w_fprop, (size_t)C1_SLOTS * c.co * 8 * 2));
-      launch_pdl(h, pack_conv1_kernel<TA>, dim3(nblk(C1_SLOTS * c.co * 8, 256)), dim3(256), 0, h->params + c.w_off, (TA*)c.w_fprop, c.ci, c.co);
+      c.w_fprop.grow((size_t)C1_SLOTS * c.co * 8 * 2, (size_t)C1_SLOTS * c.co * 8 * 2);
+      launch_pdl(h, pack_conv1_kernel<TA>, dim3(nblk(C1_SLOTS * c.co * 8, 256)), dim3(256), 0, h->params + c.w_off, (TA*)c.w_fprop.get(), c.ci, c.co);
       LAUNCH_CHECK(h);
       launch_pdl(h, pad_cast8_kernel<TA>, dim3(nblk(M, 256)), dim3(256), 0, x_dev, ws.x8, c.ci, M);
       LAUNCH_CHECK(h);
@@ -477,7 +477,7 @@ static void train_step_t(Handle* h, const float* x_dev, const float* y_dev, cons
     // overlaps the HBM-bound kernels of layer l-1's backward.  dZ is double-buffered; before a buffer is rewritten the
     // main stream waits for the wgrad that read it two layers ago.
     TA* DZ = ws.DZb[l & 1];
-    const ActBuf dA = backward_to_dz(h, norm_layer(l), dOut, ws.T, DZ, l + 2 <= L - 1 ? h->ev_wgrad[l & 1] : nullptr);
+    const ActBuf dA = backward_to_dz(h, norm_layer(l), dOut, ws.T, DZ, l + 2 <= L - 1 ? h->ev_wgrad[l & 1].get() : nullptr);
     if (dA.p) debug_keep<TA>(h, "da:" + c.scope, (const TA*)dA.p, dA.cs, dA.co, c.co, M);
     debug_keep<TA>(h, "dz:" + c.scope, DZ, c.co, 0, c.co, M);
     CUDA_CHECK(cudaEventRecord(h->ev_dz[l & 1], h->stream));
@@ -610,14 +610,16 @@ static void train_step(Handle* h, const float* x_dev, const float* y_dev, const 
       }
       h->capturing = nullptr;
       CUDA_CHECK(cudaStreamEndCapture(h->stream, &graph));
-      cudaError_t e = cudaGraphInstantiate(&g.exec, graph, 0);
+      cudaGraphExec_t exec = nullptr;
+      cudaError_t e = cudaGraphInstantiate(&exec, graph, 0);
       cudaGraphDestroy(graph);
       CUDA_CHECK(e);
+      g.exec = GraphExec(exec);
       CUDA_CHECK(cudaGraphUpload(g.exec, h->stream));   // pay the device-side set-up now, not at the first replay
       g.launches = h->launches - l0;
       g.conv_launches = h->conv_launches - cl0;
       g.conv_flops = h->conv_flops - f0;
-      auto ins = h->graphs.emplace(key, g);
+      auto ins = h->graphs.emplace(key, std::move(g));
       replay = &ins.first->second;
       if (capture_only) {                            // drs_train_prepare: undo the host-side bookkeeping of the dry capture
         h->launches = l0;
@@ -683,7 +685,7 @@ extern "C" int drs_debug_dgrad(drs_handle_t h, const float* dy_host, const float
   const int64_t M = (int64_t)B * crop * crop;
   const int64_t nw = (int64_t)k * k * Ci * Co;
   ensure_arena(h, (size_t)M * (Ci + Co) * 8 + nw * 8 + (1 << 20));
-  h->arena.reset();
+  h->arena->reset();
   float* dy32 = (float*)arena_take(h, M * Co * 4);
   float* w32 = (float*)arena_take(h, nw * 4);
   float* dx32 = (float*)arena_take(h, M * Ci * 4);
@@ -744,7 +746,7 @@ extern "C" int drs_debug_layer(drs_handle_t h, const float* z_host, const float*
   CUDA_CHECK(cudaSetDevice(h->cfg.device));
   const int64_t M = (int64_t)B * crop * crop;
   ensure_arena(h, (size_t)M * C * (4 * 4 + 6 * 4 + 1) + (8 << 20));
-  h->arena.reset();
+  h->arena->reset();
   float* z32 = (float*)arena_take(h, M * C * 4);
   float* g32 = (float*)arena_take(h, M * C * 4);
   float* o32 = (float*)arena_take(h, M * C * 4);
@@ -809,16 +811,7 @@ extern "C" int drs_reserve_workspace(drs_handle_t h, int32_t B, int32_t crop_max
   if (training) {
     // both device staging slots of the planned gather (drs_gather_plan_dev): worst case = every patch noisy
     const size_t need = (size_t)M * C * 8 + (size_t)B * 128 + 8192;
-    for (int s = 0; s < 2; ++s) {
-      if (h->plan_stage_cap[s] >= need) continue;
-      CUDA_CHECK(cudaStreamSynchronize(h->stream));
-      CUDA_CHECK(cudaStreamSynchronize(h->plan_stream));
-      if (h->plan_stage[s]) CUDA_CHECK(cudaFree(h->plan_stage[s]));
-      h->plan_stage[s] = nullptr;
-      h->plan_stage_cap[s] = 0;
-      CUDA_CHECK(cudaMalloc(&h->plan_stage[s], need));
-      h->plan_stage_cap[s] = need;
-    }
+    for (int s = 0; s < 2; ++s) h->plan_stage[s].grow(need, need, {h->stream, h->plan_stream});
   }
   // staging of the *_host entry points (x, y, two masks, int64 + uint8 predictions, confusion counts, logits)
   ensure_dstage(h, round_up((size_t)M * C * 4, 256) + round_up((size_t)M * 4, 256) + 2 * round_up((size_t)M, 256) +
@@ -845,7 +838,7 @@ extern "C" int drs_train_step_host(drs_handle_t h, const float* x_host, const fl
   const int C = h->net.channels, K = h->net.classes;
   const size_t xb = round_up((size_t)M * C * 4, 256), yb = round_up((size_t)M * 4, 256), mb = round_up((size_t)M, 256);
   ensure_dstage(h, xb + yb + 2 * mb + (size_t)M * 9 + 4096 + 1024);
-  char* d = (char*)h->dstage;
+  char* d = h->dstage;
   float* x_dev = (float*)d;
   float* y_dev = (float*)(d + xb);
   uint8_t* m_dev = (uint8_t*)(d + xb + yb);
