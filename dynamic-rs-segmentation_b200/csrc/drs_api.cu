@@ -11,6 +11,8 @@
 #include "conv1_tc.cuh"
 #include "npz_io.h"
 
+#include <functional>
+
 thread_local char g_drs_err[1024] = {0};
 
 #define API_BEGIN try {
@@ -611,6 +613,13 @@ static void repack_filter(Handle* h, const float* w, void* out, int taps, int ci
   LAUNCH_CHECK(h);
 }
 
+// conv1's tensor-core operand (conv1_tc.cuh): the HWIO filter in core-matrix order, C1_SLOTS * co * 8 16-bit elements
+template <typename TA>
+static void pack_conv1(Handle* h, const float* w, void* out, int ci, int co) {
+  launch_pdl(h, pack_conv1_kernel<TA>, dim3(nblk(C1_SLOTS * co * 8, 256)), dim3(256), 0, w, (TA*)out, ci, co);
+  LAUNCH_CHECK(h);
+}
+
 // training needs only the layer operands; inference additionally the folded eval-mode BN and conv1's tensor-core operand
 static void refresh_packed(Handle* h, bool training) {
   const int et = act_type(h);
@@ -651,11 +660,10 @@ static void refresh_packed(Handle* h, bool training) {
       // 16-bit inference runs conv1 on the tensor cores (conv1_tc.cuh) from a core-matrix-ordered operand; training and the
       // fp32 mode run it on the CUDA-core kernel straight from the HWIO weights
       if (l == 0 && et != ET_F32 && conv1_tc_supported(c.k, c.rate, c.ci, c.co)) {
-        const int n = C1_SLOTS * c.co * 8;
-        c.w_fprop.grow((size_t)n * 2, (size_t)n * 2);
-        if (et == ET_F16) pack_conv1_kernel<__half><<<nblk(n, 256), 256, 0, h->stream>>>(h->params + c.w_off, (__half*)c.w_fprop.get(), c.ci, c.co);
-        else pack_conv1_kernel<__nv_bfloat16><<<nblk(n, 256), 256, 0, h->stream>>>(h->params + c.w_off, (__nv_bfloat16*)c.w_fprop.get(), c.ci, c.co);
-        LAUNCH_CHECK(h);
+        const size_t bytes = (size_t)C1_SLOTS * c.co * 8 * 2;
+        c.w_fprop.grow(bytes, bytes);
+        if (et == ET_F16) pack_conv1<__half>(h, h->params + c.w_off, c.w_fprop, c.ci, c.co);
+        else pack_conv1<__nv_bfloat16>(h, h->params + c.w_off, c.w_fprop, c.ci, c.co);
       }
     }
     h->eval_dirty = false;
@@ -733,6 +741,50 @@ static void run_conv(Handle* h, const ActBuf& in, int ci, const float* w_simt, c
   h->conv_launches += nsplit;
 }
 
+// conv1 on the tensor cores (conv1_tc.cuh) for the shapes conv1_tc_supported accepts, in 16-bit: the fp32 input [M, ci] padded
+// to 8 channels and rounded into x8 (pad_cast8_kernel), then the 25-tap kernel from the filter pack_conv1 packed into wpack.
+// The inference forward, the training forward and drs_debug_conv all run conv1 through here.  `on_x8` runs between the two
+// launches (the training forward builds conv1's im2col matrix from x8 there).  `timed`: the launch counts as one of the
+// convolutions of the per-convolution profile (inference; the training profile covers the conv_tc and wgrad_tc kernels).
+template <typename TA>
+static void conv1_tc_forward(Handle* h, const float* x32, int ci, TA* x8, const void* wpack, const ActBuf& out, int co, int B, int crop,
+                             const float* scale, const float* shift, int act, const BnFinish* stats, bool timed,
+                             const std::function<void()>& on_x8 = nullptr) {
+  const int64_t M = (int64_t)B * crop * crop;
+  launch_pdl(h, pad_cast8_kernel<TA>, dim3(nblk(M, 256)), dim3(256), 0, x32, x8, ci, M);
+  LAUNCH_CHECK(h);
+  if (on_x8) on_x8();
+  cudaEvent_t ea = nullptr, eb = nullptr;
+  if (timed) prof_begin(h, &ea, &eb);
+  Conv1TcArgs a;
+  a.x8 = x8; a.wpack = wpack; a.out = out.p; a.out_cstride = out.cs; a.out_coff = out.co; a.co = co;
+  a.B = B; a.crop = crop; a.scale = scale; a.shift = shift; a.act = act; a.etype = ElemTag<TA>::v;
+  a.stats = stats;
+  launch_conv1_tc(h, a);
+  if (!timed) return;
+  prof_end(h, eb);
+  h->conv_flops += 2.0 * (double)M * 25 * ci * co;   // algorithmic FLOPs: the real input channels
+  h->conv_launches += 1;
+}
+
+// DRS_DEBUG_KEEP=1: an fp32 copy of a layer's tensor, registered as the activation tap `name` (the inference forward's
+// feature buffers rotate, and the training step's buffers are reused, so a tap of the buffer itself would not survive)
+template <typename T>
+static void debug_keep(Handle* h, const std::string& name, const T* ptr, int cs, int co, int C, int64_t M) {
+  if (!h->debug_keep) return;
+  h->keep.emplace_back(M * C * 4);
+  float* buf = h->keep.back();
+  slice_to_f32_kernel<T><<<nblk(M * C, 256), 256, 0, h->stream>>>(ptr, cs, co, C, M, buf);
+  LAUNCH_CHECK(h);
+  h->taps[name] = {buf, ET_F32, C, 0, C, M};
+}
+static void debug_keep_reset(Handle* h) {
+  h->debug_keep = getenv("DRS_DEBUG_KEEP") != nullptr;
+  if (h->keep.empty()) return;
+  cudaStreamSynchronize(h->stream);
+  h->keep.clear();
+}
+
 // ------------------------------------------------------------------------------------------------
 // inference forward (eval-mode BN folded into the conv epilogue)
 // ------------------------------------------------------------------------------------------------
@@ -787,6 +839,7 @@ static void forward_eval_t(Handle* h, const float* x_dev, int B, int crop, float
   }
   float* logits = logits_dev ? logits_dev : ws.logits;
   h->taps.clear();
+  debug_keep_reset(h);
 
   ActBuf cur{nullptr, 0, 0};
   int xi = 0;   // index of the buffer holding the current input (non-dense)
@@ -800,17 +853,7 @@ static void forward_eval_t(Handle* h, const float* x_dev, int B, int crop, float
     else if (sq_part >= 1) { cur = {ws.bufs[sq_s], fs, 0}; out = {ws.bufs[sq_c], fs, c.out_coff}; }
     else out = {ws.bufs[(xi + 1) % 3], fs, 0};
     if (l == 0 && ws.x8 && c.w_fprop) {
-      pad_cast8_kernel<TA><<<nblk(M, 256), 256, 0, h->stream>>>(x_dev, ws.x8, c.ci, M);
-      LAUNCH_CHECK(h);
-      cudaEvent_t ea = nullptr, eb = nullptr;
-      prof_begin(h, &ea, &eb);
-      Conv1TcArgs a1;
-      a1.x8 = ws.x8; a1.wpack = c.w_fprop; a1.out = out.p; a1.out_cstride = out.cs; a1.out_coff = out.co; a1.co = c.co;
-      a1.B = B; a1.crop = crop; a1.scale = c.fold_scale; a1.shift = c.fold_shift; a1.act = n.act; a1.etype = ElemTag<TA>::v;
-      launch_conv1_tc(h, a1);
-      prof_end(h, eb);
-      h->conv_flops += 2.0 * (double)M * c.k * c.k * c.ci * c.co;   // algorithmic FLOPs: the real C channels
-      h->conv_launches += 1;
+      conv1_tc_forward<TA>(h, x_dev, c.ci, ws.x8, c.w_fprop, out, c.co, B, crop, c.fold_scale, c.fold_shift, n.act, nullptr, true);
     } else if (l == 0) {
       launch_conv_simt<float, TA>(h, x_dev, n.channels, 0, n.channels, h->params + c.w_off, (TA*)out.p, out.cs, out.co, c.co,
                                   B, crop, c.k, c.rate, c.pad_b, c.fold_scale, c.fold_shift, n.act);
@@ -860,7 +903,11 @@ static void forward_eval_t(Handle* h, const float* x_dev, int B, int crop, float
       cur = out;
       xi = (xi + 1) % 3;
     }
-    h->taps[c.scope] = {n.dense ? out.p : cur.p, ElemTag<TA>::v, fs, n.dense ? c.out_coff : 0, c.co, M};
+    // a layer that writes a channel slice of a shared buffer (dense concat, the two expand convolutions of a squeeze module)
+    // is tapped at that slice; any other layer at its finished output, after the pool or gate
+    const ActBuf tap = (n.dense || sq_part >= 1) ? out : cur;
+    h->taps[c.scope] = {tap.p, ElemTag<TA>::v, fs, tap.co, c.co, M};
+    debug_keep<TA>(h, c.scope, (const TA*)tap.p, fs, tap.co, c.co, M);     // a later layer reuses this buffer
   }
   launch_classifier_fwd<TA>(h, (const TA*)cur.p, cur.cs, cur.co, n.cls_in, h->params + n.cls_w_off, h->params + n.cls_b_off, n.classes,
                             logits, pred_dev, M);
@@ -913,22 +960,6 @@ extern "C" int drs_forward_host(drs_handle_t h, const float* x_host, int32_t B, 
   int rc = drs_synchronize(h);
   if (rc) return rc;
   API_END
-}
-
-template <typename T>
-static void debug_keep(Handle* h, const std::string& name, const T* ptr, int cs, int co, int C, int64_t M) {
-  if (!h->debug_keep) return;
-  h->keep.emplace_back(M * C * 4);
-  float* buf = h->keep.back();
-  slice_to_f32_kernel<T><<<nblk(M * C, 256), 256, 0, h->stream>>>(ptr, cs, co, C, M, buf);
-  LAUNCH_CHECK(h);
-  h->taps[name] = {buf, ET_F32, C, 0, C, M};
-}
-static void debug_keep_reset(Handle* h) {
-  h->debug_keep = getenv("DRS_DEBUG_KEEP") != nullptr;
-  if (h->keep.empty()) return;
-  cudaStreamSynchronize(h->stream);
-  h->keep.clear();
 }
 
 #include "drs_train.cuh"

@@ -614,15 +614,21 @@ extern "C" int drs_debug_activation(drs_handle_t h, const char* name, float* out
 }
 
 // One convolution through the production path (unit tests): y = act(conv(x, w) * scale + shift).  16-bit precisions cast
-// the input and pack the filter as refresh_packed packs a layer's.
+// the input and pack the filter as refresh_packed packs a layer's; the conv1 shape (conv1_tc_supported) runs on conv1's
+// tensor-core kernel like the first layer of both forwards, any other shape on the generic one.
 template <typename T>
 static void debug_conv_tc(Handle* h, const float* x32, const float* w32, const float* sc, const float* sh, const ConvLayer& c, int B,
                           int crop, int act, T* xa, void* wp, T* ya, float* y32) {
   const int64_t M = (int64_t)B * crop * crop;
-  cast_kernel<float, T><<<nblk(M * c.ci, 256), 256, 0, h->stream>>>(x32, xa, M * c.ci);
-  LAUNCH_CHECK(h);
-  repack_filter(h, w32, wp, c.k * c.k, c.ci, c.co, 0, ElemTag<T>::v);
-  run_conv<T>(h, ActBuf{xa, c.ci, 0}, c.ci, w32, wp, ActBuf{ya, c.co, 0}, c.co, B, crop, c.k, c.rate, c.pad_b, sc, sh, act);
+  if (conv1_tc_supported(c.k, c.rate, c.ci, c.co)) {
+    pack_conv1<T>(h, w32, wp, c.ci, c.co);
+    conv1_tc_forward<T>(h, x32, c.ci, xa, wp, ActBuf{ya, c.co, 0}, c.co, B, crop, sc, sh, act, nullptr, true);
+  } else {
+    cast_kernel<float, T><<<nblk(M * c.ci, 256), 256, 0, h->stream>>>(x32, xa, M * c.ci);
+    LAUNCH_CHECK(h);
+    repack_filter(h, w32, wp, c.k * c.k, c.ci, c.co, 0, ElemTag<T>::v);
+    run_conv<T>(h, ActBuf{xa, c.ci, 0}, c.ci, w32, wp, ActBuf{ya, c.co, 0}, c.co, B, crop, c.k, c.rate, c.pad_b, sc, sh, act);
+  }
   cast_kernel<T, float><<<nblk(M * c.co, 256), 256, 0, h->stream>>>(ya, y32, M * c.co);
   LAUNCH_CHECK(h);
 }
@@ -645,8 +651,9 @@ extern "C" int drs_debug_conv(drs_handle_t h, const float* x_host, const float* 
   if (precision == DRS_PREC_FP32) {
     run_conv<float>(h, ActBuf{x32, Ci, 0}, Ci, w32, nullptr, ActBuf{y32, Co, 0}, Co, B, crop, k, rate, c.pad_b, sc, sh, act);
   } else {
-    xa = DevMem<void>(M * Ci * 2);
-    wp = DevMem<void>(nw * 2);
+    // (conv1's kernel reads the input padded to 8 channels and a filter of C1_SLOTS x Co x 8 elements)
+    xa = DevMem<void>(M * std::max(Ci, 8) * 2);
+    wp = DevMem<void>(std::max<int64_t>(nw, (int64_t)C1_SLOTS * Co * 8) * 2);
     ya = DevMem<void>(M * Co * 2);
     if (precision == DRS_PREC_F16) debug_conv_tc<__half>(h, x32, w32, sc, sh, c, B, crop, act, (__half*)xa.get(), wp, (__half*)ya.get(), y32);
     else debug_conv_tc<__nv_bfloat16>(h, x32, w32, sc, sh, c, B, crop, act, (__nv_bfloat16*)xa.get(), wp, (__nv_bfloat16*)ya.get(), y32);

@@ -368,12 +368,11 @@ static void train_step_t(Handle* h, const float* x_dev, const float* y_dev, cons
     if (l == 0 && ws.x8) {
       // conv1 on the tensor cores as in inference (conv1_tc.cuh): input and filter rounded to bf16 like every other layer's
       // operands; the filter is re-packed every step (13 K elements).  The filter gradient keeps the fp32 input.
-      c.w_fprop.grow((size_t)C1_SLOTS * c.co * 8 * 2, (size_t)C1_SLOTS * c.co * 8 * 2);
-      launch_pdl(h, pack_conv1_kernel<TA>, dim3(nblk(C1_SLOTS * c.co * 8, 256)), dim3(256), 0, h->params + c.w_off, (TA*)c.w_fprop.get(), c.ci, c.co);
-      LAUNCH_CHECK(h);
-      launch_pdl(h, pad_cast8_kernel<TA>, dim3(nblk(M, 256)), dim3(256), 0, x_dev, ws.x8, c.ci, M);
-      LAUNCH_CHECK(h);
-      if (ws.xcol) {
+      const size_t wbytes = (size_t)C1_SLOTS * c.co * 8 * 2;
+      c.w_fprop.grow(wbytes, wbytes);
+      pack_conv1<TA>(h, h->params + c.w_off, c.w_fprop, c.ci, c.co);
+      auto build_xcol = [&]() {
+        if (!ws.xcol) return;
         // the im2col matrix is only needed at the very end of the backward: built on the side stream, under the forward
         const bool side = !h->time_convs && !getenv("DRS_NO_OVERLAP");
         if (side) CUDA_CHECK(cudaEventRecord(h->ev_x8, h->stream));
@@ -381,12 +380,9 @@ static void train_step_t(Handle* h, const float* x_dev, const float* y_dev, cons
         if (side) CUDA_CHECK(cudaStreamWaitEvent(h->stream, h->ev_x8, 0));
         launch_pdl(h, im2col_conv1_kernel<TA>, dim3(nblk(M * 16, 256)), dim3(256), 0, ws.x8, ws.xcol, c.ci, crop, M);
         LAUNCH_CHECK(h);
-      }
-      Conv1TcArgs a1;
-      a1.x8 = ws.x8; a1.wpack = c.w_fprop; a1.out = ws.Z[l]; a1.out_cstride = c.co; a1.out_coff = 0; a1.co = c.co;
-      a1.B = B; a1.crop = crop; a1.scale = h->ones; a1.shift = h->params + c.b_off; a1.act = ACT_NONE; a1.etype = ElemTag<TA>::v;
-      a1.stats = fused_stats ? &fin : nullptr;
-      launch_conv1_tc(h, a1);
+      };
+      conv1_tc_forward<TA>(h, x_dev, c.ci, ws.x8, c.w_fprop, ActBuf{ws.Z[l], c.co, 0}, c.co, B, crop, h->ones, h->params + c.b_off,
+                           ACT_NONE, fused_stats ? &fin : nullptr, false, build_xcol);
     } else if (l == 0) {
       launch_conv_simt<float, TA>(h, x_dev, n.channels, 0, n.channels, h->params + c.w_off, ws.Z[l], c.co, 0, c.co, B, crop, c.k,
                                   c.rate, c.pad_b, h->ones, h->params + c.b_off, ACT_NONE);
@@ -394,7 +390,9 @@ static void train_step_t(Handle* h, const float* x_dev, const float* y_dev, cons
       run_conv<TA>(h, input_of(l), c.ci, h->params + c.w_off, c.w_fprop, ActBuf{ws.Z[l], c.co, 0}, c.co, B, crop, c.k, c.rate, c.pad_b,
                    h->ones, h->params + c.b_off, ACT_NONE, fused_stats ? &fin : nullptr);
     }
+    debug_keep<TA>(h, "z:" + c.scope, ws.Z[l], c.co, 0, c.co, M);
     forward_normalise(h, q, fused_stats);
+    // the layer outputs need no copy: the backward reads them but writes only T, the dZ buffers and the gradient buffers
     h->taps[c.scope] = {q.out.p, ElemTag<TA>::v, q.out.cs, q.out.co, c.co, M};
   }
   ActBuf feat = n.dense ? ActBuf{ws.F, n.feat_stride, 0}

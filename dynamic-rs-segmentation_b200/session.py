@@ -23,7 +23,9 @@ from . import nets
 class Session:
     def __init__(self, net_type, channels, num_classes, weight_decay=0.005, lr_initial=0.01, decay_steps=50000,
                  decay_rate=0.5, momentum=0.9, precision="bf16", device=0, isprs_scopes=True, bn_unbiased_ema=True,
-                 seed=None):
+                 seed=None, bn_decay=0.999):
+        """bn_decay: decay of the BN moving averages (tf.contrib.layers.batch_norm's 0.999 by default); 0 makes the moving
+        statistics after a step that step's batch statistics."""
         if net_type not in L.NET_TYPES:
             # same message the reference prints before returning (isprs:1679)
             raise ValueError("Error! Net type not identified: " + str(net_type))
@@ -32,7 +34,7 @@ class Session:
         self.precision = precision
         self.isprs_scopes = bool(isprs_scopes)
         cfg = L.Config(L.NET_TYPES[net_type], channels, num_classes, L.PREC[precision], weight_decay, lr_initial,
-                       decay_steps, decay_rate, momentum, 0.999, 0.001, int(bool(bn_unbiased_ema)), device,
+                       decay_steps, decay_rate, momentum, float(bn_decay), 0.001, int(bool(bn_unbiased_ema)), device,
                        int(self.isprs_scopes))
         self._h = C.c_void_p()
         L.check(self._lib.drs_create(C.byref(self._h), C.byref(cfg)))

@@ -330,7 +330,9 @@ int drs_profile_read(drs_handle_t h, float* conv_ms, int64_t* conv_launches, dou
 int drs_last_conv_ms(drs_handle_t h, float* ms_out);
 /* debug: copy the activation of conv scope `name` from the last forward (post act/pool) as fp32 NHWC */
 int drs_debug_activation(drs_handle_t h, const char* name, float* out_host, int64_t count);
-/* unit-test entry: one dilated SAME convolution through the tcgen05 path (or SIMT when precision=FP32).
+/* unit-test entry: one dilated SAME convolution through the tcgen05 path (or SIMT when precision=FP32).  In F16 / BF16
+ * the conv1 shape (5x5, rate 1, Ci <= 8, Co 32 or 64) runs on conv1's tensor-core kernel, as the first layer of both
+ * forwards does; every other shape on the generic tcgen05 kernel.
  *   x [B,crop,crop,Ci] fp32 host, w HWIO fp32 host, scale/shift [Co] (y = act(conv*scale+shift)), act 0/1/2 */
 int drs_debug_conv(drs_handle_t h, const float* x_host, const float* w_host, const float* scale_host,
                    const float* shift_host, int32_t B, int32_t crop, int32_t k, int32_t rate, int32_t Ci, int32_t Co,
