@@ -373,7 +373,7 @@ struct drs_handle_s {
   PinnedMem<float> result_host;     // [RESULT_RING][RESULT_STRIDE]
   Event result_ev[RESULT_RING];
   int64_t next_ticket = 0;
-  // DRS_DEBUG_KEEP=1: fp32 copies of backward intermediates ("dz:<scope>", "da:<scope>")
+  // DRS_DEBUG_KEEP=1: fp32 copies of training-step tensors whose buffers are reused ("z:", "dout:", "da:", "dz:<scope>")
   std::vector<DevMem<float>> keep;
   bool debug_keep = false;
 };

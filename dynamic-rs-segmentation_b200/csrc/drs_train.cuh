@@ -185,11 +185,11 @@ static void forward_normalise(Handle* h, const NormLayer<TA>& q, bool stats_fuse
 
 // Pooling layers in bf16 take the backward in two passes instead of four: the BN-backward sums on the pooled side (window
 // gradients and pooled activations: bn_partial_kernel MODE 2), then ONE kernel scatters the window gradients to their
-// winners and applies the BN backward to the finished fp32 row; the pool's input gradient is never stored.  (DRS_DEBUG_KEEP
-// wants that gradient, so it takes the separate kernels.)
+// winners and applies the BN backward to the finished fp32 row; the pool's input gradient is never stored, so DRS_DEBUG_KEEP
+// records no "da:" tap for these layers.
 template <typename TA>
-static bool fused_pool_bn_backward(const Handle* h, const NormLayer<TA>& q) {
-  return q.pool && q.post == 0 && ElemTag<TA>::v == ET_BF16 && q.co <= 512 && pool_lean_enabled() && !h->debug_keep &&
+static bool fused_pool_bn_backward(const NormLayer<TA>& q) {
+  return q.pool && q.post == 0 && ElemTag<TA>::v == ET_BF16 && q.co <= 512 && pool_lean_enabled() &&
          !getenv("DRS_NO_FUSED_POOL_APPLY");
 }
 
@@ -206,7 +206,7 @@ static ActBuf backward_to_dz(Handle* h, const NormLayer<TA>& q, const ActBuf& dO
     CUDA_CHECK(cudaStreamWaitEvent(h->stream, wgrad_done, 0));
     h->pdl_prev = false;                 // the next kernel also depends on another stream
   };
-  if (fused_pool_bn_backward(h, q)) {
+  if (fused_pool_bn_backward(q)) {
     launch_pdl(h, bn_partial_kernel<TA, TA, 2>, dim3(nb), dim3(BN_THREADS), 0, (const TA*)q.out.p, q.co, 0, (const TA*)dOut.p, dOut.cs,
                dOut.co, (const float*)q.mean, (const float*)q.istd, q.act, q.part_bn, q.co, M, rows, finb);
     LAUNCH_CHECK(h);
@@ -394,6 +394,8 @@ static void train_step_t(Handle* h, const float* x_dev, const float* y_dev, cons
     forward_normalise(h, q, fused_stats);
     // the layer outputs need no copy: the backward reads them but writes only T, the dZ buffers and the gradient buffers
     h->taps[c.scope] = {q.out.p, ElemTag<TA>::v, q.out.cs, q.out.co, c.co, M};
+    // nor does the activation in front of an average pool or SE gate
+    if (h->debug_keep && c.post) h->taps["pre:" + c.scope] = {ws.Apre[l], ElemTag<TA>::v, c.co, 0, c.co, M};
   }
   ActBuf feat = n.dense ? ActBuf{ws.F, n.feat_stride, 0}
                         : ActBuf{ws.Xn[L - 1], n.convs[L - 1].out_cs > 0 ? n.convs[L - 1].out_cs : n.convs[L - 1].co, 0};
@@ -419,6 +421,10 @@ static void train_step_t(Handle* h, const float* x_dev, const float* y_dev, cons
   LAUNCH_CHECK(h);
   launch_pdl(h, sum_fixed_kernel, dim3(1), dim3(256), 0, ws.part_ce, ws.nb_ce, h->loss_dev, 1.0f, h->loss_dev + 3);
   LAUNCH_CHECK(h);
+  if (h->debug_keep) {                 // neither is written again in the step
+    h->taps["logits"] = {ws.logits, ET_F32, K, 0, K, M};
+    h->taps["dlogits"] = {ws.dlogits, ET_F32, K, 0, K, M};
+  }
   // fused calc_accuracy_by_crop (isprs:510-531)
   CUDA_CHECK(cudaMemsetAsync(h->cm_dev, 0, (K * K + 1) * 4, h->stream));
   h->pdl_prev = false;
@@ -475,6 +481,8 @@ static void train_step_t(Handle* h, const float* x_dev, const float* y_dev, cons
     // overlaps the HBM-bound kernels of layer l-1's backward.  dZ is double-buffered; before a buffer is rewritten the
     // main stream waits for the wgrad that read it two layers ago.
     TA* DZ = ws.DZb[l & 1];
+    // (a copy: Gcur / GF / Gg are rewritten later in the step)
+    debug_keep<TA>(h, "dout:" + c.scope, (const TA*)dOut.p, dOut.cs, dOut.co, c.co, M);
     const ActBuf dA = backward_to_dz(h, norm_layer(l), dOut, ws.T, DZ, l + 2 <= L - 1 ? h->ev_wgrad[l & 1].get() : nullptr);
     if (dA.p) debug_keep<TA>(h, "da:" + c.scope, (const TA*)dA.p, dA.cs, dA.co, c.co, M);
     debug_keep<TA>(h, "dz:" + c.scope, DZ, c.co, 0, c.co, M);

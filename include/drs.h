@@ -328,7 +328,10 @@ int64_t drs_launch_count(drs_handle_t h);
 int drs_set_profiling(drs_handle_t h, int32_t on);
 int drs_profile_read(drs_handle_t h, float* conv_ms, int64_t* conv_launches, double* conv_flops);
 int drs_last_conv_ms(drs_handle_t h, float* ms_out);
-/* debug: copy the activation of conv scope `name` from the last forward (post act/pool) as fp32 NHWC */
+/* debug: copy the activation of conv scope `name` from the last forward (post act/pool) as fp32 NHWC.  After a training step
+ * under DRS_DEBUG_KEEP=1 also "z:<scope>" (raw conv output), "pre:<scope>" (activation in front of an average pool or SE
+ * gate), "logits", "dlogits", "dout:<scope>" (gradient of the layer output), "da:<scope>" (gradient in front of the BN
+ * backward; not for the fused bf16 pool + BN backward, which never stores it) and "dz:<scope>". */
 int drs_debug_activation(drs_handle_t h, const char* name, float* out_host, int64_t count);
 /* unit-test entry: one dilated SAME convolution through the tcgen05 path (or SIMT when precision=FP32).  In F16 / BF16
  * the conv1 shape (5x5, rate 1, Ci <= 8, Co 32 or 64) runs on conv1's tensor-core kernel, as the first layer of both

@@ -992,11 +992,13 @@ def _step_fingerprints(env, net="dilated_grsl", crops="13,25", steps=3):
 
 
 def test_launch_modes_do_not_change_a_bit():
-    """Programmatic dependent launch, CUDA graphs and the side-stream overlap only move kernels in time: the variables after
-    three steps are bit-identical with each of them switched off.  (Environment switches read once per process -> subprocesses.)"""
+    """Programmatic dependent launch, CUDA graphs and the side-stream overlap only move kernels in time, and the debug copies
+    of DRS_DEBUG_KEEP only read: the variables after three steps are bit-identical with each of them switched off (or the
+    copies on).  (Environment switches read once per process -> subprocesses.)"""
     ref = _step_fingerprints({})
     assert len(ref) == 2
-    for env in ({"DRS_NO_PDL": "1"}, {"DRS_GRAPHS": "0"}, {"DRS_NO_OVERLAP": "1"}, {"DRS_NO_PDL": "1", "DRS_GRAPHS": "0"}):
+    for env in ({"DRS_NO_PDL": "1"}, {"DRS_GRAPHS": "0"}, {"DRS_NO_OVERLAP": "1"}, {"DRS_NO_PDL": "1", "DRS_GRAPHS": "0"},
+                {"DRS_DEBUG_KEEP": "1"}):
         assert _step_fingerprints(env) == ref, env
 
 
