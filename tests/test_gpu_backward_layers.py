@@ -52,9 +52,10 @@ SLOPE = {0: 1.0, 1: 0.0, 2: 0.1}                                 # act'(x) for x
 
 
 # ------------------------------------------------------------------------------------------------ float64 references
-def ce_ref(lg, y, on):
+def ce_ref(lg, y, on, count=None):
     """Mean softmax cross entropy over the pixels `on` (labels outside [0, K) add no loss) and its gradient; also the per-pixel
-    bound of the loss term and of the fp32 lse (every operation one ulp, expf two)."""
+    bound of the loss term and of the fp32 lse (every operation one ulp, expf two).  count: the pixels of the mean (None: the
+    pixels `on`; data parallel: those of every rank)."""
     lg = lg.astype(np.float64)
     M, K = lg.shape
     yi = y.astype(np.int64)
@@ -64,7 +65,7 @@ def ce_ref(lg, y, on):
     p = np.exp(lg - lse)
     onehot = (np.arange(K)[None, :] == yi[:, None]).astype(np.float64)
     valid = on & (yi >= 0) & (yi < K)
-    count = float(on.sum())
+    count = float(on.sum()) if count is None else float(count)
     loss_px = np.where(valid, lse[:, 0] - lg[np.arange(M), np.clip(yi, 0, K - 1)], 0.0)
     dl = np.where(on[:, None], (p - onehot) / max(count, 1.0), 0.0)
     dlse = ULP * (2 + K + np.abs(lg - mx).max(1, keepdims=True) + 2 * np.abs(np.log(se)) + np.abs(lse))
@@ -247,6 +248,16 @@ def cls_wgrad_depth(M, ci, sm):
     return ceil(ceil(M / nb) / lanes) + lanes + nb
 
 
+def rank_sum(parts):
+    """Sum over ranks of per-rank (reference, bound) pairs, plus the exchange: one fixed-order fp32 sum of W terms,
+    gamma(W - 1) sum_r |v_r| with |v_r| <= |ref_r| + bound_r (nothing for one rank)."""
+    ref = sum(p[0] for p in parts)
+    bound = sum(p[1] for p in parts)
+    if len(parts) > 1:
+        bound = bound + gamma(len(parts) - 1) * sum(np.abs(p[0]) + p[1] for p in parts)
+    return ref, bound
+
+
 def wgrad_tc_supported(ci, co):
     return (ci % 64 == 0 or ci == 32) and (co % 64 == 0 or co == 32) and co <= 256
 
@@ -287,22 +298,26 @@ class TrainRun:
     """One train_step (bn_decay = 0, DRS_DEBUG_KEEP=1) and every tap and gradient the checks read."""
 
     def __init__(self, drs, monkeypatch, net, C, K, prec, B, crop, use_mask=False, ignore=False, env=(), seed=5, x=None,
-                 session_kw=None):
+                 session_kw=None, y=None, mask=None, step=True):
+        """x, y, mask: the feeds (None: drawn from the seed); step=False: create the session only (a data-parallel rank:
+        its exchange is attached, then train() and collect() run)."""
         from oracle import nets_torch
         monkeypatch.setenv("DRS_DEBUG_KEEP", "1")
         for k in env:
             monkeypatch.setenv(k, "1")
+        self.drs = drs
         self.layers, self.cls_inputs, self.act = net_layers(net, C)
         self.net, self.C, self.K, self.prec, self.B, self.crop = net, C, K, prec, B, crop
-        self.M = M = B * crop * crop
+        self.M = B * crop * crop
         self.p = p = nets_torch.init_params(net, C, K, seed=seed)
         rs = np.random.RandomState(seed + 1)
         self.x = rs.randn(B, crop * crop * C).astype(np.float32) if x is None else x
-        y = rs.randint(0, K, size=(B, crop * crop)).astype(np.float32)
-        if ignore:                                       # about 20 % of the labels are the ignored label K
-            y = np.where(rs.rand(B, crop * crop) < 0.2, K, y).astype(np.float32)
-        self.y, self.ignore = y, ignore
-        self.mask = (rs.rand(B, crop * crop) > 0.3) if use_mask else None
+        if y is None:
+            y = rs.randint(0, K, size=(B, crop * crop)).astype(np.float32)
+            if ignore:                                   # about 20 % of the labels are the ignored label K
+                y = np.where(rs.rand(B, crop * crop) < 0.2, K, y).astype(np.float32)
+            mask = (rs.rand(B, crop * crop) > 0.3) if use_mask else None
+        self.y, self.ignore, self.mask = y, ignore, mask
         kw = dict(precision=prec, bn_decay=0.0, weight_decay=0.0)
         kw.update(session_kw or {})
         s = drs.Session(net, C, K, **kw)
@@ -310,26 +325,45 @@ class TrainRun:
         if ignore:
             s.set_ignore_label(K)
         self.s = s
-        self.loss = float(s.train_step(self.x, y, crop, mask=self.mask)[0])
+        import torch
+        self.sm = torch.cuda.get_device_properties(0).multi_processor_count
+        if step:
+            self.train()
+            self.collect()
+
+    def train(self):
+        """The training step: loss, pred and the confusion counts it returns."""
+        loss, self.pred, self.cm, self.n_correct = self.s.train_step(self.x, self.y, self.crop, mask=self.mask, want_cm=True)
+        self.loss = float(loss)
+
+    def collect(self, bn_count=None):
+        """Every tap and gradient the checks read.  bn_count: the pixels behind the batch statistics (None: this run's M;
+        SyncBN: those of every rank), which the inverse std recovered from the unbiased moving variance needs."""
+        s, B, crop, K, M = self.s, self.B, self.crop, self.K, self.M
+        n = M if bn_count is None else bn_count
         self.taps = {}
         for L in self.layers:
             sc, co = L["scope"], L["co"]
             for t in ("z:", "", "dout:", "dz:", "da:", "pre:"):
                 try:
                     self.taps[t + sc] = s.debug_activation(t + sc, B, crop, co)
-                except drs.lib.DrsError:
+                except self.drs.lib.DrsError:
                     assert t in ("da:", "pre:"), (t, sc)
         self.logits = s.debug_activation("logits", B, crop, K).reshape(M, K)
         self.dlogits = s.debug_activation("dlogits", B, crop, K).reshape(M, K)
         self.mean = {L["scope"]: s.get_variable(L["scope"] + "/moving_mean").astype(np.float64) for L in self.layers}
-        self.istd = {L["scope"]: 1.0 / np.sqrt(s.get_variable(L["scope"] + "/moving_variance").astype(np.float64) * (M - 1) / M + EPS)
+        self.istd = {L["scope"]: 1.0 / np.sqrt(s.get_variable(L["scope"] + "/moving_variance").astype(np.float64) * (n - 1) / n + EPS)
                      for L in self.layers}
         self.grad = {n: s.get_gradient(n) for n, _ in s.variable_names() if n.endswith(("/weights", "/biases")) and "/Momentum" not in n}
-        import torch
-        self.sm = torch.cuda.get_device_properties(0).multi_processor_count
 
     def close(self):
         self.s.close()
+
+    def loss_on(self):
+        """The pixels in the mean of the loss: the mask, else every label but the ignored one."""
+        if self.mask is not None:
+            return self.mask.reshape(-1)
+        return self.y.reshape(-1).astype(np.int64) != (self.K if self.ignore else -1)
 
     def w(self, scope):
         return rounded(np.asarray(self.p[scope + "/weights"], np.float32), self.prec).astype(np.float64)
@@ -345,47 +379,70 @@ class TrainRun:
     def check(self, tag, idx=None, wcols=None, mut=None):
         """{quantity: largest err / bound} over every stage of the backward; idx: pixels of the data-gradient check (None:
         all), wcols: output-channel subset of the filter-gradient check (None: all)."""
-        mut = mut or {}
-        B, crop, K, M, prec = self.B, self.crop, self.K, self.M, self.prec
-        u = U[prec]
-        res = {}
+        return check_step([self], tag, idx, wcols, mut)
 
-        def rec(name, got, ref, bound):
-            res[name] = ratio((tag, prec, name), got, ref, bound)
+    def part_cap(self):
+        """Floats of the filter gradients' split partials (TrainWs::layout): the largest filter x 48."""
+        return max(L["k"] ** 2 * L["ci"] * L["co"] for L in self.layers) * 48
 
-        by_scope = {L["scope"]: (j, L) for j, L in enumerate(self.layers)}
-        # ---- loss and dlogits
-        if self.mask is not None:
-            on = self.mask.reshape(-1)
-        else:
-            on = self.y.reshape(-1).astype(np.int64) != (K if self.ignore else -1)
-        ce = ce_ref(self.logits, self.y.reshape(-1), on)
-        cnt = max(ce["count"], 1.0)
-        d = (ce["p"] * (2 * ULP + ULP * np.abs(self.logits - ce["lse"]) + ce["dlse"]) + ULP * np.abs(ce["p"] - ce["onehot"])) / cnt
-        rec("dlogits", self.dlogits, ce["dl"], np.where(on[:, None], d + 2 * ULP * np.abs(ce["dl"]), 0.0) + TINY)
+
+def check_step(runs, tag, idx=None, wcols=None, mut=None, sync_bn=False):
+    """{quantity: largest err / bound over the ranks} over every stage of the backward of one step.  runs: the ranks of a
+    data-parallel step, each with its own batch and taps (one run: the single-process step).  The per-pixel stages (dlogits,
+    dout, routing, dz) are checked per rank from its own taps; the global quantities come from every rank: the loss count,
+    the BN-backward sums with SyncBN (sync_bn), and the loss and parameter gradients (sums over ranks, rank_sum)."""
+    mut = mut or {}
+    r0 = runs[0]
+    W = len(runs)
+    B, crop, K, M, prec = r0.B, r0.crop, r0.K, r0.M, r0.prec
+    u = U[prec]
+    res = {}
+
+    def rec(name, got, ref, bound):
+        res[name] = max(res.get(name, 0.0), ratio((tag, prec, name), got, ref, bound))
+
+    by_scope = {L["scope"]: (j, L) for j, L in enumerate(r0.layers)}
+    # ---- loss and dlogits: every rank divides by the pixel count of all ranks
+    ons = [r.loss_on() for r in runs]
+    total = float(sum(on.sum() for on in ons))
+    parts = []
+    for r, on in zip(runs, ons):
+        count = float(on.sum()) if mut.get("local_count") else (float(r.M) if mut.get("count_is_m") else total)
+        ce = ce_ref(r.logits, r.y.reshape(-1), on, count)
+        cnt = max(count, 1.0)
+        d = (ce["p"] * (2 * ULP + ULP * np.abs(r.logits - ce["lse"]) + ce["dlse"]) + ULP * np.abs(ce["p"] - ce["onehot"])) / cnt
+        rec("dlogits", r.dlogits, ce["dl"], np.where(on[:, None], d + 2 * ULP * np.abs(ce["dl"]), 0.0) + TINY)
         lb = ((ce["dlse"][:, 0] + ULP * ce["loss_px"]) * ce["valid"]).sum() / cnt + 8 * ULP * ce["loss_px"].sum() / cnt + 3 * ULP * abs(ce["loss"])
-        rec("loss", np.array([self.loss]), np.array([ce["loss"]]), np.array([lb + TINY]))
-        dl = self.dlogits.astype(np.float64)
-        # ---- classifier filter gradient (fp32 weights as stored)
-        xc = np.concatenate([self.taps[n].reshape(M, -1) for n in self.cls_inputs], 1).astype(np.float64)
-        h = cls_wgrad_depth(M, xc.shape[1], self.sm)
-        rec("classifier dW", self.grad["conv_classifier/weights"].reshape(-1, K), xc.T @ dl, gamma(h) * (np.abs(xc).T @ np.abs(dl)) + TINY)
-        rec("classifier db", self.grad["conv_classifier/biases"], dl.sum(0), gamma(h) * np.abs(dl).sum(0) + TINY)
-        # ---- data gradients: dout:<l> from the classifier and every consumer, in step order
-        idx_all = np.arange(M) if idx is None else idx
-        wc = np.asarray(self.p["conv_classifier/weights"], np.float64).reshape(-1, K)
-        consumers = {L["scope"]: [] for L in self.layers}
-        off = 0
-        for n in self.cls_inputs:
-            consumers[n].append(("classifier", off))
-            off += by_scope[n][1]["co"]
-        for j in range(len(self.layers) - 1, -1, -1):
-            Lj, off = self.layers[j], 0
-            for n in Lj["inputs"]:
-                if n != "x":
-                    consumers[n].append((j, off))
-                    off += by_scope[n][1]["co"]
-        for L in self.layers:
+        parts.append((ce["loss"], lb))
+    loss, lb = rank_sum(parts)
+    for r in runs:
+        rec("loss", np.array([r.loss]), np.array([loss]), np.array([lb + TINY]))
+    dls = [r.dlogits.astype(np.float64) for r in runs]
+    # ---- classifier filter gradient (fp32 weights as stored)
+    xcs = [np.concatenate([r.taps[n].reshape(M, -1) for n in r.cls_inputs], 1).astype(np.float64) for r in runs]
+    h = cls_wgrad_depth(M, xcs[0].shape[1], r0.sm)
+    v, b = rank_sum([(xc.T @ dl, gamma(h) * (np.abs(xc).T @ np.abs(dl))) for xc, dl in zip(xcs, dls)])
+    for r in runs:
+        rec("classifier dW", r.grad["conv_classifier/weights"].reshape(-1, K), v, b + TINY)
+    v, b = rank_sum([(dl.sum(0), gamma(h) * np.abs(dl).sum(0)) for dl in dls])
+    for r in runs:
+        rec("classifier db", r.grad["conv_classifier/biases"], v, b + TINY)
+    # ---- data gradients: dout:<l> from the classifier and every consumer, in step order (per rank)
+    idx_all = np.arange(M) if idx is None else idx
+    wc = np.asarray(r0.p["conv_classifier/weights"], np.float64).reshape(-1, K)
+    consumers = {L["scope"]: [] for L in r0.layers}
+    off = 0
+    for n in r0.cls_inputs:
+        consumers[n].append(("classifier", off))
+        off += by_scope[n][1]["co"]
+    for j in range(len(r0.layers) - 1, -1, -1):
+        Lj, off = r0.layers[j], 0
+        for n in Lj["inputs"]:
+            if n != "x":
+                consumers[n].append((j, off))
+                off += by_scope[n][1]["co"]
+    for r, dl in zip(runs, dls):
+        for L in r0.layers:
             sc, co = L["scope"], L["co"]
             S, Bd = None, None
             for ci, (j, o) in enumerate(consumers[sc]):
@@ -395,8 +452,8 @@ class TrainRun:
                     c = dl[idx_all] @ wc[o:o + co].T
                     cb = gamma(K) * (np.abs(dl[idx_all]) @ np.abs(wc[o:o + co]).T)
                 else:
-                    Lj = self.layers[j]
-                    v, sab = dgrad_at(self.taps["dz:" + Lj["scope"]], self.w(Lj["scope"]), Lj["rate"], idx_all, crop,
+                    Lj = r0.layers[j]
+                    v, sab = dgrad_at(r.taps["dz:" + Lj["scope"]], r0.w(Lj["scope"]), Lj["rate"], idx_all, crop,
                                       swap=mut.get("unswapped_pads") != Lj["scope"])
                     c, cb = v[:, o:o + co], gamma(Lj["k"] ** 2 * Lj["co"]) * sab[:, o:o + co]
                 cb = u * np.abs(c) + (1 + u) * cb                   # its own rounding (direct write or the add_slice scratch)
@@ -405,77 +462,98 @@ class TrainRun:
                 else:
                     S = S + c
                     Bd = Bd + cb + u * (np.abs(S) + Bd + cb)      # the add_slice rounding
-            rec("dout " + sc, self.taps["dout:" + sc].reshape(M, co)[idx_all], S, Bd + TINY)
-        # ---- per layer: post-op backward, BN backward, filter gradient
-        for L in self.layers:
-            sc, co, post = L["scope"], L["co"], L["post"]
-            Z = self.taps["z:" + sc]
-            G = self.taps["dout:" + sc]
-            mean, istd = self.mean[sc], self.istd[sc]
+            rec("dout " + sc, r.taps["dout:" + sc].reshape(M, co)[idx_all], S, Bd + TINY)
+    # ---- per layer: post-op backward (per rank), BN backward (its sums over every rank with SyncBN), filter gradient
+    Mbn = M * W if sync_bn else M
+    exh = 4 * E24
+    for L in r0.layers:
+        sc, co, post = L["scope"], L["co"], L["post"]
+        per, se_parts = [], {}
+        for r in runs:
+            Z = r.taps["z:" + sc]
+            G = r.taps["dout:" + sc]
+            mean, istd = r.mean[sc], r.istd[sc]
             eg = np.zeros((M, co))
             fused = None
             if post is None:
-                gin = self.taps["da:" + sc].reshape(M, co).astype(np.float64)
-                assert np.array_equal(self.taps["da:" + sc], G), sc       # no post-op: the BN reads dout itself
+                gin = r.taps["da:" + sc].reshape(M, co).astype(np.float64)
+                assert np.array_equal(r.taps["da:" + sc], G), sc       # no post-op: the BN reads dout itself
             elif post[0] == "max":
                 ref, sab, _, zmax = pool_route(Z, G, last=mut.get("last_tie", False))
-                if "da:" + sc in self.taps:
-                    rec("pool " + sc, self.taps["da:" + sc], ref, u * np.abs(ref) + (1 + u) * gamma(9) * sab + TINY)
-                    gin = self.taps["da:" + sc].reshape(M, co).astype(np.float64)
+                if "da:" + sc in r.taps:
+                    rec("pool " + sc, r.taps["da:" + sc], ref, u * np.abs(ref) + (1 + u) * gamma(9) * sab + TINY)
+                    gin = r.taps["da:" + sc].reshape(M, co).astype(np.float64)
                 else:                                          # fused pool + BN backward: the routed sum in fp32
                     assert prec == "bf16" and not mut.get("last_tie"), sc
                     gin, eg = ref.reshape(M, co), gamma(9) * sab.reshape(M, co)
                     zw = zmax.reshape(M, co).astype(np.float64)
-                    f = np.where(zw > mean, 1.0, SLOPE[self.act])
+                    f = np.where(zw > mean, 1.0, SLOPE[r.act])
                     t0 = np.abs(G.reshape(M, co) * f)
                     fused = (t0.sum(0), (t0 * np.abs(zw - mean) * istd).sum(0))
             elif post[0] == "avg":
                 ref, sab = avg_route(G, post[1], by_receiver=mut.get("avg_by_receiver", False))
-                rec("avgpool " + sc, self.taps["da:" + sc], ref, u * np.abs(ref) + (1 + u) * (gamma(post[1] ** 2) + E24) * sab + TINY)
-                gin = self.taps["da:" + sc].reshape(M, co).astype(np.float64)
+                rec("avgpool " + sc, r.taps["da:" + sc], ref, u * np.abs(ref) + (1 + u) * (gamma(post[1] ** 2) + E24) * sab + TINY)
+                gin = r.taps["da:" + sc].reshape(M, co).astype(np.float64)
             else:
                 px = crop * crop
-                A = self.taps["pre:" + sc].reshape(B, px, co).astype(np.float64)
-                out = se_backward(A, G.reshape(B, px, co).astype(np.float64), self.p, post[2], px)
+                A = r.taps["pre:" + sc].reshape(B, px, co).astype(np.float64)
+                out = se_backward(A, G.reshape(B, px, co).astype(np.float64), r.p, post[2], px)
                 v, e = out.pop("da")
-                rec("se da " + sc, self.taps["da:" + sc].reshape(B, px, co), v, u * np.abs(v) + (1 + u) * e + TINY)
-                for q, (v, e) in out.items():
-                    rec("se %s %s" % (q, sc), self.grad[post[2] + "_" + q].reshape(v.shape), v, e + TINY)
-                gin = self.taps["da:" + sc].reshape(M, co).astype(np.float64)
-            # BN backward
+                rec("se da " + sc, r.taps["da:" + sc].reshape(B, px, co), v, u * np.abs(v) + (1 + u) * e + TINY)
+                for q, ve in out.items():
+                    se_parts.setdefault(q, []).append(ve)
+                gin = r.taps["da:" + sc].reshape(M, co).astype(np.float64)
+            # BN-backward sums of this rank: S0 = sum g, S1 = sum g xh
             Zr = Z.reshape(M, co)
-            xh, g, m0, m1 = bn_backward(Zr, gin, mean, istd, self.act)
-            neg = (Zr <= mean) & (self.act == 2)
-            eg = eg * np.where(Zr > mean, 1.0, SLOPE[self.act]) + np.where(neg, 2 * E24 * np.abs(g), 0.0)
-            h, nb = bn_depth(M, co, self.sm)
+            xh, g, _, _ = bn_backward(Zr, gin, mean, istd, r.act)
+            neg = (Zr <= mean) & (r.act == 2)
+            eg = eg * np.where(Zr > mean, 1.0, SLOPE[r.act]) + np.where(neg, 2 * E24 * np.abs(g), 0.0)
+            h, nb = bn_depth(M, co, r0.sm)
             A0, A1 = (np.abs(g).sum(0), np.abs(g * xh).sum(0)) if fused is None else fused
-            exh = 4 * E24
-            dS0 = (gamma(h) + 2 * E24) * A0 + nb * 2.0 ** -40 + E24 * np.abs(m0 * M)
-            dS1 = (gamma(h) + 2 * E24 + exh + (u + 4 * E24 if fused is not None else 0.0)) * A1 + nb * 2.0 ** -40 + E24 * np.abs(m1 * M)
-            dm0, dm1 = dS0 / M + E24 * np.abs(m0), dS1 / M + E24 * np.abs(m1)
+            S0, S1 = g.sum(0), (g * xh).sum(0)
+            dS0 = (gamma(h) + 2 * E24) * A0 + nb * 2.0 ** -40 + E24 * np.abs(S0)
+            dS1 = (gamma(h) + 2 * E24 + exh + (u + 4 * E24 if fused is not None else 0.0)) * A1 + nb * 2.0 ** -40 + E24 * np.abs(S1)
+            per.append(dict(xh=xh, g=g, eg=eg, istd=istd, s0=(S0, dS0), s1=(S1, dS1)))
+        for q, parts in se_parts.items():
+            v, e = rank_sum(parts)
+            for r in runs:
+                rec("se %s %s" % (q, sc), r.grad[post[2] + "_" + q].reshape(v.shape), v, e + TINY)
+        if sync_bn and not mut.get("bn_sums_one_rank"):          # the all-reduced sums
+            s0, s1 = rank_sum([q["s0"] for q in per]), rank_sum([q["s1"] for q in per])
+            for q in per:
+                q["s0"], q["s1"] = s0, s1
+        # BN backward dZ = istd (g - m0 - xh m1), m0 / m1 the sums over the pixels behind the statistics
+        for r, q in zip(runs, per):
+            xh, g, eg, istd = q["xh"], q["g"], q["eg"], q["istd"]
+            (S0, dS0), (S1, dS1) = q["s0"], q["s1"]
+            m0, m1 = S0 / Mbn, S1 / Mbn
+            dm0, dm1 = dS0 / Mbn + E24 * np.abs(m0), dS1 / Mbn + E24 * np.abs(m1)
             ref = istd * (g - m0 - (0.0 if mut.get("bn_drop_s1") else xh * m1))
             err = istd * (eg + dm0 + np.abs(xh) * dm1 + exh * np.abs(xh) * np.abs(m1) + 3 * E24 * (np.abs(g) + np.abs(m0) + np.abs(xh * m1)))
             err = err + 2 * E24 * np.abs(ref)
-            rec("dz " + sc, self.taps["dz:" + sc].reshape(M, co), ref, u * np.abs(ref) + (1 + u) * err + TINY)
-            # filter gradient and the (absent) bias gradient
-            cols = np.arange(co) if wcols is None else wcols(co)
-            v, sab = wgrad_ref(self.wgrad_inputs(L), self.taps["dz:" + sc], L["k"], L["rate"], cols)
+            rec("dz " + sc, r.taps["dz:" + sc].reshape(M, co), ref, u * np.abs(ref) + (1 + u) * err + TINY)
+        # filter gradient (summed over ranks) and the (absent) bias gradient
+        cols = np.arange(co) if wcols is None else wcols(co)
+        if L["inputs"] == ["x"]:
+            tc = conv1_uses_im2col(L, prec)
+            depth = wgrad_tc_depth(M, 1, 128, co, r0.sm, r0.part_cap()) if tc else 2 * M
+        else:
+            tc = prec == "bf16" and wgrad_tc_supported(L["ci"], co)
+            depth = wgrad_tc_depth(M, L["k"], L["ci"], co, r0.sm, r0.part_cap()) if tc else 2 * M
+        parts = []
+        for i, r in enumerate(runs):
+            if mut.get("drop_rank_share") == sc and i == W - 1:
+                continue
+            v, sab = wgrad_ref(r.wgrad_inputs(L), r.taps["dz:" + sc], L["k"], L["rate"], cols)
             if mut.get("transpose_taps"):
                 v = v.transpose(1, 0, 2, 3)
-            if L["inputs"] == ["x"]:
-                tc = conv1_uses_im2col(L, prec)
-                depth = wgrad_tc_depth(M, 1, 128, co, self.sm, self.part_cap()) if tc else 2 * M
-            else:
-                tc = prec == "bf16" and wgrad_tc_supported(L["ci"], co)
-                depth = wgrad_tc_depth(M, L["k"], L["ci"], co, self.sm, self.part_cap()) if tc else 2 * M
-            gw = self.grad[sc + "/weights"].reshape(L["k"], L["k"], L["ci"], co)[..., cols]
-            rec("dW " + sc, gw, v, gamma(depth) * sab + TINY)
-            assert not self.grad[sc + "/biases"].any(), sc
-        return res
-
-    def part_cap(self):
-        """Floats of the filter gradients' split partials (TrainWs::layout): the largest filter x 48."""
-        return max(L["k"] ** 2 * L["ci"] * L["co"] for L in self.layers) * 48
+            parts.append((v, gamma(depth) * sab))
+        v, b = rank_sum(parts)
+        for r in runs:
+            gw = r.grad[sc + "/weights"].reshape(L["k"], L["k"], L["ci"], co)[..., cols]
+            rec("dW " + sc, gw, v, b + TINY)
+            assert not r.grad[sc + "/biases"].any(), sc
+    return res
 
 
 def _assert_within(res, what):
