@@ -440,13 +440,27 @@ def check_train_forward(drs, monkeypatch, net, C, K, prec, B, crop, use_mask, sa
     taps = {"x": rounded(x.reshape(B, crop, crop, C), prec)}
     M = B * crop * crop
     idx = sample_pixels(B, crop, rs) if sampled else np.arange(M)
+    stats = {}
+    for L in layers:
+        sc, co = L["scope"], L["co"]
+        taps["z:" + sc] = s.debug_activation("z:" + sc, B, crop, co)
+        taps[sc] = s.debug_activation(sc, B, crop, co)
+        stats[sc] = (s.get_variable(sc + "/moving_mean"), s.get_variable(sc + "/moving_variance"))
+    s.close()
+    _assert_within(train_forward_checks(layers, act, p, taps, stats, prec, B, crop, idx, tag), (tag, prec, B, crop))
+
+
+def train_forward_checks(layers, act, p, taps, stats, prec, B, crop, idx, tag):
+    """The checks of check_train_forward on the taps of one training step: taps "x" (the input rounded to the session
+    precision), "z:<scope>" and "<scope>" per layer, stats {scope: (moving mean, moving variance)} after the step
+    (bn_decay = 0), p the variables the step started from.  Returns {quantity: largest err / bound}."""
+    M = B * crop * crop
     u, tiny = U[prec], TINY[prec]
     res = {}
     for L in layers:
         sc, co = L["scope"], L["co"]
-        Z = s.debug_activation("z:" + sc, B, crop, co)
-        taps[sc] = s.debug_activation(sc, B, crop, co)
-        mm, mv = s.get_variable(sc + "/moving_mean"), s.get_variable(sc + "/moving_variance")
+        Z = taps["z:" + sc]
+        mm, mv = stats[sc]
         # Z = conv + bias, stored in the session precision
         w = rounded(np.asarray(p[sc + "/weights"], np.float32), prec)
         b = np.asarray(p[sc + "/biases"], np.float64)
@@ -475,8 +489,7 @@ def check_train_forward(drs, monkeypatch, net, C, K, prec, B, crop, use_mask, sa
         ba = u * np.abs(a) + 8 * E24 * (np.abs(zn) + np.abs(mg)) * istd + tiny
         ref, bound = apply_post(L, a, ba, need, win, idx, B, crop, p, prec)
         res["out " + sc] = ratio((tag, prec, "out " + sc), taps[sc].reshape(-1, co)[idx], ref, bound)
-    s.close()
-    _assert_within(res, (tag, prec, B, crop))
+    return res
 
 
 @pytest.mark.parametrize("net,C,K,use_mask", TRAIN_NETS)
