@@ -240,6 +240,8 @@ struct PassGeometry {
   int key[8];
   std::vector<int32_t> pos, inst;
   CellTables ct;
+  int chunk = 0;                   // chunk size the accumulation ranges were split for
+  std::vector<int32_t> cuts;       // accumulation ranges [cuts[r], cuts[r+1]) (drs_scene_api.cuh: accum_ranges)
 };
 
 constexpr int RESULT_STRIDE = 64 + MAX_CLASSES * MAX_CLASSES;   // floats per pinned result slot: loss, then K*K+1 counts

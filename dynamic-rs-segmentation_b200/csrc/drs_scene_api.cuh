@@ -274,6 +274,49 @@ static void build_cells(const std::vector<int32_t>& pos, int H, int W, int crop,
   for (int64_t p = 0; p < P; ++p) ct.seq[fill[cell_of[p]]++] = (int32_t)p;   // ascending visit order per cell
 }
 
+// Visit ranges [cuts[r], cuts[r+1]) accumulated by one launch each: every chunk of `chunk` visits starts a range, and a
+// range ends before the visit that would give one of its pixels more than ACCUM_MAX_CONTRIB contributions.  The contest
+// grid visits a cell up to 3 times on a contest-shaped scene and up to 11 times on a tall one, so a chunk may need several
+// launches; the isprs grid and the coffee grid (square tiles) visit every cell once and never split a chunk.  Pixels
+// between two consecutive patch borders of each axis are covered by the same patches, so the counts are kept per pair of
+// such segments.
+static void accum_ranges(const std::vector<int32_t>& pos, int H, int W, int crop, int chunk, std::vector<int32_t>& cuts) {
+  const int P = (int)(pos.size() / 2);
+  std::vector<int32_t> seg[2];                       // segment of every row / column
+  int nseg[2];
+  for (int a = 0; a < 2; ++a) {
+    const int L = a ? W : H;
+    std::vector<uint8_t> border(L + 1, 0);
+    for (int p = 0; p < P; ++p) { border[pos[2 * p + a]] = 1; border[pos[2 * p + a] + crop] = 1; }
+    seg[a].resize(L);
+    int s = 0;
+    for (int y = 0; y < L; ++y) { if (y > 0 && border[y]) ++s; seg[a][y] = s; }
+    nseg[a] = s + 1;
+  }
+  std::vector<uint16_t> cnt((size_t)nseg[0] * nseg[1], 0);
+  std::vector<int32_t> stamp((size_t)nseg[0] * nseg[1], -1);    // range whose visits cnt[] counts
+  cuts.clear();
+  for (int p = 0; p < P; ++p) {
+    const int r0 = seg[0][pos[2 * p]], r1 = seg[0][pos[2 * p] + crop - 1];
+    const int c0 = seg[1][pos[2 * p + 1]], c1 = seg[1][pos[2 * p + 1] + crop - 1];
+    bool full = p % chunk == 0;
+    for (int r = r0; r <= r1 && !full; ++r)
+      for (int c = c0; c <= c1 && !full; ++c) {
+        const size_t i = (size_t)r * nseg[1] + c;
+        full = stamp[i] == (int32_t)cuts.size() - 1 && cnt[i] >= ACCUM_MAX_CONTRIB;
+      }
+    if (full) cuts.push_back(p);
+    const int32_t range = (int32_t)cuts.size() - 1;
+    for (int r = r0; r <= r1; ++r)
+      for (int c = c0; c <= c1; ++c) {
+        const size_t i = (size_t)r * nseg[1] + c;
+        if (stamp[i] != range) { stamp[i] = range; cnt[i] = 0; }
+        ++cnt[i];
+      }
+  }
+  cuts.push_back(P);
+}
+
 static void accumulate_chunk(Handle* h, const CellTables& ct, const float* logits, const std::vector<int32_t>& pos,
                              int seq0, int seq1, int H, int W, int K, int crop, int row_begin, int row_end) {
   int y_lo = H, y_hi = 0;
@@ -316,7 +359,7 @@ static void scene_pass_finish(Handle* h, int rows, int W, int K, uint8_t* labels
   CUDA_CHECK(cudaStreamSynchronize(h->stream));
   if (h->diag_host[15]) {
     h->diag_host[15] = 0;
-    DRS_FAIL("accumulate: a pixel is covered by more than %d patch visits of one chunk; the label map would be wrong", ACCUM_MAX_CONTRIB);
+    DRS_FAIL("accumulate: a pixel is covered by more than %d patch visits in one accumulation launch; the label map would be wrong", ACCUM_MAX_CONTRIB);
   }
 }
 
@@ -329,8 +372,11 @@ extern "C" int drs_accumulate_argmax(drs_handle_t h, const float* logits_dev, co
   std::vector<int32_t> pos(pos_host, pos_host + (size_t)P * 2);
   CellTables ct;
   build_cells(pos, H, W, crop, ct);
+  std::vector<int32_t> cuts;
+  accum_ranges(pos, H, W, crop, std::max(P, 1), cuts);
   scene_pass_begin(h, ct, H, W, K);
-  accumulate_chunk(h, ct, logits_dev, pos, 0, P, H, W, K, crop, 0, H);
+  for (size_t r = 0; r + 1 < cuts.size(); ++r)
+    accumulate_chunk(h, ct, logits_dev + (size_t)cuts[r] * crop * crop * K, pos, cuts[r], cuts[r + 1], H, W, K, crop, 0, H);
   scene_pass_finish(h, H, W, K, labels_out_host, mean_out_host);
   API_END
 }
@@ -468,6 +514,11 @@ static void scene_infer_impl(drs_handle_t h, int32_t scene_id, int32_t crop, int
   const int waves = getenv("DRS_CHUNK_WAVES") ? std::max(1, atoi(getenv("DRS_CHUNK_WAVES"))) : 40;
   const int64_t target_tiles = (int64_t)h->sm_count * waves;
   int chunk = (int)std::max<int64_t>(1, std::min<int64_t>(P, (target_tiles * CONV_TC_BM) / pp));
+  if (pg.chunk != chunk) {
+    accum_ranges(pos, H, W, crop, chunk, pg.cuts);
+    pg.chunk = chunk;
+  }
+  const std::vector<int32_t>& cuts = pg.cuts;
   const cudaStream_t main_stream = h->stream;
   auto cleanup = [&]() {
     cudaStreamSynchronize(main_stream);
@@ -483,6 +534,7 @@ static void scene_infer_impl(drs_handle_t h, int32_t scene_id, int32_t crop, int
     InferLane& L = h->lane;
     CUDA_CHECK(cudaEventRecord(h->lane_ready, main_stream));
     CUDA_CHECK(cudaStreamWaitEvent(L.stream, h->lane_ready, 0));
+    size_t r = 0;                                    // next accumulation range
     for (int s0 = 0; s0 < P; s0 += chunk) {
       const int nb = std::min(chunk, P - s0);
       {                                              // gather + forward of the chunk on the lane
@@ -506,7 +558,9 @@ static void scene_infer_impl(drs_handle_t h, int32_t scene_id, int32_t crop, int
         CUDA_CHECK(cudaEventRecord(L.fwd_done, L.stream));
       }
       CUDA_CHECK(cudaStreamWaitEvent(main_stream, L.fwd_done, 0));
-      accumulate_chunk(h, ct, L.lg, pos, s0, s0 + nb, H, W, K, crop, row_begin, row_end);
+      // the chunk's ranges in visit order on one stream: each pixel's sum keeps the script's order across launches
+      for (; cuts[r] < s0 + nb; ++r)
+        accumulate_chunk(h, ct, L.lg + (size_t)(cuts[r] - s0) * pp * K, pos, cuts[r], cuts[r + 1], H, W, K, crop, row_begin, row_end);
       CUDA_CHECK(cudaEventRecord(L.acc_done, main_stream));
     }
     scene_pass_finish(h, rows, W, K, labels_out_host, mean_out_host);

@@ -154,10 +154,12 @@ static void grid_positions(int H, int W, int crop, int batch, int variant, std::
 }
 
 // ------------------------------------------------------------------------------------------------
-// ordered accumulation.  The lattice of patch origins is {i*s} U {H-c} x {j*s} U {W-c}; a cell may be
-// visited 0, 1 or (contest bug) 2 times.  cell_off/cell_seq list, per cell, the visit numbers in
-// ascending order.  Each thread owns one pixel and adds its contributions in visit order, which makes
-// the fp32 sum bit-identical to NumPy's sequential `prob_im[...] += logits[j]` without atomics.
+// ordered accumulation.  The lattice of patch origins is {i*s} U {H-c} x {j*s} U {W-c}; a cell is
+// visited once by the isprs grid and the coffee grid (square tiles) and any number of times by the
+// contest grid (bug F10).
+// cell_off/cell_seq list, per cell, the visit numbers in ascending order.  Each thread owns one pixel
+// and adds its contributions in visit order, which makes the fp32 sum bit-identical to NumPy's
+// sequential `prob_im[...] += logits[j]` without atomics.
 // ------------------------------------------------------------------------------------------------
 struct AccumParams {
   const float* logits;      // [n_chunk, c, c, K], patch `seq` lives at (seq - seq0)
@@ -169,9 +171,11 @@ struct AccumParams {
   int row_begin, row_end;   // stripe owned by this rank
   int y_lo, y_hi;           // pixel rows touched by this chunk (clipped to the stripe)
   int seq0, seq1;           // visit numbers held in `logits`
-  uint32_t* overflow;       // host-mapped flag: a pixel had more contributions in one chunk than the kernel can order
+  uint32_t* overflow;       // host-mapped flag: a pixel had more contributions in one launch than the kernel can order
 };
-constexpr int ACCUM_MAX_CONTRIB = 32;   // 4 x 4 covering lattice cells (odd crop + shifted border row/col), each visited at most twice (contest)
+// Contributions one launch orders per pixel.  A pixel lies under at most 4 x 4 lattice cells (odd crop + shifted border
+// row/col); the host splits a chunk into visit ranges that stay within this limit (drs_scene_api.cuh: accum_ranges).
+constexpr int ACCUM_MAX_CONTRIB = 32;
 
 __device__ __forceinline__ int cover_range(int y, int L, int crop, int stride, int n, int* first, int* extra) {
   // regular origins i*s for i in [0, n-2] (and n-1 when the last origin is not shifted), last origin L-crop
