@@ -9,6 +9,7 @@ closed-form stand-in to pin the host logic against reference-generated traces wi
     train_on_plan(plan, loss_mask=None)  == train_result(submit_train(...))
     eval_on_plan(plan, scene_offset=0)   -> (pred int64 [B,c,c], labels [B,c,c]) gather + normalise + sess.run(pred_up)
     scene_labels(scene_id, crop, batch, variant) -> uint8 [H,W]   whole sliding-window inference
+    scene_multiscale_labels(scene_id, crops, batch, variant) -> uint8 [H,W]   multi-scale evaluation, one pass per crop
     save(path) / restore(path)                                    tf.train.Saver stand-in (one .npz keyed by TF names)
 """
 import numpy as np
@@ -212,6 +213,23 @@ class GpuBackend:
             self.s.scene_infer(scene_id, crop, batch, H, W, variant=variant, row_begin=r0, row_end=r1, keep_on_device=True)
             return self.s.scene_gather_labels(H, W, ddist.stripe_bounds(H, self.world), self.rank, all_ranks=True)
         stripe = self.s.scene_infer(scene_id, crop, batch, H, W, variant=variant, row_begin=r0, row_end=r1)
+        return ddist.gather_label_stripes(stripe, H, W, self.rank, self.world, device=self.dev, all_ranks=True)
+
+    def scene_multiscale_labels(self, scene_id, crops, batch, variant="isprs"):
+        """Label map of the multi-scale evaluation (isprs:1380-1411) over ``crops`` in order, computed on the device: the
+        argmax of the summed softmax of every scale's mean map, bit for bit the host composition.  Striped over the ranks
+        like scene_labels."""
+        H, W = self.shapes[scene_id]
+        crops = [int(c) for c in crops]
+        if self.world == 1:
+            return self.s.scene_infer_multiscale(scene_id, crops, batch, H, W, variant=variant)
+        from . import dist as ddist
+        r0, r1 = ddist.stripe_bounds(H, self.world, self.rank)
+        if self.s.has_nccl:
+            self.s.scene_infer_multiscale(scene_id, crops, batch, H, W, variant=variant, row_begin=r0, row_end=r1,
+                                          keep_on_device=True)
+            return self.s.scene_gather_labels(H, W, ddist.stripe_bounds(H, self.world), self.rank, all_ranks=True)
+        stripe = self.s.scene_infer_multiscale(scene_id, crops, batch, H, W, variant=variant, row_begin=r0, row_end=r1)
         return ddist.gather_label_stripes(stripe, H, W, self.rank, self.world, device=self.dev, all_ranks=True)
 
     def scene_mean_logits(self, scene_id, crop, batch, variant="isprs"):

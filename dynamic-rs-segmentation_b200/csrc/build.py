@@ -18,7 +18,7 @@ OUT = os.path.join(PKG, "libdrs.so")
 STAMP = os.path.join(PKG, ".libdrs.stamp")
 OBJ_DIR = os.path.join(HERE, "_build")
 CUDA_DEPS = ["drs_api.cu", "drs_train.cuh", "drs_scene_api.cuh", "drs_common.cuh", "ptx_sm100.cuh", "conv_tc.cuh",
-             "conv_simt.cuh", "ops.cuh", "scene.cuh", "wgrad_tc.cuh", "conv1_tc.cuh", "drs_comm.cuh", "variants.cuh", "pool_train.cuh", "npz_io.h", "../../include/drs.h"]
+             "conv_simt.cuh", "ops.cuh", "scene.cuh", "wgrad_tc.cuh", "conv1_tc.cuh", "drs_comm.cuh", "variants.cuh", "pool_train.cuh", "npz_io.h", "np_softmax.h", "../../include/drs.h"]
 CUDA_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-std=c++17", "-lineinfo", "-Xcompiler", "-fPIC",
               "-Xcompiler", "-fvisibility=default", "--expt-relaxed-constexpr"]
 # host planner: the Gaussian values must be bit-identical to NumPy's, so no fast-math and no FMA contraction
@@ -28,6 +28,8 @@ UNITS = [
     ("drs_api.cu", CUDA_DEPS, "nvcc", CUDA_FLAGS),
     ("host_plan.cpp", ["host_plan.cpp", "../../include/drs.h"], "g++", HOST_FLAGS),
     ("npz_io.cpp", ["npz_io.cpp", "npz_io.h"], "g++", HOST_FLAGS),
+    # the multi-scale softmax of the scene pass, for the host (drs_debug_np_softmax): same no-contraction rule as the planner
+    ("np_softmax.cpp", ["np_softmax.cpp", "np_softmax.h", "../../include/drs.h"], "g++", HOST_FLAGS),
 ]
 LINK_FLAGS = ["-shared", "-cudart", "static", "-Xcompiler", "-fPIC", "-Xlinker", "-ldl", "-Xcompiler", "-pthread"]
 

@@ -326,6 +326,7 @@ struct drs_handle_s {
     DevMem<int32_t> cell_off, cell_seq;   // cell tables of the visiting order
     DevMem<uint8_t> labels;               // label map [rows][W]
     DevMem<double> mean;                  // mean score map [rows][W][K]
+    DevMem<float> prob_sum;               // multi-scale: sum over the scales of softmax(mean) [rows][W][K]
     DevMem<int32_t> inst;                 // (scene, row, col) of every patch of the pass
     DevMem<uint8_t> assembled;            // [H][W] label map assembled from every rank's stripe
   } pass;

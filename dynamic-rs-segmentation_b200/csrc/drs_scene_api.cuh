@@ -348,6 +348,14 @@ static void scene_pass_begin(Handle* h, const CellTables& ct, int rows, int W, i
   if (!ct.seq.empty()) CUDA_CHECK(cudaMemcpyAsync(cell_seq, ct.seq.data(), ct.seq.size() * 4, cudaMemcpyHostToDevice, h->stream));
 }
 
+// after the pass's stream has been synchronised
+static void accum_overflow_check(Handle* h) {
+  if (h->diag_host[15]) {
+    h->diag_host[15] = 0;
+    DRS_FAIL("accumulate: a pixel is covered by more than %d patch visits in one accumulation launch; the label map would be wrong", ACCUM_MAX_CONTRIB);
+  }
+}
+
 static void scene_pass_finish(Handle* h, int rows, int W, int K, uint8_t* labels_host, double* mean_host) {
   const int64_t npix = (int64_t)rows * W;
   uint8_t* lab_dev = pass_buf(h, h->pass.labels, npix);
@@ -357,10 +365,7 @@ static void scene_pass_finish(Handle* h, int rows, int W, int K, uint8_t* labels
   if (labels_host) CUDA_CHECK(cudaMemcpyAsync(labels_host, lab_dev, npix, cudaMemcpyDeviceToHost, h->stream));
   if (mean_host) CUDA_CHECK(cudaMemcpyAsync(mean_host, mean_dev, npix * K * 8, cudaMemcpyDeviceToHost, h->stream));
   CUDA_CHECK(cudaStreamSynchronize(h->stream));
-  if (h->diag_host[15]) {
-    h->diag_host[15] = 0;
-    DRS_FAIL("accumulate: a pixel is covered by more than %d patch visits in one accumulation launch; the label map would be wrong", ACCUM_MAX_CONTRIB);
-  }
+  accum_overflow_check(h);
 }
 
 extern "C" int drs_accumulate_argmax(drs_handle_t h, const float* logits_dev, const int32_t* pos_host, int32_t P, int32_t crop,
@@ -394,7 +399,7 @@ static void lane_ensure(Handle* h, size_t arena_bytes, size_t x_bytes, size_t lg
   }
   L.arena.mem.grow(arena_bytes, arena_bytes, {L.stream});
   L.x.grow(x_bytes, x_bytes, {L.stream});
-  L.lg.grow(lg_bytes, lg_bytes, {L.stream});
+  L.lg.grow(lg_bytes, lg_bytes, {L.stream, h->stream});   // the accumulation of an earlier pass may still read the logits
 }
 
 // Streamed upload of a host scene during a scene pass: rows are copied on a separate stream, in ~8 MB pieces, just ahead of
@@ -470,12 +475,12 @@ static PassGeometry& pass_geometry(Handle* h, int scene_id, int H, int W, int cr
   const int key[8] = {scene_id, H, W, crop, batch, variant, row_begin, row_end};
   for (auto& g : cache)
     if (memcmp(g.key, key, sizeof(key)) == 0) return g;
+  std::vector<int32_t> all;
+  grid_positions(H, W, crop, batch, variant, all);   // throws for a crop that does not fit: nothing is cached then
   if (cache.size() >= 8) cache.erase(cache.begin());
   cache.emplace_back();
   PassGeometry& g = cache.back();
   memcpy(g.key, key, sizeof(key));
-  std::vector<int32_t> all;
-  grid_positions(H, W, crop, batch, variant, all);
   for (size_t p = 0; p < all.size() / 2; ++p)
     if (all[2 * p] < row_end && all[2 * p] + crop > row_begin) { g.pos.push_back(all[2 * p]); g.pos.push_back(all[2 * p + 1]); }
   build_cells(g.pos, H, W, crop, g.ct);
@@ -483,6 +488,86 @@ static PassGeometry& pass_geometry(Handle* h, int scene_id, int H, int W, int cr
   g.inst.resize(P * 3);
   for (size_t p = 0; p < P; ++p) { g.inst[3 * p] = scene_id; g.inst[3 * p + 1] = g.pos[2 * p]; g.inst[3 * p + 2] = g.pos[2 * p + 1]; }
   return g;
+}
+
+// The geometry of a pass of `crop` over rows [row_begin, row_end) of a resident scene (row bounds already clipped), checked
+// against the rows that are resident, with its accumulation ranges for the current chunk size.  Launches nothing.
+static PassGeometry& scene_pass_geometry(Handle* h, const Scene& sc, int32_t scene_id, int32_t crop, int32_t batch,
+                                         int32_t variant, int32_t row_begin, int32_t row_end) {
+  const int H = sc.H, W = sc.W;
+  // visiting order of the script, restricted to patches that touch the stripe (order preserved), with its per-cell visit
+  // tables: pure functions of the geometry, memoised (a validation run visits the same scenes with the same crop again
+  // and again; for a 6000x6000 tile they take several milliseconds of host time per call)
+  PassGeometry& pg = pass_geometry(h, scene_id, H, W, crop, batch, variant, row_begin, row_end);
+  const std::vector<int32_t>& pos = pg.pos;
+  const int P = (int)(pos.size() / 2);
+  for (int p = 0; p < P; ++p)
+    DRS_CHECK(pos[2 * p] >= sc.row0 && pos[2 * p] + crop <= sc.row0 + sc.rows,
+              "scene_infer: stripe [%d,%d) needs scene rows [%d,%d) but only [%d,%d) are resident", row_begin, row_end, pos[2 * p],
+              pos[2 * p] + crop, sc.row0, sc.row0 + sc.rows);
+  // chunk = a whole number of 128-pixel tiles close to a multiple of the SM count (full conv waves), ~0.75 M pixels
+  const int64_t pp = (int64_t)crop * crop;
+  const int waves = getenv("DRS_CHUNK_WAVES") ? std::max(1, atoi(getenv("DRS_CHUNK_WAVES"))) : 40;
+  const int64_t target_tiles = (int64_t)h->sm_count * waves;
+  int chunk = (int)std::max<int64_t>(1, std::min<int64_t>(P, (target_tiles * CONV_TC_BM) / pp));
+  if (pg.chunk != chunk) {
+    accum_ranges(pos, H, W, crop, chunk, pg.cuts);
+    pg.chunk = chunk;
+  }
+  return pg;
+}
+
+// The loop of a scene pass: prob / occur cleared, then gather, forward and ordered accumulation of every chunk.  The caller
+// turns h->pass.prob / occur into labels (scene_pass_finish, or the multi-scale softmax) on the handle's stream.
+static void scene_pass_accumulate(Handle* h, const Scene& sc, const PassGeometry& pg, int32_t crop, int32_t row_begin,
+                                  int32_t row_end, HostSceneFeed* feed) {
+  const int H = sc.H, W = sc.W, K = h->net.classes, C = h->net.channels;
+  const std::vector<int32_t>& pos = pg.pos;
+  const CellTables& ct = pg.ct;
+  const int P = (int)(pos.size() / 2);
+  const int rows = row_end - row_begin;
+  const int64_t pp = (int64_t)crop * crop;
+  const int chunk = pg.chunk;
+  const std::vector<int32_t>& cuts = pg.cuts;
+  const cudaStream_t main_stream = h->stream;
+  scene_pass_begin(h, ct, rows, W, K);
+  const std::vector<int32_t>& inst = pg.inst;
+  int32_t* inst_dev = pass_buf(h, h->pass.inst, std::max<size_t>(inst.size(), 1) * 4);
+  CUDA_CHECK(cudaMemcpyAsync(inst_dev, inst.data(), inst.size() * 4, cudaMemcpyHostToDevice, h->stream));
+  refresh_packed(h, false);                       // packed weights / folded BN once, before the lane starts
+  lane_ensure(h, eval_arena_bytes(h, chunk, crop), (size_t)chunk * pp * C * 4, (size_t)chunk * pp * K * 4);
+  InferLane& L = h->lane;
+  CUDA_CHECK(cudaEventRecord(h->lane_ready, main_stream));
+  CUDA_CHECK(cudaStreamWaitEvent(L.stream, h->lane_ready, 0));
+  size_t r = 0;                                    // next accumulation range
+  for (int s0 = 0; s0 < P; s0 += chunk) {
+    const int nb = std::min(chunk, P - s0);
+    {                                              // gather + forward of the chunk on the lane
+      StreamScope on_lane(h, true, L.stream, &L.arena);
+      if (s0 > 0) CUDA_CHECK(cudaStreamWaitEvent(L.stream, L.acc_done, 0));   // logits buffer of the previous chunk consumed
+      if (feed) {
+        // rows this chunk's patches read, plus one more chunk's worth so that the copy runs ahead of the compute
+        int need = 0;
+        const int s1 = std::min(P, s0 + 2 * chunk);
+        for (int s = s0; s < s1; ++s) need = std::max(need, pos[2 * s] + crop);
+        feed_rows(h, *feed, sc, need, L.stream);
+      }
+      GatherParams gp;
+      memset(&gp, 0, sizeof(gp));
+      gp.inst = inst_dev + (size_t)s0 * 3;
+      gp.x_out = L.x;
+      gp.B = nb;
+      gp.crop = crop;
+      launch_gather(h, gp);
+      forward_eval(h, L.x, nb, crop, L.lg, nullptr);
+      CUDA_CHECK(cudaEventRecord(L.fwd_done, L.stream));
+    }
+    CUDA_CHECK(cudaStreamWaitEvent(main_stream, L.fwd_done, 0));
+    // the chunk's ranges in visit order on one stream: each pixel's sum keeps the script's order across launches
+    for (; cuts[r] < s0 + nb; ++r)
+      accumulate_chunk(h, ct, L.lg + (size_t)(cuts[r] - s0) * pp * K, pos, cuts[r], cuts[r + 1], H, W, K, crop, row_begin, row_end);
+    CUDA_CHECK(cudaEventRecord(L.acc_done, main_stream));
+  }
 }
 
 static void scene_infer_impl(drs_handle_t h, int32_t scene_id, int32_t crop, int32_t batch, int32_t variant, int32_t row_begin,
@@ -493,76 +578,19 @@ static void scene_infer_impl(drs_handle_t h, int32_t scene_id, int32_t crop, int
   auto it = h->scenes.find(scene_id);
   DRS_CHECK(it != h->scenes.end(), "scene_infer: scene %d not uploaded", scene_id);
   const Scene& sc = it->second;
-  const int H = sc.H, W = sc.W, K = h->net.classes, C = h->net.channels;
+  const int H = sc.H, W = sc.W, K = h->net.classes;
   if (row_end <= 0 || row_end > H) row_end = H;
   if (row_begin < 0) row_begin = 0;
   DRS_CHECK(row_begin < row_end, "scene_infer: empty stripe");
-  // visiting order of the script, restricted to patches that touch the stripe (order preserved), with its per-cell visit
-  // tables: pure functions of the geometry, memoised (a validation run visits the same scenes with the same crop again
-  // and again; for a 6000x6000 tile they take several milliseconds of host time per call)
-  PassGeometry& pg = pass_geometry(h, scene_id, H, W, crop, batch, variant, row_begin, row_end);
-  const std::vector<int32_t>& pos = pg.pos;
-  const CellTables& ct = pg.ct;
-  const int P = (int)(pos.size() / 2);
-  for (int p = 0; p < P; ++p)
-    DRS_CHECK(pos[2 * p] >= sc.row0 && pos[2 * p] + crop <= sc.row0 + sc.rows,
-              "scene_infer: stripe [%d,%d) needs scene rows [%d,%d) but only [%d,%d) are resident", row_begin, row_end, pos[2 * p],
-              pos[2 * p] + crop, sc.row0, sc.row0 + sc.rows);
+  const PassGeometry& pg = scene_pass_geometry(h, sc, scene_id, crop, batch, variant, row_begin, row_end);
   const int rows = row_end - row_begin;
-  // chunk = a whole number of 128-pixel tiles close to a multiple of the SM count (full conv waves), ~0.75 M pixels
-  const int64_t pp = (int64_t)crop * crop;
-  const int waves = getenv("DRS_CHUNK_WAVES") ? std::max(1, atoi(getenv("DRS_CHUNK_WAVES"))) : 40;
-  const int64_t target_tiles = (int64_t)h->sm_count * waves;
-  int chunk = (int)std::max<int64_t>(1, std::min<int64_t>(P, (target_tiles * CONV_TC_BM) / pp));
-  if (pg.chunk != chunk) {
-    accum_ranges(pos, H, W, crop, chunk, pg.cuts);
-    pg.chunk = chunk;
-  }
-  const std::vector<int32_t>& cuts = pg.cuts;
   const cudaStream_t main_stream = h->stream;
   auto cleanup = [&]() {
     cudaStreamSynchronize(main_stream);
     if (h->lane.stream) cudaStreamSynchronize(h->lane.stream);
   };
   try {
-    scene_pass_begin(h, ct, rows, W, K);
-    const std::vector<int32_t>& inst = pg.inst;
-    int32_t* inst_dev = pass_buf(h, h->pass.inst, std::max<size_t>(inst.size(), 1) * 4);
-    CUDA_CHECK(cudaMemcpyAsync(inst_dev, inst.data(), inst.size() * 4, cudaMemcpyHostToDevice, h->stream));
-    refresh_packed(h, false);                       // packed weights / folded BN once, before the lane starts
-    lane_ensure(h, eval_arena_bytes(h, chunk, crop), (size_t)chunk * pp * C * 4, (size_t)chunk * pp * K * 4);
-    InferLane& L = h->lane;
-    CUDA_CHECK(cudaEventRecord(h->lane_ready, main_stream));
-    CUDA_CHECK(cudaStreamWaitEvent(L.stream, h->lane_ready, 0));
-    size_t r = 0;                                    // next accumulation range
-    for (int s0 = 0; s0 < P; s0 += chunk) {
-      const int nb = std::min(chunk, P - s0);
-      {                                              // gather + forward of the chunk on the lane
-        StreamScope on_lane(h, true, L.stream, &L.arena);
-        if (s0 > 0) CUDA_CHECK(cudaStreamWaitEvent(L.stream, L.acc_done, 0));   // logits buffer of the previous chunk consumed
-        if (feed) {
-          // rows this chunk's patches read, plus one more chunk's worth so that the copy runs ahead of the compute
-          int need = 0;
-          const int s1 = std::min(P, s0 + 2 * chunk);
-          for (int s = s0; s < s1; ++s) need = std::max(need, pos[2 * s] + crop);
-          feed_rows(h, *feed, sc, need, L.stream);
-        }
-        GatherParams gp;
-        memset(&gp, 0, sizeof(gp));
-        gp.inst = inst_dev + (size_t)s0 * 3;
-        gp.x_out = L.x;
-        gp.B = nb;
-        gp.crop = crop;
-        launch_gather(h, gp);
-        forward_eval(h, L.x, nb, crop, L.lg, nullptr);
-        CUDA_CHECK(cudaEventRecord(L.fwd_done, L.stream));
-      }
-      CUDA_CHECK(cudaStreamWaitEvent(main_stream, L.fwd_done, 0));
-      // the chunk's ranges in visit order on one stream: each pixel's sum keeps the script's order across launches
-      for (; cuts[r] < s0 + nb; ++r)
-        accumulate_chunk(h, ct, L.lg + (size_t)(cuts[r] - s0) * pp * K, pos, cuts[r], cuts[r + 1], H, W, K, crop, row_begin, row_end);
-      CUDA_CHECK(cudaEventRecord(L.acc_done, main_stream));
-    }
+    scene_pass_accumulate(h, sc, pg, crop, row_begin, row_end, feed);
     scene_pass_finish(h, rows, W, K, labels_out_host, mean_out_host);
     h->last_scene = scene_id; h->last_row_begin = row_begin; h->last_rows = rows; h->last_W = W;
     if (feed) {                                      // rows no patch reads (none for the grids of the scripts) and the tail
@@ -571,6 +599,85 @@ static void scene_infer_impl(drs_handle_t h, int32_t scene_id, int32_t crop, int
     }
   } catch (...) { cleanup(); throw; }
   cleanup();
+}
+
+// validate_test_multiscale (isprs:1347-1474): the scene pass of each crop, in the order given, each followed by the softmax of
+// its mean map added to a float32 sum (multiscale_softmax_add_kernel); the last one also writes the label map.  Every crop
+// is checked before the first launch, so a refused call leaves the handle as it was.
+extern "C" int drs_scene_infer_multiscale(drs_handle_t h, int32_t scene_id, int32_t n_scales, const int32_t* crops_host, int32_t batch,
+                                          int32_t variant, int32_t row_begin, int32_t row_end, uint8_t* labels_out_host,
+                                          float* prob_sum_out_host) {
+  API_BEGIN
+  DRS_CHECK(h, "null argument");
+  DRS_CHECK(n_scales >= 1, "scene_infer_multiscale: n_scales=%d, need at least one scale", n_scales);
+  DRS_CHECK(crops_host, "scene_infer_multiscale: null crop list");
+  DRS_CHECK(batch >= 1, "grid: batch must be >= 1");
+  CUDA_CHECK(cudaSetDevice(h->cfg.device));
+  auto it = h->scenes.find(scene_id);
+  DRS_CHECK(it != h->scenes.end(), "scene_infer: scene %d not uploaded", scene_id);
+  const Scene& sc = it->second;
+  const int H = sc.H, W = sc.W, K = h->net.classes;
+  DRS_CHECK(K >= 1 && K <= MAX_CLASSES, "K=%d out of range", K);
+  if (row_end <= 0 || row_end > H) row_end = H;
+  if (row_begin < 0) row_begin = 0;
+  DRS_CHECK(row_begin < row_end, "scene_infer: empty stripe");
+  for (int s = 0; s < n_scales; ++s) {
+    const int crop = crops_host[s];
+    DRS_CHECK(crop / 2 >= 1 && crop <= H && crop <= W, "grid: crop %d does not fit scene %dx%d", crop, H, W);
+    scene_pass_geometry(h, sc, scene_id, crop, batch, variant, row_begin, row_end);   // resident rows cover every patch
+  }
+  const int rows = row_end - row_begin;
+  const int64_t npix = (int64_t)rows * W;
+  const cudaStream_t main_stream = h->stream;
+  auto cleanup = [&]() {
+    cudaStreamSynchronize(main_stream);
+    if (h->lane.stream) cudaStreamSynchronize(h->lane.stream);
+  };
+  h->last_scene = -1;                                // the label buffer is rewritten from here on
+  try {
+    float* sum = pass_buf(h, h->pass.prob_sum, (size_t)npix * K * 4);
+    uint8_t* lab = pass_buf(h, h->pass.labels, npix);
+    for (int s = 0; s < n_scales; ++s) {
+      // (looked up again: the geometry cache keeps only the last few passes)
+      const PassGeometry& pg = scene_pass_geometry(h, sc, scene_id, crops_host[s], batch, variant, row_begin, row_end);
+      scene_pass_accumulate(h, sc, pg, crops_host[s], row_begin, row_end, nullptr);
+      multiscale_softmax_add_kernel<<<nblk(npix, 256), 256, 0, h->stream>>>(h->pass.prob, h->pass.occur, npix, K, s == 0, sum,
+                                                                            s == n_scales - 1 ? lab : nullptr);
+      LAUNCH_CHECK(h);
+    }
+    if (labels_out_host) CUDA_CHECK(cudaMemcpyAsync(labels_out_host, lab, npix, cudaMemcpyDeviceToHost, h->stream));
+    if (prob_sum_out_host) CUDA_CHECK(cudaMemcpyAsync(prob_sum_out_host, sum, (size_t)npix * K * 4, cudaMemcpyDeviceToHost, h->stream));
+    CUDA_CHECK(cudaStreamSynchronize(h->stream));
+    accum_overflow_check(h);
+    h->last_scene = scene_id; h->last_row_begin = row_begin; h->last_rows = rows; h->last_W = W;
+  } catch (...) { cleanup(); throw; }
+  cleanup();
+  API_END
+}
+
+// One launch of multiscale_softmax_add_kernel on caller-given sums and counts (unit tests: the device arithmetic over any
+// range of means, not only the ones a net produces).  prob [npix,K], occur [npix], acc [npix,K] in/out (ignored on input when
+// first != 0); labels_out_host non-null = the last scale (argmax written).
+extern "C" int drs_debug_multiscale_softmax_add(drs_handle_t h, const float* prob_host, const uint32_t* occur_host, int64_t npix,
+                                                int32_t first, float* acc_inout_host, uint8_t* labels_out_host) {
+  API_BEGIN
+  DRS_CHECK(h && prob_host && occur_host && acc_inout_host && npix >= 1, "null argument");
+  CUDA_CHECK(cudaSetDevice(h->cfg.device));
+  const int K = h->net.classes;
+  DevMem<float> prob(npix * K * 4), acc(npix * K * 4);
+  DevMem<uint32_t> occur(npix * 4);
+  DevMem<uint8_t> lab(npix);
+  CUDA_CHECK(cudaMemcpyAsync(prob, prob_host, npix * K * 4, cudaMemcpyHostToDevice, h->stream));
+  CUDA_CHECK(cudaMemcpyAsync(occur, occur_host, npix * 4, cudaMemcpyHostToDevice, h->stream));
+  CUDA_CHECK(cudaMemcpyAsync(acc, acc_inout_host, npix * K * 4, cudaMemcpyHostToDevice, h->stream));
+  multiscale_softmax_add_kernel<<<nblk(npix, 256), 256, 0, h->stream>>>(prob, occur, npix, K, first != 0, acc,
+                                                                        labels_out_host ? lab.get() : nullptr);
+  LAUNCH_CHECK(h);
+  CUDA_CHECK(cudaMemcpyAsync(acc_inout_host, acc, npix * K * 4, cudaMemcpyDeviceToHost, h->stream));
+  if (labels_out_host) CUDA_CHECK(cudaMemcpyAsync(labels_out_host, lab, npix, cudaMemcpyDeviceToHost, h->stream));
+  int rc = drs_synchronize(h);
+  if (rc) return rc;
+  API_END
 }
 
 // Scene-level confusion matrix (isprs:1289-1296, contest:944-951): the label map of the last drs_scene_infer pass over

@@ -2,10 +2,12 @@
 //   patch gather (+flip, +noise, +override) + normalize_images   isprs:245-334, 74-81
 //   sliding-window grid (host, integer, bit-exact)               isprs:337-400, contest:257-328, coffee:296-349
 //   ordered overlap accumulation + argmax                        isprs:1261-1284
+//   multi-scale softmax sum + argmax                              isprs:1380-1411
 #pragma once
 #include <algorithm>
 
 #include "drs_common.cuh"
+#include "np_softmax.h"
 
 constexpr int GATHER_INLINE_MAX = 256;
 // Small batches carry their instance table inside the kernel parameters: no staging copy, no host synchronisation.
@@ -252,4 +254,37 @@ __global__ void scene_argmax_kernel(const float* __restrict__ prob, const uint32
     if (v > best) { best = v; bi = k; }
   }
   labels[i] = (uint8_t)bi;
+}
+
+// validate_test_multiscale (isprs:1380-1411), per pixel after each scale's pass, in NumPy's float32 arithmetic:
+//   acc += softmax(float32(prob / float64(occur)))     (occur==0 -> 1; the first scale adds to 0, which is exact)
+// and on the last scale (labels non-null) label = np.argmax(acc): the first maximum, or the first NaN.
+static_assert(MAX_CLASSES <= NP_SOFTMAX_MAX_K, "np_softmax_pixel holds MAX_CLASSES values");
+__global__ void multiscale_softmax_add_kernel(const float* __restrict__ prob, const uint32_t* __restrict__ occur, int64_t npix,
+                                              int K, int first, float* __restrict__ acc, uint8_t* __restrict__ labels) {
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= npix) return;
+  uint32_t oc = occur[i];
+  if (oc == 0) oc = 1;
+  const double d = (double)oc;
+  float m[NP_SOFTMAX_MAX_K], p[NP_SOFTMAX_MAX_K];
+#pragma unroll
+  for (int k = 0; k < NP_SOFTMAX_MAX_K; ++k)
+    if (k < K) m[k] = __double2float_rn(__ddiv_rn((double)prob[i * K + k], d));   // mean_prob[scale] = prob_im / occur_im
+  np_softmax_pixel(m, K, p);
+  float best = 0.0f;
+  int bi = 0;
+  bool nan_seen = false;
+#pragma unroll
+  for (int k = 0; k < NP_SOFTMAX_MAX_K; ++k)
+    if (k < K) {
+      const float a = __fadd_rn(first ? 0.0f : acc[i * K + k], p[k]);
+      acc[i * K + k] = a;
+      if (!nan_seen && (k == 0 || !(a <= best))) {
+        best = a;
+        bi = k;
+        nan_seen = a != a;
+      }
+    }
+  if (labels) labels[i] = (uint8_t)bi;
 }

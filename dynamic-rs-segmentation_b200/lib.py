@@ -106,6 +106,10 @@ _SIGNATURES = {
     "drs_confusion_dev": (C.c_int, [_P, _P, _P, _P, C.c_int64, C.c_int32, C.c_int32, _P]),
     "drs_scene_infer_host": (C.c_int, [_P, C.c_int32, _P, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32,
                                        C.c_int32, _P, _P]),
+    "drs_scene_infer_multiscale": (C.c_int, [_P, C.c_int32, C.c_int32, _P, C.c_int32, C.c_int32, C.c_int32, C.c_int32, _P, _P]),
+    "drs_debug_np_softmax": (C.c_int, [_P, C.c_int64, C.c_int32, _P]),
+    "drs_debug_np_expf": (C.c_int, [_P, C.c_int64, _P]),
+    "drs_debug_multiscale_softmax_add": (C.c_int, [_P, _P, _P, C.c_int64, C.c_int32, _P, _P]),
     "drs_scene_confusion": (C.c_int, [_P, C.c_int32, C.c_int32, C.c_int32, _P]),
     "drs_launch_count": (C.c_int64, [_P]),
     "drs_set_profiling": (C.c_int, [_P, C.c_int32]),

@@ -343,6 +343,20 @@ class Session:
                                           L.ptr(labels), L.ptr(mean)))
         return (labels, mean) if want_mean else labels
 
+    def scene_infer_multiscale(self, scene_id, crops, batch, H, W, variant="isprs", row_begin=0, row_end=None, want_sum=False,
+                               keep_on_device=False):
+        """validate_test_multiscale (isprs:1347-1474) for one scene (stripe): a scene pass per crop, in the order given, each
+        mean map softmax-ed with NumPy's float32 arithmetic and added to a float32 sum; the labels are its argmax.
+        want_sum: also return the sum ([rows, W, K] float32, ``np.sum(mean_prob, axis=0)``).  keep_on_device: as scene_infer."""
+        c = np.ascontiguousarray(np.asarray(crops, dtype=np.int32).reshape(-1))
+        row_end = H if row_end is None else row_end
+        rows = row_end - row_begin
+        labels = None if keep_on_device else np.empty((rows, W), dtype=np.uint8)
+        psum = np.empty((rows, W, self.num_classes), dtype=np.float32) if want_sum else None
+        L.check(self._lib.drs_scene_infer_multiscale(self._h, scene_id, int(c.size), L.ptr(c), batch, L.GRID[variant], row_begin,
+                                                     row_end, L.ptr(labels), L.ptr(psum)))
+        return (labels, psum) if want_sum else labels
+
     def scene_infer_host(self, scene_id, scene, crop, batch, variant="isprs", want_mean=False):
         """scene_infer for a scene that is still a host array (a fresh tile): the upload is streamed just ahead of the
         chunks that read it and overlaps the convolutions.  The scene stays resident as scene_id."""
@@ -421,6 +435,20 @@ class Session:
                                           L.ptr(out), L.ptr(dz), L.ptr(mean), L.ptr(istd)))
         return out, dz, mean, istd
 
+    def debug_multiscale_softmax_add(self, prob, occur, acc=None, want_labels=True):
+        """One launch of the multi-scale kernel: (acc + softmax(float32(prob / occur)), first argmax of it or None).
+        prob [N, K] float32 score sums, occur [N] visit counts, acc [N, K] float32 or None (the first scale)."""
+        p = np.ascontiguousarray(np.asarray(prob, dtype=np.float32))
+        o = np.ascontiguousarray(np.asarray(occur, dtype=np.uint32))
+        n = o.size
+        if p.shape != (n, self.num_classes):
+            raise ValueError("prob must be [N, K] = [%d, %d]" % (n, self.num_classes))
+        out = np.zeros_like(p) if acc is None else np.array(acc, dtype=np.float32, order="C", copy=True)
+        labels = np.empty(n, dtype=np.uint8) if want_labels else None
+        L.check(self._lib.drs_debug_multiscale_softmax_add(self._h, L.ptr(p), L.ptr(o), n, int(acc is None), L.ptr(out),
+                                                           L.ptr(labels)))
+        return out, labels
+
     def debug_wgrad(self, x, dy, k, rate, precision="bf16"):
         x = np.ascontiguousarray(x, dtype=np.float32)
         dy = np.ascontiguousarray(dy, dtype=np.float32)
@@ -464,6 +492,24 @@ def npz_read(path):
         a = np.empty(cnt.value, dtype=np.float32)
         L.check(lib.drs_npz_read(str(path).encode(), buf.value, L.ptr(a), cnt.value))
         out[buf.value.decode("utf-8", "replace")] = a.reshape([dims[j] for j in range(nd.value)])
+    return out
+
+
+def np_softmax(values):
+    """The multi-scale kernel's per-pixel softmax over the last axis, compiled for the host (drs_debug_np_softmax, no GPU):
+    equal bit for bit to ``loops.reference_softmax`` of a float32 array."""
+    a = np.ascontiguousarray(np.asarray(values, dtype=np.float32))
+    K = a.shape[-1]
+    out = np.empty_like(a)
+    L.check(L.load().drs_debug_np_softmax(L.ptr(a), a.size // K, K, L.ptr(out)))
+    return out
+
+
+def np_expf(values):
+    """The exp of that softmax (NumPy's float32 exp restated), compiled for the host (drs_debug_np_expf, no GPU)."""
+    a = np.ascontiguousarray(np.asarray(values, dtype=np.float32))
+    out = np.empty_like(a)
+    L.check(L.load().drs_debug_np_expf(L.ptr(a), a.size, L.ptr(out)))
     return out
 
 

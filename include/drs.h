@@ -307,6 +307,23 @@ int drs_scene_infer_host(drs_handle_t h, int32_t scene_id, const void* scene_hos
                          int32_t dtype, int32_t crop, int32_t batch, int32_t variant, uint8_t* labels_out_host,
                          double* mean_out_host);
 
+/* validate_test_multiscale (isprs:1347-1474): one drs_scene_infer pass per crop, in the order given, over rows
+ * [row_begin,row_end); after each pass every pixel adds softmax(float32(prob_im/occur_im)) with NumPy's float32 arithmetic
+ * to a float32 sum; the label map is its first argmax.  labels_out_host NULL = stay on the device for
+ * drs_scene_confusion / drs_scene_gather_labels; prob_sum_out_host [rows,W,K] float32 (np.sum(mean_prob, axis=0)) or NULL. */
+int drs_scene_infer_multiscale(drs_handle_t h, int32_t scene_id, int32_t n_scales, const int32_t* crops_host, int32_t batch,
+                               int32_t variant, int32_t row_begin, int32_t row_end, uint8_t* labels_out_host,
+                               float* prob_sum_out_host);
+/* host-only (no device): the kernel's per-pixel softmax, compiled for the host, for CPU tests. in/out [n_pixels, K] float32 */
+int drs_debug_np_softmax(const float* in_host, int64_t n_pixels, int32_t K, float* out_host);
+/* host-only: the exp of that softmax (NumPy's float32 exp restated) on n float32 values */
+int drs_debug_np_expf(const float* in_host, int64_t n, float* out_host);
+/* unit-test entry: one launch of the multi-scale kernel on given sums and counts (K = the net's classes):
+ * acc += softmax(float32(prob/occur)) (acc ignored on input when first != 0), labels_out_host (or NULL) = first argmax(acc).
+ * prob [npix,K] float32, occur [npix] uint32, acc_inout [npix,K] float32, labels [npix] uint8, all host memory. */
+int drs_debug_multiscale_softmax_add(drs_handle_t h, const float* prob_host, const uint32_t* occur_host, int64_t npix,
+                                     int32_t first, float* acc_inout_host, uint8_t* labels_out_host);
+
 /* calc_accuracy_by_crop (isprs:510-531) / per-pixel scene confusion (isprs:1289-1296, contest:944-948):
  *   truth, pred [n] uint8 device; mask [n] or NULL; ignore_label <0 = none.
  *   cm_out [K*K+1] uint32 host: counts[true][pred] then #correct. */

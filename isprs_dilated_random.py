@@ -5,6 +5,7 @@ Same positional command line (isprs:1987-2042):
   input_path output_path currentModelPath trainingInstances testing_instances learningRate weight_decay batch_size niter
   reference_crop_size reference_stride_crop net_type distribution_type probValues update_type process
 process: training | validate_test | generate_final_maps.   Multi-GPU: launch under torchrun (one process per GPU).
+DRS_NUM_SCALES=N (N > 1): validate_test evaluates at the N best patch sizes (multi-scale, isprs:1347-1474).
 """
 import os
 import sys
@@ -41,6 +42,9 @@ def main():
     net_type, distribution_type = a[12], a[13]
     values = [int(i) for i in a[14].split(',')]
     update_type, process = a[15], a[16]
+    # the reference hard-codes num_scales=1, eval_type='single_scale' (isprs:2128-2131); DRS_NUM_SCALES=N > 1 turns
+    # validate_test into its multi-scale evaluation over the N best patch sizes of the saved score arrays
+    num_scales = int(os.environ.get("DRS_NUM_SCALES", "1"))
     display_step = 50
     if dataset == 'vaihingen':
         resample_batch = 20
@@ -116,7 +120,11 @@ def main():
                 pal = np.load(output_path + 'patch_acc_loss_step_' + str(step) + '.npy')
                 occ = np.load(output_path + 'patch_occur_step_' + str(step) + '.npy')
                 crop_size = host.select_best_patch_size(distribution_type, values, pal, occ, update_type, debug=True)
-            if process == 'validate_test':
+            if process == 'validate_test' and num_scales > 1:    # eval_type='multi_scale' (isprs:1347-1474)
+                loops.isprs_validate_test_multiscale(be, testing_data, testing_labels, testing_instances, batch_size, step,
+                                                     distribution_type, values, update_type, num_scales, False, output_path,
+                                                     NUM_CLASSES)
+            elif process == 'validate_test':
                 loops.isprs_validate_test(be, testing_data, testing_labels, testing_instances, batch_size, crop_size, step,
                                           NUM_CLASSES)
             else:
